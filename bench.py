@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference ...                     (the reference algorithm on the host cores: CPU oracle)
+  python bench.py ... --dump-outputs bench_outputs         (also write the last timed step's images to bench_outputs/<name>.npy)
 
 A "step" is one full render of the workload: Kerr a=0.998, observer r=1000 theta=60deg, ThinDisc(0,50),
 2048 x 2048 image plane per GPU, two fused point functions (redshift + disc radius), Tsit5 abstol=reltol=1e-9
@@ -142,9 +143,11 @@ def run_reference(args, rank, world):
         oracle.render_fast(p, ic, pfs, rng=rng, nthreads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.render_fast(p, ic, pfs, rng=rng, nthreads=threads)
+        imgs = oracle.render_fast(p, ic, pfs, rng=rng, nthreads=threads)
     dt = (time.perf_counter() - t0) / args.steps
     val = rng.count / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"redshift": imgs[0], "disc_radius": imgs[1]})
     t0 = time.perf_counter()
     oracle.render(p, ic, pfs, rng=cabi.Range(0, max(1, rng.count // 4), stride * 4), nthreads=threads)
     checker = max(1, rng.count // 4) / (time.perf_counter() - t0)
@@ -230,6 +233,8 @@ def run_ours(args, rank, world, local):
     total_rays = gd.sum_over_ranks(float(n_local), dev)
     total_attempts = gd.sum_over_ranks(float(attempts), dev)
     value = total_rays / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"redshift": d_imgs[0].cpu().numpy(), "disc_radius": d_imgs[1].cpu().numpy()})
 
     # ---- end-to-end arm: the reference-facing C-ABI call with HOST buffers (D2H inside the timed region)
     h_imgs = [torch.empty(n_local, dtype=torch.float64, pin_memory=True) for _ in pfs]
@@ -350,6 +355,24 @@ def run_ours(args, rank, world, local):
     emit(out)
 
 
+DUMP_RAYS = 1 << 21  # rays kept per dumped image: 2 images x (16 MiB of float64 + 8 MiB of float32 mask)
+
+
+def dump_outputs(path, images):
+    """Write each image of the last timed step as float64 `path/<name>.npy`, with `path/<name>_finite.npy` (float32, 1 where
+    the ray has a value): a ray that a filter drops (NaN, e.g. one that misses the disc) is stored as 0 and 0 in the mask, so
+    every stored number is finite.  An image of more than DUMP_RAYS rays is cut to the same seeded sample of rays (in ray
+    order) every run, so the dumps of two builds compare ray for ray."""
+    os.makedirs(path, exist_ok=True)
+    n = len(next(iter(images.values())))
+    keep = np.arange(n) if n <= DUMP_RAYS else np.sort(np.random.default_rng(0).choice(n, DUMP_RAYS, replace=False))
+    for name, img in images.items():
+        img = np.asarray(img, np.float64)[keep]
+        finite = np.isfinite(img)
+        np.save(os.path.join(path, f"{name}.npy"), np.where(finite, img, 0.0))
+        np.save(os.path.join(path, f"{name}_finite.npy"), finite.astype(np.float32))
+
+
 def run_callers(ens):
     """Secondary, N = 1 only: the two callers of the path built on host orchestration + device traces (SURVEY 8 f1/f2).
     Wall clock through the public API (host buffers both ways); the device share is launch-latency bound."""
@@ -432,8 +455,6 @@ def run_strong(args, rank, world, local, ens, dev, stream, sptr):
     p, ic = cfg.to_c()
     pfs = np.array([cabi.PF_REDSHIFT, cabi.PF_DISC_RADIUS], np.int32)
     flush = torch.empty(64 * 1024 * 1024, dtype=torch.float32, device=dev)
-    steps = max(3, args.steps)
-
     def time_shard(r, n):
         rng = gd.strip_interleaved_range(ic, r, n)
         imgs = [torch.empty(rng.count, dtype=torch.float64, device=dev) for _ in pfs]
@@ -442,12 +463,12 @@ def run_strong(args, rank, world, local, ens, dev, stream, sptr):
         for _ in range(2):
             call()
         torch.cuda.synchronize()
-        evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
+        evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
         for a, b in evs:
             flush.fill_(1.0)
             a.record(stream); call(); b.record(stream)
         torch.cuda.synchronize()
-        return sum(a.elapsed_time(b) for a, b in evs) / steps, rng.count, float(torch.nansum(imgs[0]).item())
+        return sum(a.elapsed_time(b) for a, b in evs) / args.steps, rng.count, float(torch.nansum(imgs[0]).item())
 
     out = {"workload": f"the same {w}x{h} C2 image split over N GPUs (strips of 4 columns, strip r, r+N, ... on rank r)"}
     if world > 1:
@@ -602,7 +623,12 @@ def main():
     ap.add_argument("--no-callers", action="store_true", help="skip the transfer-function / emissivity-profile timings")
     ap.add_argument("--lp-n", type=int, default=4096)
     ap.add_argument("--lp-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the images of the last timed step (rank 0's rays, a fixed seeded "
+                                                          f"sample of {DUMP_RAYS} per image) to DIR/<name>.npy as float64, "
+                                                          "NaN stored as 0 with DIR/<name>_finite.npy marking the rays that have a value")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
