@@ -209,10 +209,9 @@ def load():
     global _lib
     if _lib is not None:
         return _lib
-    path = os.environ.get("GB200_LIB", LIB_PATH)  # GB200_LIB: tuning variants of the same library (tools/)
-    if not os.path.exists(path):
-        raise GradusB200Error(ERR_NO_DEVICE, f"{path} not built; run __graft_entry__.build() (no CPU fallback exists)")
-    lib = C.CDLL(path)
+    if not os.path.exists(LIB_PATH):
+        raise GradusB200Error(ERR_NO_DEVICE, f"{LIB_PATH} not built; run __graft_entry__.build() (no CPU fallback exists)")
+    lib = C.CDLL(LIB_PATH)
     vp = C.c_void_p
     lib.gb200_version.restype = C.c_int
     lib.gb200_init.argtypes = [C.c_int, C.POINTER(vp)]

@@ -9,8 +9,7 @@
 // and a warp refills its lanes (one warp-aggregated atomicAdd) once GB_REFILL_THRESH of them have terminated.
 // Terminated lanes keep their last step and are finalised together (event root find on the dense output, discrete
 // callbacks, point function, endpoint store), so the divergent epilogue is paid once per batch, not once per ray.
-// The GB_OPT_* switches document the tuning steps of profiles/r01_tuning_log.md: each can be turned off to reproduce
-// the measurement behind it.
+// The measurements behind each of these choices are in profiles/r0{1,2}_tuning_log.md.
 //
 // What it replaces in the reference (all per ray, on CPU threads):
 //   prob_func -> velfunc(i) -> constrain_all         src/tracing/geodesic-problem.jl:121-154
@@ -25,76 +24,27 @@
 #include "gb200_device.cuh"
 #include "gb200_internal.h"
 
-#ifndef GB_BLOCK
-#define GB_BLOCK 32 /* one warp per CTA: the service decision needs no cross-warp barrier (v21 sweep, profiles/r01_tuning_log.md) */
-#endif
-#ifndef GB_MIN_BLOCKS
-#define GB_MIN_BLOCKS 12 /* 12 warps per SM at 168 registers per thread */
-#endif
-#ifndef GB_REFILL_THRESH
-#define GB_REFILL_THRESH 16 /* idle lanes per warp that trigger a service pass (per CTA: x warps per CTA) */
-#endif
-#ifndef GB_BLOCK_SYNC
-#define GB_BLOCK_SYNC 1 /* CTA-synchronous stepping: one barrier per step attempt keeps the warps of a CTA in lockstep */
-#endif
-#ifndef GB_SYNC_EVERY
-#define GB_SYNC_EVERY 16 /* service decision (a single-warp barrier count) every n-th attempt */
-#endif
-
-#ifndef GB_OPT_LOGEXP
-#define GB_OPT_LOGEXP 1 /* branch-free log/exp with constant-bank coefficients in the step controller */
-#endif
-
-#ifndef GB_OPT_QRCP_LO
-#define GB_OPT_QRCP_LO 0
-#endif
-#ifndef GB_OPT_INVQ
-#define GB_OPT_INVQ 0 /* step-size update from 1/q = clamp(gamma exp(-arg)): no reciprocal, no division on the reject path */
-#endif
-#ifndef GB_OPT_PROGERR
-#define GB_OPT_PROGERR 1 /* error sums accumulated stage by stage, error scales formed under the seventh RHS */
-#endif
-#ifndef GB_OPT_PARK
-#define GB_OPT_PARK 1 /* event lanes park their stage data in shared memory until finalise */
-#endif
-#ifndef GB_OPT_INTMAX
-#define GB_OPT_INTMAX 1 /* event-scan pre-test bound from integer maxima of the high words */
-#endif
-#ifndef GB_OPT_ERRDT
-#define GB_OPT_ERRDT 1 /* error norm with dt factored out of the eight components */
-#endif
-
-#if GB_OPT_PROGERR && !GB_OPT_ERRDT
-#error "GB_OPT_PROGERR accumulates the error sums without the dt factor: it needs GB_OPT_ERRDT"
-#endif
+constexpr int GB_BLOCK = 32;         // one warp per CTA: the service decision needs no cross-warp barrier (v21 sweep, profiles/r01_tuning_log.md)
+constexpr int GB_MIN_BLOCKS = 12;    // 12 warps per SM at 168 registers per thread
+constexpr int GB_REFILL_THRESH = 16; // idle lanes per warp that trigger a service pass (per CTA: x warps per CTA)
+constexpr int GB_SYNC_EVERY = 16;    // service decision (a single-warp barrier count) every n-th attempt
 
 #define LANE_EMPTY 0
 #define LANE_RUN 1
 #define LANE_PENDING 2
 #define FULLMASK 0xffffffffu
 
-// stage input  u + dt * sum_{l<S} a_{S+1,l+1} k_l   (S = 1..6 -> stages 2..7), summed left to right like the reference.
-// k0 is the FSAL slope (k1 of the tableau); k[1..5] are k2..k6.
-#ifndef GB_OPT_SMEMK
-#define GB_OPT_SMEMK 1 /* stage values k2..k6 live in shared memory instead of 60 registers */
-#endif
-// Storage of the stage values of one component: get(0) = k1 (FSAL), get(1..5) = k2..k6, get(6) = k7.  With GB_OPT_SMEMK
-// k2..k6 sit in shared memory ([stage][thread], conflict-free), k1 and k7 in registers; the indices are compile-time
-// constants after unrolling, so the selection folds away.
-#if GB_OPT_SMEMK
+// Storage of the stage values of one component: get(0) = k1 (FSAL), get(1..5) = k2..k6, get(6) = k7.  k2..k6 sit in
+// shared memory ([stage][thread], conflict-free) instead of 60 registers, k1 and k7 in registers; the indices are
+// compile-time constants after unrolling, so the selection folds away.
 struct GbK {
     double k1, k7;
     double* p; // &sh_k[first row of this component][threadIdx.x]
     GB_D double get(int j) const { return j == 0 ? k1 : (j == 6 ? k7 : p[(j - 1) * GB_BLOCK]); }
     GB_D void set(int j, double v) { if (j == 0) k1 = v; else if (j == 6) k7 = v; else p[(j - 1) * GB_BLOCK] = v; }
 };
-#else
-struct GbK {
-    double v[7];
-    GB_D double get(int j) const { return v[j]; }
-    GB_D void set(int j, double x) { v[j] = x; }
-};
-#endif
+// stage input  u + dt * sum_{l<S} a_{S+1,l+1} k_l   (S = 1..6 -> stages 2..7), summed left to right like the reference.
+// k0 is the FSAL slope (k1 of the tableau); k[1..5] are k2..k6.
 template <int S>
 GB_D double comb(double u, double dt, double k0, const GbK& k) {
     if (S == 1) return fma(dt * GB_A21, k0, u);
@@ -103,10 +53,6 @@ GB_D double comb(double u, double dt, double k0, const GbK& k) {
     if (S == 4) return fma(dt, fma(GB_A54, k.get(3), fma(GB_A53, k.get(2), fma(GB_A52, k.get(1), GB_A51 * k0))), u);
     if (S == 5) return fma(dt, fma(GB_A65, k.get(4), fma(GB_A64, k.get(3), fma(GB_A63, k.get(2), fma(GB_A62, k.get(1), GB_A61 * k0)))), u);
     return fma(dt, fma(GB_A76, k.get(5), fma(GB_A75, k.get(4), fma(GB_A74, k.get(3), fma(GB_A73, k.get(2), fma(GB_A72, k.get(1), GB_A71 * k0))))), u);
-}
-// sum_j btilde_j k_j with k_1 = k0, k_7 = k6
-GB_D double errcomb(double k0, const GbK& k, double k6) {
-    return fma(GB_BT7, k6, fma(GB_BT6, k.get(5), fma(GB_BT5, k.get(4), fma(GB_BT4, k.get(3), fma(GB_BT3, k.get(2), fma(GB_BT2, k.get(1), GB_BT1 * k0))))));
 }
 template <int S> GB_D constexpr double a7coef() {
     return S == 0 ? GB_A71 : S == 1 ? GB_A72 : S == 2 ? GB_A73 : S == 3 ? GB_A74 : S == 4 ? GB_A75 : GB_A76;
@@ -132,72 +78,25 @@ GB_D double ctrl_pow_log(double logx, double x, double y, int mode) {
     return exp(y * logx);
 }
 
-// The argument of larger magnitude (the caller applies fabs as an operand modifier: selecting |a| or |b| directly makes the
-// compiler materialise both absolute values with two extra FP64 instructions).
-#ifndef GB_OPT_INTCMP
-#define GB_OPT_INTCMP 0 /* comparisons of non-negative doubles as 64-bit integers: measured slower (42.8 vs 42.5 ms), kept as a switch */
-#endif
-#if GB_OPT_INTCMP
-// IEEE doubles of equal sign order like their bit patterns; a nan compares as larger than every finite value, so it is
-// the one selected and keeps propagating (the FP form selects b for a nan a).
-GB_D double gb_absmax(double a, double b) {
-    return (__double_as_longlong(a) & 0x7fffffffffffffffLL) > (__double_as_longlong(b) & 0x7fffffffffffffffLL) ? a : b;
-}
-GB_D double gb_max_pos(double a, double b) { return __double_as_longlong(a) > __double_as_longlong(b) ? a : b; } // a, b >= 0
-GB_D double gb_min_pos(double a, double b) { return __double_as_longlong(a) < __double_as_longlong(b) ? a : b; }
-GB_D bool gb_le_one_pos(double a) { return (unsigned long long)__double_as_longlong(a) <= 0x3ff0000000000000ULL; } // 0 <= a <= 1 (false for nan)
-#else
-GB_D double gb_absmax(double a, double b) { return fabs(a) > fabs(b) ? a : b; }
-GB_D double gb_max_pos(double a, double b) { return gb_max(a, b); }
-GB_D double gb_min_pos(double a, double b) { return gb_min(a, b); }
-GB_D bool gb_le_one_pos(double a) { return a <= 1.0; }
-#endif
+// The step acceptance test EEst^2 <= 1.  Written as a call it yields the same instructions as the comparison written
+// in place, but a different schedule of the step counters that follow it.
+GB_D bool gb_le_one(double a) { return a <= 1.0; }
 
 // 1 / (abstol + reltol max(|a|, |b|)): the reciprocal error scale of one component (calculate_residuals,
 // DiffEqBase).  The estimate it feeds enters the controller through EEst^(7/50) and the test EEst <= 1, and the reference
-// itself evaluates that power at Float32 accuracy (FastPower), so the scale does not need 53 bits:
-//   0  hardware seed + one Newton step (2^-40)
-//   1  hardware seed alone (rcp.approx.f64: 2^-20 and better) -- two DFMAs fewer per component
-//   2  Float32 on the otherwise idle FP32 / integer / special-function pipes: max(|a|, |b|) from the high words (20
-//      mantissa bits), one FFMA, one rcp.approx.f32, widened back through the exponent field -- no FP64 instruction at all
-//   3  as 2 with conversion instructions instead of the integer exponent arithmetic
-// Measured on C2 (profiles/r02_tuning_log.md): 40.48 / 39.93 / 39.79 / 39.98 ms for 0 / 1 / 2 / 3.  1 is the default: 2 moves
-// 36 of 1.94 M disc hits across the grazing band (its truncated |u| biases every scale by up to 1e-6), 1 moves one.
-#ifndef GB_OPT_NORMRCP
-#define GB_OPT_NORMRCP 1
-#endif
-GB_D double gb_inv_scale(double a, double b, double reltol, double abstol, float reltolf, float abstolf) {
-#if GB_OPT_NORMRCP == 0
-    return gb_rcp_lo(fma(fabs(gb_absmax(a, b)), reltol, abstol));
-#elif GB_OPT_NORMRCP == 1
+// itself evaluates that power at Float32 accuracy (FastPower), so the scale does not need 53 bits: the hardware seed alone
+// (rcp.approx.f64: 2^-20 and better) is used, two DFMAs fewer per component than one Newton step on it.  Measured on C2
+// (profiles/r02_tuning_log.md): 39.93 ms; seed + one Newton step (2^-40) 40.48 ms; the scale in Float32 on the FP32 /
+// integer / special-function pipes 39.79 ms, but its truncated |u| biases every scale by up to 1e-6 and moves 36 of 1.94 M
+// disc hits across the grazing band, where the seed moves one.
+GB_D double gb_inv_scale(double a, double b, double reltol, double abstol) {
+    // fabs is applied to the argument of larger magnitude as an operand modifier: selecting |a| or |b| directly makes the
+    // compiler materialise both absolute values with two extra FP64 instructions
+    const double m = fabs(a) > fabs(b) ? a : b;
     double y;
-    const double x = fma(fabs(gb_absmax(a, b)), reltol, abstol);
+    const double x = fma(fabs(m), reltol, abstol);
     asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
     return y;
-#elif GB_OPT_NORMRCP == 2
-    int h = max(__double2hiint(a) & 0x7fffffff, __double2hiint(b) & 0x7fffffff);
-    h = min(max(h, 0x38100000), 0x47e00000); // keep the exponent inside the normal range of a float
-    const float m = __int_as_float((h - 0x38000000) << 3);
-    float is;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(is) : "f"(fmaf(m, reltolf, abstolf)));
-    const int fb = __float_as_int(is);
-    return __hiloint2double((fb >> 3) + 0x38000000, fb << 29);
-#else
-    const float m = fmaxf(fabsf((float)a), fabsf((float)b));
-    float is;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(is) : "f"(fmaf(m, reltolf, abstolf)));
-    return (double)is;
-#endif
-}
-
-// An upper bound of max_i |a_i| from the high words alone (integer pipe): doubles order like their bit patterns, and
-// (hi + 1, 0) exceeds every double whose high word is hi.  inf/nan inputs give a nan bound, which the caller's
-// comparisons treat as "cannot skip".
-GB_D double absmax7_bound(double a0, double a1, double a2, double a3, double a4, double a5, double a6) {
-    const int m = 0x7fffffff;
-    const int h = max(max(max(__double2hiint(a0) & m, __double2hiint(a1) & m), max(__double2hiint(a2) & m, __double2hiint(a3) & m)),
-                      max(max(__double2hiint(a4) & m, __double2hiint(a5) & m), __double2hiint(a6) & m));
-    return __hiloint2double(h + 1, 0);
 }
 
 // Can the disc condition become negative anywhere on this step?  Conservative bound from the dense-output
@@ -244,19 +143,10 @@ __device__ __noinline__ void gb_hist_add(const GbParams& P, unsigned long long* 
     gb_acc128(&sh_hist[bin], &sh_hist[P.lp_nbins + bin], wlo, whi);
 }
 
-#ifdef GB_MAXRREG /* tuning: explicit register cap instead of the occupancy target */
-#define GB_LAUNCH_BOUNDS __maxnreg__(GB_MAXRREG)
-#else
-#ifndef GB_MIN_BLOCKS_KERR
-#define GB_MIN_BLOCKS_KERR GB_MIN_BLOCKS /* the Kerr instantiations tolerate 16 warps per SM at 128 registers (tuning log) */
-#endif
-#define GB_LAUNCH_BOUNDS __launch_bounds__(GB_BLOCK, (METRIC == GB200_METRIC_KERR ? GB_MIN_BLOCKS_KERR : GB_MIN_BLOCKS))
-#endif
 template <int METRIC, int GEOM>
-__global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbParams P) {
+__global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(const __grid_constant__ GbParams P) {
     const unsigned lane = threadIdx.x & 31u;
     const double abstol = P.abstol, reltol = P.reltol;
-    const float abstolf = fmaxf((float)P.abstol, 1e-30f), reltolf = (float)P.reltol; // GB_OPT_NORMRCP >= 2
     const double tstop = P.lam1;
     const double dtmax = P.dtmax;
     const double dtmin = 2.220446049250313e-16;
@@ -281,7 +171,6 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
     const int maxit = (int)(P.maxiters < 0x7fffffff ? P.maxiters : 0x7fffffff); // step attempts are counted in 32 bits
     bool exhausted = false;
     unsigned long long tot_acc = 0, tot_rej = 0, tot_flag = 0;
-#if GB_OPT_SMEMK
     // k2..k6 of the four accelerations and of the r, theta stage velocities: 30 rows; rows 30..33 park the k7
     // accelerations of a lane whose step ended in a disc event until it is finalised.
     __shared__ double sh_k[34][GB_BLOCK];
@@ -290,7 +179,6 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
     kR.k1 = kR.k7 = kT.k1 = kT.k7 = 0.0;
 #pragma unroll
     for (int j = 0; j < 34; ++j) sh_k[j][threadIdx.x] = 0.0;
-#endif
 #pragma unroll
     for (int j = 0; j < 7; ++j) { kA0.set(j, 0.0); kA1.set(j, 0.0); kA2.set(j, 0.0); kA3.set(j, 0.0); }
 #pragma unroll
@@ -299,50 +187,25 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
     extern __shared__ unsigned long long sh_hist[]; // 2 * lp_nbins words when the line-profile histogram is fused, else empty
     if (P.lp_bins)
         for (int b = threadIdx.x; b < 2 * P.lp_nbins; b += GB_BLOCK) sh_hist[b] = 0ull;
-#if GB_OPT_PARK && !GB_OPT_SMEMK
-    // Stage data of a lane whose step ended in a disc event, parked until the lane is finalised: k2..k7 accelerations
-    // (24) and the k2..k6 stage velocities of r and theta (10), [value][thread] so a warp's accesses are conflict-free.
-    // Keeping them in registers instead made every attempt spill ~20 of them for the (rare) root find.
-    __shared__ double sh_park[34][GB_BLOCK];
-#endif
-#if GB_BLOCK_SYNC
     unsigned loop_count = 0;
     __shared__ int sh_exhausted;
     if (threadIdx.x == 0) sh_exhausted = 0;
     __syncthreads();
-#endif
     for (;;) {
-#if GB_BLOCK_SYNC
         // A barrier every GB_SYNC_EVERY-th step attempt: the warps of a CTA walk the (long, straight-line) step code
         // together and share its instruction-cache lines, and the decision to run the cold service code is CTA-uniform,
         // so that code is fetched once per CTA instead of once per warp.
         bool service = false;
-        if (GB_SYNC_EVERY == 1 || (loop_count++ % GB_SYNC_EVERY) == 0) {
+        if ((loop_count++ % GB_SYNC_EVERY) == 0) {
             const int idle_cta = __syncthreads_count(state != LANE_RUN);
             service = idle_cta >= GB_REFILL_THRESH * (GB_BLOCK / 32) || idle_cta == GB_BLOCK;
         }
-#else
-        unsigned run_mask = __ballot_sync(FULLMASK, state == LANE_RUN);
-        const unsigned pend_mask = __ballot_sync(FULLMASK, state == LANE_PENDING);
-        const int nidle = 32 - __popc(run_mask);
-        const bool service = (run_mask == 0) || (nidle >= GB_REFILL_THRESH && (pend_mask != 0 || !exhausted));
-#endif
         if (service) {
             // ================= finalise terminated lanes =================
             if (state == LANE_PENDING) {
                 int status = pend_status;
                 if (GEOM != GB200_GEOMETRY_NONE && pend_event) {
-#if GB_OPT_SMEMK
                     kA0.k7 = sh_k[30][threadIdx.x]; kA1.k7 = sh_k[31][threadIdx.x]; kA2.k7 = sh_k[32][threadIdx.x]; kA3.k7 = sh_k[33][threadIdx.x];
-#elif GB_OPT_PARK
-#pragma unroll
-                    for (int j = 0; j < 6; ++j) {
-                        kA0.set(j + 1, sh_park[j][threadIdx.x]); kA1.set(j + 1, sh_park[6 + j][threadIdx.x]);
-                        kA2.set(j + 1, sh_park[12 + j][threadIdx.x]); kA3.set(j + 1, sh_park[18 + j][threadIdx.x]);
-                    }
-#pragma unroll
-                    for (int j = 0; j < 5; ++j) { kR.set(j + 1, sh_park[24 + j][threadIdx.x]); kT.set(j + 1, sh_park[29 + j][threadIdx.x]); }
-#endif
                     // ContinuousCallback root find on the dense output (DiffEqBase find_callback_time, LeftRootFind)
                     double C2r, C3r, C4r, C2t, C3t, C4t;
                     dense_coeffs(vr, kR, nvr, C2r, C3r, C4r);
@@ -538,19 +401,12 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
                 }
                 if ((int64_t)base + nfree >= P.count) {
                     exhausted = true;
-#if GB_BLOCK_SYNC
                     if (lane == 0) *(volatile int*)&sh_exhausted = 1;
-#endif
                 }
             }
-#if GB_BLOCK_SYNC
             const int running_cta = __syncthreads_count(state == LANE_RUN);
             exhausted = (*(volatile int*)&sh_exhausted) != 0; // written only inside a service pass, read only after its closing barrier
             if (running_cta == 0) break;                       // CTA-uniform: queue drained and every lane finalised
-#else
-            run_mask = __ballot_sync(FULLMASK, state == LANE_RUN);
-            if (run_mask == 0) break;
-#endif
         }
 
         // ================= one Tsit5 step attempt for every running lane (straight-line: no taken branches) ==========
@@ -571,58 +427,42 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
             double acc[4], s_ = 0, c_ = 1;
             double tsum = GB_A71 * vt, psum = GB_A71 * vph; // sum_j a7j k_j[1], k_j[4]
             double terr = GB_BT1 * vt, perr = GB_BT1 * vph; // sum_j btilde_j k_j[1], k_j[4]
-#if GB_OPT_PROGERR
-            // the other six error sums are accumulated stage by stage too (same order of summation as errcomb): their
-            // FMAs fill the latency gaps of the next stage instead of forming a serial tail after the seventh
+            // the other six error sums are accumulated stage by stage too (btilde_1 .. btilde_7 in order): their FMAs fill
+            // the latency gaps of the next stage instead of forming a serial tail after the seventh
             double rerr = GB_BT1 * vr, therr = GB_BT1 * vth;
             double a0err = GB_BT1 * kA0.get(0), a1err = GB_BT1 * kA1.get(0), a2err = GB_BT1 * kA2.get(0), a3err = GB_BT1 * kA3.get(0);
-#define GB_STAGE_ERR_V(S) rerr = fma(btcoef<S>(), w1, rerr); therr = fma(btcoef<S>(), w2, therr);
-#define GB_STAGE_ERR_A(S)                                                                                               \
-    a0err = fma(btcoef<S>(), acc[0], a0err); a1err = fma(btcoef<S>(), acc[1], a1err);                                   \
-    a2err = fma(btcoef<S>(), acc[2], a2err); a3err = fma(btcoef<S>(), acc[3], a3err);
-#else
-#define GB_STAGE_ERR_V(S)
-#define GB_STAGE_ERR_A(S)
-#endif
-#if GB_OPT_SMEMK && GB_OPT_INTMAX
             // running maxima of the high words of |k_j[r]|, |k_j[theta]| for the event-scan pre-test (no re-read from shared memory)
             int mxr = __double2hiint(vr) & 0x7fffffff, mxt = __double2hiint(vth) & 0x7fffffff;
-#define GB_STAGE_MAX mxr = max(mxr, __double2hiint(w1) & 0x7fffffff); mxt = max(mxt, __double2hiint(w2) & 0x7fffffff);
-#else
-#define GB_STAGE_MAX
-#endif
 #define GB_STAGE(S)                                                                                                     \
     {                                                                                                                   \
         const double xr = comb<S>(r, dt, vr, kR), xt = comb<S>(th, dt, vth, kT);                                        \
-        const double w0 = comb<S>(vt, dt, kA0.get(0), kA0), w1 = comb<S>(vr, dt, kA1.get(0), kA1),                              \
-                     w2 = comb<S>(vth, dt, kA2.get(0), kA2), w3 = comb<S>(vph, dt, kA3.get(0), kA3);                            \
+        const double w0 = comb<S>(vt, dt, kA0.get(0), kA0), w1 = comb<S>(vr, dt, kA1.get(0), kA1),                      \
+                     w2 = comb<S>(vth, dt, kA2.get(0), kA2), w3 = comb<S>(vph, dt, kA3.get(0), kA3);                    \
         kR.set(S, w1); kT.set(S, w2);                                                                                   \
-        GB_STAGE_MAX                                                                                                    \
+        mxr = max(mxr, __double2hiint(w1) & 0x7fffffff); mxt = max(mxt, __double2hiint(w2) & 0x7fffffff);              \
         tsum = fma(a7coef<S>(), w0, tsum); psum = fma(a7coef<S>(), w3, psum);                                           \
         terr = fma(btcoef<S>(), w0, terr); perr = fma(btcoef<S>(), w3, perr);                                           \
-        GB_STAGE_ERR_V(S)                                                                                               \
+        rerr = fma(btcoef<S>(), w1, rerr); therr = fma(btcoef<S>(), w2, therr);                                         \
         rhs_accel<METRIC>(P, xr, xt, w0, w1, w2, w3, acc, s_, c_);                                                      \
         kA0.set(S, acc[0]); kA1.set(S, acc[1]); kA2.set(S, acc[2]); kA3.set(S, acc[3]);                                 \
-        GB_STAGE_ERR_A(S)                                                                                               \
+        a0err = fma(btcoef<S>(), acc[0], a0err); a1err = fma(btcoef<S>(), acc[1], a1err);                               \
+        a2err = fma(btcoef<S>(), acc[2], a2err); a3err = fma(btcoef<S>(), acc[3], a3err);                               \
     }
             GB_STAGE(1) GB_STAGE(2) GB_STAGE(3) GB_STAGE(4) GB_STAGE(5)
 #undef GB_STAGE
-#if GB_OPT_SC7
             const double th6 = comb<5>(th, dt, vth, kT); // the sixth stage's polar angle (the compiler merges it with the stage's own)
-#endif
             // 7th stage = the proposed state (FSAL)
             nr = comb<6>(r, dt, vr, kR); nth = comb<6>(th, dt, vth, kT);
             nvt = comb<6>(vt, dt, kA0.get(0), kA0); nvr = comb<6>(vr, dt, kA1.get(0), kA1);
             nvth = comb<6>(vth, dt, kA2.get(0), kA2); nvph = comb<6>(vph, dt, kA3.get(0), kA3);
             nct = fma(dt, tsum, ct); nph = fma(dt, psum, ph);
             terr = fma(GB_BT7, nvt, terr); perr = fma(GB_BT7, nvph, perr);
-#if GB_OPT_PROGERR
             rerr = fma(GB_BT7, nvr, rerr); therr = fma(GB_BT7, nvth, therr);
             // the eight error scales only need u_prev and u: they are formed while the seventh RHS is in flight
-            const double is0 = gb_inv_scale(ct, nct, reltol, abstol, reltolf, abstolf), is1 = gb_inv_scale(r, nr, reltol, abstol, reltolf, abstolf);
-            const double is2 = gb_inv_scale(th, nth, reltol, abstol, reltolf, abstolf), is3 = gb_inv_scale(ph, nph, reltol, abstol, reltolf, abstolf);
-            const double is4 = gb_inv_scale(vt, nvt, reltol, abstol, reltolf, abstolf), is5 = gb_inv_scale(vr, nvr, reltol, abstol, reltolf, abstolf);
-            const double is6 = gb_inv_scale(vth, nvth, reltol, abstol, reltolf, abstolf), is7 = gb_inv_scale(vph, nvph, reltol, abstol, reltolf, abstolf);
+            const double is0 = gb_inv_scale(ct, nct, reltol, abstol), is1 = gb_inv_scale(r, nr, reltol, abstol);
+            const double is2 = gb_inv_scale(th, nth, reltol, abstol), is3 = gb_inv_scale(ph, nph, reltol, abstol);
+            const double is4 = gb_inv_scale(vt, nvt, reltol, abstol), is5 = gb_inv_scale(vr, nvr, reltol, abstol);
+            const double is6 = gb_inv_scale(vth, nvth, reltol, abstol), is7 = gb_inv_scale(vph, nvph, reltol, abstol);
             double ee = 0;
             {
                 double q_;
@@ -631,15 +471,9 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
                 q_ = therr * is2; ee = fma(q_, q_, ee);
                 q_ = perr * is3; ee = fma(q_, q_, ee);
             }
-#endif
-#if GB_OPT_SC7
             rhs_accel_near<METRIC>(P, nr, nth, nvt, nvr, nvth, nvph, th6, s_, c_, acc, s_, c_);
-#else
-            rhs_accel<METRIC>(P, nr, nth, nvt, nvr, nvth, nvph, acc, s_, c_);
-#endif
             kA0.set(6, acc[0]); kA1.set(6, acc[1]); kA2.set(6, acc[2]); kA3.set(6, acc[3]);
             // ---- error estimate: rms( dt*sum btilde_j k_j / (abstol + max(|u_prev|,|u|) reltol) )
-#if GB_OPT_PROGERR
             {
                 double q_;
                 q_ = fma(GB_BT7, acc[0], a0err) * is4; ee = fma(q_, q_, ee);
@@ -647,97 +481,39 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
                 q_ = fma(GB_BT7, acc[2], a2err) * is6; ee = fma(q_, q_, ee);
                 q_ = fma(GB_BT7, acc[3], a3err) * is7; ee = fma(q_, q_, ee);
             }
-#else
-            double ee = 0;
-            {
-#if GB_OPT_ERRDT
-                const double edt = 1.0; // dt multiplies the norm once, below
-#else
-                const double edt = dt;
-#endif
-                const double e0 = edt * terr, e1 = edt * errcomb(vr, kR, nvr), e2 = edt * errcomb(vth, kT, nvth), e3 = edt * perr;
-                const double e4 = edt * errcomb(kA0.get(0), kA0, kA0.get(6)), e5 = edt * errcomb(kA1.get(0), kA1, kA1.get(6));
-                const double e6 = edt * errcomb(kA2.get(0), kA2, kA2.get(6)), e7 = edt * errcomb(kA3.get(0), kA3, kA3.get(6));
-                double q_;
-                q_ = e0 * gb_rcp_lo(fma(fabs(gb_absmax(ct, nct)), reltol, abstol)); ee = fma(q_, q_, ee);
-                q_ = e1 * gb_rcp_lo(fma(fabs(gb_absmax(r, nr)), reltol, abstol)); ee = fma(q_, q_, ee);
-                q_ = e2 * gb_rcp_lo(fma(fabs(gb_absmax(th, nth)), reltol, abstol)); ee = fma(q_, q_, ee);
-                q_ = e3 * gb_rcp_lo(fma(fabs(gb_absmax(ph, nph)), reltol, abstol)); ee = fma(q_, q_, ee);
-                q_ = e4 * gb_rcp_lo(fma(fabs(gb_absmax(vt, nvt)), reltol, abstol)); ee = fma(q_, q_, ee);
-                q_ = e5 * gb_rcp_lo(fma(fabs(gb_absmax(vr, nvr)), reltol, abstol)); ee = fma(q_, q_, ee);
-                q_ = e6 * gb_rcp_lo(fma(fabs(gb_absmax(vth, nvth)), reltol, abstol)); ee = fma(q_, q_, ee);
-                q_ = e7 * gb_rcp_lo(fma(fabs(gb_absmax(vph, nvph)), reltol, abstol)); ee = fma(q_, q_, ee);
-            }
-#endif
             // EEst^2 = dt^2 sum_i (.)^2 / 8; the controller only needs log EEst = log(EEst^2) / 2 and the test EEst <= 1, so no
             // square root is taken (the Float32 controller mode takes it where it needs EEst itself).  An exactly zero
             // estimate is raised to 1e-150: the controller clamps q to 1/qmax and qold to 1e-4 either way.
-#if GB_OPT_ERRDT
-            const double EEst2 = gb_max_pos((dt * dt) * (ee * 0.125), 1e-300);
-#else
-            const double EEst2 = gb_max(ee * 0.125, 1e-300);
-#endif
+            const double EEst2 = gb_max((dt * dt) * (ee * 0.125), 1e-300);
             // PI controller (stepsize_controller!, OrdinaryDiffEq): q = EEst^beta1 / qold^beta2 / gamma, clamped; a rejected
             // attempt uses EEst^beta1 / gamma (step_reject_controller!).  One log and one exp serve both:
             // exp(beta1 log EEst - [accepted] beta2 log qold).
-            const bool accept = gb_le_one_pos(EEst2);
+            const bool accept = gb_le_one(EEst2);
             const bool fast32 = (P.pow_mode == GB200_POW_FAST32);
-#if GB_OPT_LOGEXP
-            const double logE = 0.5 * (GB_OPT_CTRL_LO ? gb_log_pos_lo(EEst2) : gb_log_pos(EEst2));
-#else
-            const double logE = 0.5 * log(EEst2);
-#endif
+            const double logE = 0.5 * gb_log_pos_lo(EEst2);
             double EEst = 1.0; // only the Float32 mode reads it
             if (fast32) EEst = gb_sqrt_pos(EEst2);
-#if GB_OPT_INVQ
-            // The controller only ever divides by q: form 1/q = clamp(gamma / (EEst^beta1 / qold^beta2), qmin, qmax) from
-            // exp(-arg) directly -- no reciprocal of q, and the rejected step's dt / min(1/qmin, EEst^beta1 / gamma) becomes a
-            // product as well (that one was an IEEE division).
-            double Einv; // 1 / (EEst^beta1 / qold^beta2) for an accepted step, 1 / EEst^beta1 for a rejected one
-            if (fast32) {
-                double Epow = ctrl_pow_log(logE, EEst, beta1, P.pow_mode);
-                if (accept) Epow *= gb_rcp(qoldpow);
-                Einv = gb_rcp(Epow);
-            } else {
-                const double arg = accept ? fma(beta1, logE, -qoldpow) : beta1 * logE; // qoldpow = beta2 * log(qold) in this mode
-                const double narg = gb_max(-8.0, gb_min(8.0, -arg));
-                Einv = GB_OPT_CTRL_LO ? gb_exp_small_lo(narg) : gb_exp_small(narg); // 1/q is clamped to [qmin, qmax] = exp(-1.7 .. 2.3) afterwards
-            }
-            const double gEinv = gamma * Einv;
-            const double dtnew = dt * gb_max_pos(qmin, gb_min_pos(qmax, gEinv));
-#else
             double Epow;
             if (fast32) {
                 Epow = ctrl_pow_log(logE, EEst, beta1, P.pow_mode);
                 if (accept) Epow *= gb_rcp(qoldpow);
             } else {
                 const double arg = accept ? fma(beta1, logE, -qoldpow) : beta1 * logE; // qoldpow = beta2 * log(qold) in this mode
-#if GB_OPT_LOGEXP
                 const double carg = gb_max(-8.0, gb_min(8.0, arg));
-                Epow = GB_OPT_CTRL_LO ? gb_exp_small_lo(carg) : gb_exp_small(carg); // q is clamped to [1/qmax, 1/qmin] = exp(-2.2 .. 1.7) afterwards
-#else
-                Epow = exp(arg);
-#endif
+                Epow = gb_exp_small_lo(carg); // q is clamped to [1/qmax, 1/qmin] = exp(-2.2 .. 1.7) afterwards
             }
-            const double q = gb_max_pos(1.0 / qmax, gb_min_pos(1.0 / qmin, Epow * (1.0 / gamma)));
+            const double q = gb_max(1.0 / qmax, gb_min(1.0 / qmin, Epow * (1.0 / gamma)));
             // ---- accept / reject, callbacks and the commit of the step.  Everything up to the commit is computed
             // unconditionally and committed with selects: the loop-carried state then lives in the same registers on
             // every path (the branchy form cost ~200 register moves per attempt where the paths merged).
-#if GB_OPT_QRCP_LO /* q is known to 1e-7: one Newton step on the reciprocal seed (2^-40) */
-            const double dtnew = dt * gb_rcp_lo(q);
-#else
+            // Measured alternatives (profiles/r02_tuning_log.md): forming 1/q directly, with no reciprocal here and no
+            // division in dtrej, was within the spread; one Newton step instead of gb_rcp's third-order correction gained nothing.
             const double dtnew = dt * gb_rcp(q);
-#endif
-#endif
             const double ttmp = lam + dt;
             const double tnew = (fabs(ttmp - tstop) < 100.0 * (fabs(tstop) * 2.220446049250313e-16)) ? tstop : ttmp;
-            const double dtprop = gb_max_pos(gb_min_pos(dtmax, dtnew), dtmin);
-#if GB_OPT_INVQ
-            const double dtrej = gb_max(dt * gb_max_pos(qmin, gEinv), dtmin); // only read when the step is rejected
-#else
+            const double dtprop = gb_max(gb_min(dtmax, dtnew), dtmin);
             double dtrej = dt;
             if (!accept) dtrej = gb_max(dt / gb_min(1.0 / qmin, Epow / gamma), dtmin);
-#endif
             // ---- callbacks: continuous (disc) first, then discrete (user, chart)
             bool event = false;
             double cnext = 1.0;
@@ -750,16 +526,11 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
                         // cheap bound first: |u(Th) - u0| <= |dt| * L * max_j |k_j| with L = max_Th sum_j |b_j(Th)| = 7.5822
                         // for the Tsit5 dense output; only when it is inconclusive are the polynomial coefficients formed
                         const double adt = fabs(dt);
-#if GB_OPT_SMEMK && GB_OPT_INTMAX
+                        // max_j |k_j| bounded from the high words alone (integer pipe): doubles order like their bit
+                        // patterns, and (hi + 1, 0) exceeds every double whose high word is hi.  inf/nan give a nan bound,
+                        // which the comparisons in scan_needed treat as "cannot skip".
                         const double mth = __hiloint2double(max(mxt, __double2hiint(nvth) & 0x7fffffff) + 1, 0);
                         const double mr = __hiloint2double(max(mxr, __double2hiint(nvr) & 0x7fffffff) + 1, 0);
-#elif GB_OPT_INTMAX
-                        const double mth = absmax7_bound(vth, kT.get(1), kT.get(2), kT.get(3), kT.get(4), kT.get(5), nvth);
-                        const double mr = absmax7_bound(vr, kR.get(1), kR.get(2), kR.get(3), kR.get(4), kR.get(5), nvr);
-#else
-                        const double mth = fmax(fmax(fmax(fabs(vth), fabs(kT.get(1))), fmax(fabs(kT.get(2)), fabs(kT.get(3)))), fmax(fmax(fabs(kT.get(4)), fabs(kT.get(5))), fabs(nvth)));
-                        const double mr = fmax(fmax(fmax(fabs(vr), fabs(kR.get(1))), fmax(fabs(kR.get(2)), fabs(kR.get(3)))), fmax(fmax(fabs(kR.get(4)), fabs(kR.get(5))), fabs(nvr)));
-#endif
                         bool need = sprev < 0.0 || scan_needed<GEOM>(P, r, acos_prev, cprev, adt * 7.5823 * mth, adt * 7.5823 * mr);
                         double C2r = 0, C3r = 0, C4r = 0, C2t = 0, C3t = 0, C4t = 0;
                         if (need) {
@@ -782,21 +553,9 @@ __global__ void GB_LAUNCH_BOUNDS gb200_trace_kernel(const __grid_constant__ GbPa
                     }
                 }
             }
-#if GB_OPT_SMEMK
             if (GEOM != GB200_GEOMETRY_NONE && event) { // k2..k6 are in shared memory already; k7 joins them
                 sh_k[30][threadIdx.x] = kA0.k7; sh_k[31][threadIdx.x] = kA1.k7; sh_k[32][threadIdx.x] = kA2.k7; sh_k[33][threadIdx.x] = kA3.k7;
             }
-#elif GB_OPT_PARK
-            if (GEOM != GB200_GEOMETRY_NONE && event) {
-#pragma unroll
-                for (int j = 0; j < 6; ++j) {
-                    sh_park[j][threadIdx.x] = kA0.get(j + 1); sh_park[6 + j][threadIdx.x] = kA1.get(j + 1);
-                    sh_park[12 + j][threadIdx.x] = kA2.get(j + 1); sh_park[18 + j][threadIdx.x] = kA3.get(j + 1);
-                }
-#pragma unroll
-                for (int j = 0; j < 5; ++j) { sh_park[24 + j][threadIdx.x] = kR.get(j + 1); sh_park[29 + j][threadIdx.x] = kT.get(j + 1); }
-            }
-#endif
             int status = GB200_STATUS_NO_STATUS;
             bool term = false;
             if (P.callback_kind == GB200_CALLBACK_UPPER_HEMISPHERE && nr * c_ < P.callback_delta) { status = GB200_STATUS_OUT_OF_DOMAIN; term = true; }
@@ -866,16 +625,11 @@ static cudaError_t launch_one(const GbParams& P, int sm_count, cudaStream_t stre
 template <int METRIC>
 static cudaError_t launch_geom(const GbParams& P, int sm_count, cudaStream_t stream, int* blocks_out) {
     switch (P.geometry_kind) {
-#ifdef GB_TUNE_MINIMAL /* tuning builds (tools/build_variant.sh): thin disc only, Kerr and Johannsen-Psaltis only */
-    case GB200_GEOMETRY_THIN_DISC: return launch_one<METRIC, GB200_GEOMETRY_THIN_DISC>(P, sm_count, stream, blocks_out);
-    default: return cudaErrorInvalidValue;
-#else
     case GB200_GEOMETRY_NONE: return launch_one<METRIC, GB200_GEOMETRY_NONE>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_THIN_DISC: return launch_one<METRIC, GB200_GEOMETRY_THIN_DISC>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_SHAKURA_SUNYAEV: return launch_one<METRIC, GB200_GEOMETRY_SHAKURA_SUNYAEV>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_DATUM_PLANE: return launch_one<METRIC, GB200_GEOMETRY_DATUM_PLANE>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_THICK_TABLE: return launch_one<METRIC, GB200_GEOMETRY_THICK_TABLE>(P, sm_count, stream, blocks_out);
-#endif
     }
     return cudaErrorInvalidValue;
 }
@@ -884,13 +638,11 @@ cudaError_t gb200_launch_trace(const GbParams& P, int sm_count, cudaStream_t str
     switch (P.metric_kind) {
     case GB200_METRIC_KERR: return launch_geom<GB200_METRIC_KERR>(P, sm_count, stream, blocks_out);
     case GB200_METRIC_JOHANNSEN_PSALTIS: return launch_geom<GB200_METRIC_JOHANNSEN_PSALTIS>(P, sm_count, stream, blocks_out);
-#ifndef GB_TUNE_MINIMAL
     case GB200_METRIC_JOHANNSEN: return launch_geom<GB200_METRIC_JOHANNSEN>(P, sm_count, stream, blocks_out);
     case GB200_METRIC_BUMBLEBEE: return launch_geom<GB200_METRIC_BUMBLEBEE>(P, sm_count, stream, blocks_out);
     case GB200_METRIC_KERR_NEWMAN: return launch_geom<GB200_METRIC_KERR_NEWMAN>(P, sm_count, stream, blocks_out);
     case GB200_METRIC_MORRIS_THORNE: return launch_geom<GB200_METRIC_MORRIS_THORNE>(P, sm_count, stream, blocks_out);
     case GB200_METRIC_DILATON_AXION: return launch_geom<GB200_METRIC_DILATON_AXION>(P, sm_count, stream, blocks_out);
-#endif
     }
     return cudaErrorInvalidValue;
 }

@@ -538,7 +538,7 @@ def test_device_math_against_oracle(ensemble):
     assert out[~nz, 3].max() < -700.0  # log 0: very negative instead of -inf, clamped by the controller all the same
     ex = np.exp(np.clip(x, -8.0, 8.0))
     assert np.max(np.abs(out[:, 4] - ex) / ex) < 1e-15
-    # the pair the controller actually uses (GB_OPT_CTRL_LO): evaluated to the accuracy of the error estimate it acts on
+    # the pair the controller actually uses (gb_log_pos_lo / gb_exp_small_lo): evaluated to the accuracy of the error estimate it acts on
     lo = np.zeros((len(x), 2))
     cabi.check(lib.gb200_debug_math_lo(ctx, len(x), cabi.dptr(x), cabi.dptr(lo.reshape(-1))), ctx)
     assert np.max(np.abs(lo[nz, 0] - lg) / np.maximum(np.abs(lg), 1.0)) < 3e-7

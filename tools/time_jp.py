@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Kernel time of the C5 (Johannsen-Psaltis) and Shakura-Sunyaev renders for the library named by GB200_LIB."""
+"""Kernel time of the C5 (Johannsen-Psaltis), Kerr Shakura-Sunyaev and Kerr no-disc renders."""
 import math, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -16,4 +16,4 @@ for name, m, d in [("JP", gb.JohannsenPsaltisMetric(1.0, 0.6, 2.0), None), ("Ker
         if d == "none": gb.rendergeodesics(m, x, 2000.0, image_width=2048, image_height=2048, ensemble=ens)
         else: gb.rendergeodesics(m, x, gb.ShakuraSunyaev(m) if d == "ss" else d, 2000.0, pf=pf, image_width=2048, image_height=2048, ensemble=ens)
         best = min(best, ens.stats().kernel_ms)
-    print(f"{os.environ.get('GB200_LIB','default'):36s} {name:10s} kernel {best:.2f} ms")
+    print(f"{name:10s} kernel {best:.2f} ms")
