@@ -42,6 +42,7 @@ from .api import (  # noqa: F401
     TracingConfiguration,
     EndpointCache,
     HostPointFunction,
+    ImageOrder,
     apply,
     apply_point_functions,
     apply_point_functions_batch,

@@ -18,11 +18,13 @@ STATUS_OUT_OF_DOMAIN, STATUS_WITHIN_INNER_BOUNDARY, STATUS_INTERSECTED, STATUS_N
 METRIC_KERR, METRIC_JP, METRIC_JOHANNSEN, METRIC_BUMBLEBEE, METRIC_KERR_NEWMAN, METRIC_MORRIS_THORNE, METRIC_DILATON_AXION = 0, 1, 2, 3, 4, 5, 6
 GEOMETRY_NONE, GEOMETRY_THIN_DISC, GEOMETRY_SHAKURA_SUNYAEV, GEOMETRY_DATUM_PLANE, GEOMETRY_THICK_TABLE = 0, 1, 2, 3, 4
 GEOMETRY_TARGET_POINT = 5  # gb200_trace_target only
+GEOMETRY_THIN_DISC_ORDER = 6  # ImageOrder(ThinDisc, n): params inner_radius, outer_radius, n
 CALLBACK_NONE, CALLBACK_UPPER_HEMISPHERE = 0, 1
 POW_EXACT, POW_FAST32 = 0, 1
 IC_RENDER_GRID, IC_POLAR_PLANE, IC_EXPLICIT, IC_CARTESIAN_PLANE, IC_IMPACT_PARAMETERS = 0, 1, 2, 3, 4
 GRID_LINEAR, GRID_GEOMETRIC, GRID_INVERSE = 0, 1, 2
 PF_SHADOW, PF_REDSHIFT, PF_DISC_RADIUS, PF_COORDINATE_TIME, PF_STATUS, PF_AFFINE_TIME, PF_RADIUS = 0, 1, 2, 3, 4, 5, 6
+PF_EQUATORIAL_CROSSINGS = 7
 EMISSIVITY_POWERLAW, EMISSIVITY_TABLE = 0, 1
 FLAG_MAXITERS, FLAG_DT_MIN, FLAG_UNSTABLE = 1, 2, 4
 

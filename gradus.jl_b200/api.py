@@ -332,7 +332,36 @@ class PolishDoughnut(ThickDisc):
         return np.where((rho >= self.inner_radius) & (rho <= self.rho[-1]), np.interp(rho, self.rho, self.height), 0.0)
 
 
-_SUPPORTED_GEOMETRY = (ThinDisc, ShakuraSunyaev, DatumPlane, ThickDisc)
+@dataclass(frozen=True)
+class ImageOrder:
+    """`ImageOrder(disc, n)`: the order-n image of a thin disc (n = 0 the direct image, 1 and 2 the first subrings).
+    A ray hits it at its first entry into the disc's wedge in a step that starts with n equatorial crossings (see
+    `ConstPointFunctions.equatorial_crossings`); entries before that pass through, and once the count exceeds n the disc
+    is inert.  A ray that hits `disc` with c crossings gives the same end point under `ImageOrder(disc, c)`.  Not a type
+    of the reference: GB200_GEOMETRY_THIN_DISC_ORDER of include/gradus_b200.h."""
+
+    disc: ThinDisc
+    n: int
+
+    def __post_init__(self):
+        if type(self.disc) is not ThinDisc:
+            raise ValueError("ImageOrder is defined for a ThinDisc only")
+        if isinstance(self.n, bool) or not isinstance(self.n, (int, np.integer)) or self.n < 0:
+            raise ValueError("ImageOrder needs a non-negative integer order n")
+
+    @property
+    def inner_radius(self):
+        return self.disc.inner_radius
+
+    @property
+    def outer_radius(self):
+        return self.disc.outer_radius
+
+    def to_c(self):
+        return cabi.GEOMETRY_THIN_DISC_ORDER, (float(self.disc.inner_radius), float(self.disc.outer_radius), float(self.n), 0.0)
+
+
+_SUPPORTED_GEOMETRY = (ThinDisc, ShakuraSunyaev, DatumPlane, ThickDisc, ImageOrder)
 
 
 # --------------------------------------------------------------------------- charts and callbacks
@@ -971,6 +1000,8 @@ class PointFunction:
             ("status", None): cabi.PF_STATUS,
             ("affine_time", None): cabi.PF_AFFINE_TIME,
             ("radius", None): cabi.PF_RADIUS,
+            ("equatorial_crossings", None): cabi.PF_EQUATORIAL_CROSSINGS,
+            ("equatorial_crossings", "intersected"): cabi.PF_EQUATORIAL_CROSSINGS,  # filtered on the host, see apply_point_functions
         }
         key = (self.name, self.filter)
         if key not in table:
@@ -1014,6 +1045,35 @@ class ConstPointFunctions:
     def coordinate_time():
         return PointFunction("coordinate_time")
 
+    @staticmethod
+    def equatorial_crossings():
+        """The number of accepted integrator steps whose start and end differ in the sign of cos θ (GB200_PF_EQUATORIAL_
+        CROSSINGS), unfiltered.  A disc hit reports the count at the start of its event step, so
+        `equatorial_crossings() @ filter_intersected()` is the image order of each hit.  ThinDisc, ImageOrder or no
+        geometry only."""
+        return PointFunction("equatorial_crossings")
+
+
+def _filter_on_host(pfs, kinds):
+    """Point functions with no device filter of their own (the crossing count composed with `filter_intersected`):
+    the status joins the device's list and the host masks the rays that did not hit.  Returns (device kinds, mask)."""
+    masked = [k for k, f in enumerate(pfs) if (f.name, f.filter) == ("equatorial_crossings", "intersected")]
+    if not masked:
+        return kinds, None
+    if len(kinds) >= 4:  # GB_MAX_PF
+        raise ValueError("equatorial_crossings() @ filter_intersected() needs a free point-function slot (at most 3 others)")
+    return np.append(kinds, np.int32(cabi.PF_STATUS)), masked
+
+
+def _apply_host_filter(images, masked):
+    if masked is None:
+        return images
+    miss = images[-1] != cabi.STATUS_INTERSECTED
+    out = images[:-1].copy()
+    for k in masked:
+        out[k][miss] = np.nan
+    return out
+
 
 def impact_axes(width, height, alpha_lims, beta_lims):
     """src/rendering/utility.jl:43-47"""
@@ -1031,10 +1091,10 @@ def apply_point_functions(config, pfs, plunging=None):
     """Trace every ray of `config` and evaluate the point functions `pfs` at its endpoint in the same kernel
     (the fused form of `apply(pf, rendergeodesics(...))`, src/rendering/rendering.jl:64-107, for any velocity source
     including `ImpactParameters`).  Returns an array of shape (len(pfs), n_rays)."""
-    kinds = np.array([f.kind() for f in pfs], np.int32)
+    kinds, masked = _filter_on_host(pfs, np.array([f.kind() for f in pfs], np.int32))
     p, ic = config.to_c()
     n = ic.n
-    images = np.zeros((len(pfs), n))
+    images = np.zeros((len(kinds), n))
     lib = cabi.load()
     plunging = _auto_plunging(config.metric, config.geometry, config.ensemble, cabi.PF_REDSHIFT in kinds, plunging)
     pl_ref = C.byref(plunging.c) if plunging is not None else None
@@ -1042,17 +1102,17 @@ def apply_point_functions(config, pfs, plunging=None):
     comm = config.ensemble.comm()
     if comm is not None:  # several GPUs: strips interleaved over the devices inside the library
         _install_on_comm(comm, config.geometry)
-        ptrs = (cabi._dp * len(pfs))(*[cabi.dptr(images[k]) for k in range(len(pfs))])
-        cabi.check(lib.gb200_comm_render(comm, C.byref(p), C.byref(ic), cabi.iptr(kinds), len(pfs), pl_ref, ptrs))
-        return images
+        ptrs = (cabi._dp * len(kinds))(*[cabi.dptr(images[k]) for k in range(len(kinds))])
+        cabi.check(lib.gb200_comm_render(comm, C.byref(p), C.byref(ic), cabi.iptr(kinds), len(kinds), pl_ref, ptrs))
+        return _apply_host_filter(images, masked)
 
     def fn(ctx, first, count, slot):
-        ptrs = (cabi._dp * len(pfs))(*[C.cast(images[k].ctypes.data + 8 * first, cabi._dp) for k in range(len(pfs))])
+        ptrs = (cabi._dp * len(kinds))(*[C.cast(images[k].ctypes.data + 8 * first, cabi._dp) for k in range(len(kinds))])
         rng = cabi.Range(first, count, 1)
-        cabi.check(lib.gb200_render(ctx, C.byref(p), C.byref(ic), C.byref(rng), cabi.iptr(kinds), len(pfs), pl_ref, ptrs), ctx)
+        cabi.check(lib.gb200_render(ctx, C.byref(p), C.byref(ic), C.byref(rng), cabi.iptr(kinds), len(kinds), pl_ref, ptrs), ctx)
 
     _run_sharded(config.ensemble, n, fn, config.geometry)
-    return images
+    return _apply_host_filter(images, masked)
 
 
 def apply_point_functions_batch(configs: Sequence[TracingConfiguration], pfs, plungings=None) -> list:
@@ -1061,8 +1121,8 @@ def apply_point_functions_batch(configs: Sequence[TracingConfiguration], pfs, pl
     configuration.  Used by the transfer-function table, where every probe round spans all (a, θ) cells."""
     if not configs:
         return []
-    kinds = np.array([f.kind() for f in pfs], np.int32)
-    npf, nb = len(pfs), len(configs)
+    kinds, masked = _filter_on_host(pfs, np.array([f.kind() for f in pfs], np.int32))
+    npf, nb = len(kinds), len(configs)
     ens = configs[0].ensemble
     pcs = [c.to_c() for c in configs]
     problems = (cabi.Problem * nb)(*[pc[0] for pc in pcs])
@@ -1076,7 +1136,7 @@ def apply_point_functions_batch(configs: Sequence[TracingConfiguration], pfs, pl
         pl_ptrs = (PT * nb)(*[C.pointer(p.c) if p is not None else PT() for p in plungings])
     ctx = ens.ctx(ens.devices[0])
     cabi.check(cabi.load().gb200_render_batch(ctx, nb, problems, ics, ranges, cabi.iptr(kinds), npf, pl_ptrs, ptrs), ctx)
-    return images
+    return [_apply_host_filter(im, masked) for im in images]
 
 
 def rendergeodesics(m, position, *args, pf=None, image_width=375, image_height=250, ensemble=None, plunging=None, **kwargs):

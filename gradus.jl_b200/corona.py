@@ -237,6 +237,8 @@ def _intersected(gps):
 def tracecorona(m, d, model, *, lambda_max=10_000.0, n_samples=1024, sampler=None, callback="default", ensemble=None,
                 solver=None, **kwargs) -> CoronaGeodesics:
     """`tracecorona(m, g, model; λmax, n_samples, sampler, callback)` (corona-models.jl:164-190)."""
+    if isinstance(d, api.ImageOrder):
+        raise ValueError("geometry ImageOrder is outside the corona models' scope: they trace to the whole disc")
     if sampler is None:
         sampler = EvenSampler("both", "golden")
     if callback == "default":

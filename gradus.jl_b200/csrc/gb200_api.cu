@@ -163,10 +163,15 @@ static int validate(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic) 
         return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "Dilaton-Axion metric with beta != 0 needs a != 0 and b != 0 (beta / a, beta / b; dilaton-axion-ad.jl:24-26)");
     if (p->metric_kind == GB200_METRIC_KERR_NEWMAN && a * a + p->metric_params[2] * p->metric_params[2] > M * M)
         return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "Kerr-Newman metric needs a^2 + Q^2 <= M^2 (kerr-newman-ad.jl:50-52)");
-    if (p->geometry_kind < GB200_GEOMETRY_NONE || p->geometry_kind > GB200_GEOMETRY_THICK_TABLE)
+    if ((p->geometry_kind < GB200_GEOMETRY_NONE || p->geometry_kind > GB200_GEOMETRY_THICK_TABLE) && p->geometry_kind != GB200_GEOMETRY_THIN_DISC_ORDER)
         return fail(ctx, GB200_ERR_UNSUPPORTED, "geometry kind %d is outside the hot-path scope", p->geometry_kind);
-    if (p->geometry_kind == GB200_GEOMETRY_THIN_DISC && !(p->geometry_params[0] <= p->geometry_params[1]))
+    if ((p->geometry_kind == GB200_GEOMETRY_THIN_DISC || p->geometry_kind == GB200_GEOMETRY_THIN_DISC_ORDER) && !(p->geometry_params[0] <= p->geometry_params[1]))
         return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "ThinDisc needs inner_radius <= outer_radius");
+    if (p->geometry_kind == GB200_GEOMETRY_THIN_DISC_ORDER) {
+        const double n = p->geometry_params[2];
+        if (!(n >= 0.0 && n <= 2147483647.0 && n == std::floor(n)))
+            return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "ImageOrder needs a non-negative integer order below 2^31 (got %g)", n);
+    }
     if (p->callback_kind != GB200_CALLBACK_NONE && p->callback_kind != GB200_CALLBACK_UPPER_HEMISPHERE)
         return fail(ctx, GB200_ERR_UNSUPPORTED, "callback kind %d cannot run on the device", p->callback_kind);
     if (p->pow_mode != GB200_POW_EXACT && p->pow_mode != GB200_POW_FAST32) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad pow_mode");
@@ -196,6 +201,25 @@ static int validate(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic) 
         for (int k = 0; k < 4; ++k)
             if (!ic->x[k] || !ic->v[k]) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "explicit IC pointers must be non-null");
     } else return fail(ctx, GB200_ERR_UNSUPPORTED, "ic kind %d", ic->kind);
+    return GB200_OK;
+}
+
+// The image order is a rule of the throughput kernel's event handling; the generic (forward-mode, target, path) integrator
+// does not have it.  Checked before the context, like validate_crossings.
+static int reject_image_order(gb200_ctx* ctx, const gb200_problem* p, const char* entry) {
+    if (p && p->geometry_kind == GB200_GEOMETRY_THIN_DISC_ORDER)
+        return fail(ctx, GB200_ERR_UNSUPPORTED, "%s does not support GB200_GEOMETRY_THIN_DISC_ORDER", entry);
+    return GB200_OK;
+}
+
+// GB200_PF_EQUATORIAL_CROSSINGS is counted with no geometry and on the thin disc only.  Checked before anything else (a
+// device context included), so that callers can probe it without a GPU.
+static int validate_crossings(gb200_ctx* ctx, const gb200_problem* p, const int32_t* pfs, int npf) {
+    if (!p || !pfs) return GB200_OK;
+    for (int k = 0; k < npf && k < GB_MAX_PF; ++k)
+        if (pfs[k] == GB200_PF_EQUATORIAL_CROSSINGS && p->geometry_kind != GB200_GEOMETRY_NONE && p->geometry_kind != GB200_GEOMETRY_THIN_DISC &&
+            p->geometry_kind != GB200_GEOMETRY_THIN_DISC_ORDER)
+            return fail(ctx, GB200_ERR_UNSUPPORTED, "GB200_PF_EQUATORIAL_CROSSINGS needs geometry NONE, THIN_DISC or THIN_DISC_ORDER (got %d)", p->geometry_kind);
     return GB200_OK;
 }
 
@@ -695,6 +719,7 @@ int gb200_trace(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic, cons
 
 int gb200_trace_target(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic, const gb200_range* rg, const double* target, double d_tol,
                        gb200_endpoints* out, double* closest) {
+    { int rc_ = reject_image_order(ctx, p, "gb200_trace_target"); if (rc_) return rc_; }
     if (!target) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null target");
     return trace_common(ctx, p, ic, rg, out, target, d_tol, closest);
 }
@@ -822,6 +847,7 @@ int gb200_trace_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* probl
 
 int gb200_trace_path(gb200_ctx* ctx, const gb200_problem* p, const double* u0, int32_t cap, double* lambda, double* u,
                      int32_t* nrows, int32_t* status) {
+    { int rc_ = reject_image_order(ctx, p, "gb200_trace_path"); if (rc_) return rc_; }
     if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
     if (!p || !u0 || cap < 1 || !lambda || !u || !nrows || !status) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad path arguments");
     gb200_ic ic{};
@@ -905,12 +931,13 @@ int gb200_build_plunging_table(gb200_ctx* ctx, int32_t metric_kind, const double
 
 static int render_common(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic, const gb200_range* rg, const int32_t* pfs, int32_t npf,
                          const gb200_plunging_table* pl, double* const* images, bool device_out, cudaStream_t stream, int async) {
+    { int rc_ = validate_crossings(ctx, p, pfs, npf); if (rc_) return rc_; }
     if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
     int rc = validate(ctx, p, ic); if (rc) return rc;
     rc = validate_range(ctx, ic, rg); if (rc) return rc;
     if (npf < 1 || npf > GB_MAX_PF || !pfs || !images) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 1..%d point functions", GB_MAX_PF);
     for (int k = 0; k < npf; ++k) {
-        if (pfs[k] < GB200_PF_SHADOW || pfs[k] > GB200_PF_RADIUS) return fail(ctx, GB200_ERR_UNSUPPORTED, "point function %d", pfs[k]);
+        if (pfs[k] < GB200_PF_SHADOW || pfs[k] > GB200_PF_EQUATORIAL_CROSSINGS) return fail(ctx, GB200_ERR_UNSUPPORTED, "point function %d", pfs[k]);
         if (!images[k]) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null image pointer");
     }
     { int rc_ = begin_call(ctx, stream); if (rc_) return rc_; }
@@ -960,11 +987,13 @@ int gb200_render_device(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* 
 
 int gb200_render_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* problems, const gb200_ic* ics, const gb200_range* ranges,
                        const int32_t* pfs, int32_t npf, const gb200_plunging_table* const* pls, double* const* images) {
+    if (problems)
+        for (int b = 0; b < nbatch; ++b) { int rc_ = validate_crossings(ctx, &problems[b], pfs, npf); if (rc_) return rc_; }
     if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
     if (nbatch < 1 || !problems || !ics || !ranges || !pfs || !images) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad batch arguments");
     if (npf < 1 || npf > GB_MAX_PF) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 1..%d point functions", GB_MAX_PF);
     for (int k = 0; k < npf; ++k)
-        if (pfs[k] < GB200_PF_SHADOW || pfs[k] > GB200_PF_RADIUS) return fail(ctx, GB200_ERR_UNSUPPORTED, "point function %d", pfs[k]);
+        if (pfs[k] < GB200_PF_SHADOW || pfs[k] > GB200_PF_EQUATORIAL_CROSSINGS) return fail(ctx, GB200_ERR_UNSUPPORTED, "point function %d", pfs[k]);
     for (int b = 0; b < nbatch; ++b) {
         int rc = validate(ctx, &problems[b], &ics[b]); if (rc) return rc;
         rc = validate_range(ctx, &ics[b], &ranges[b]); if (rc) return rc;
@@ -1073,6 +1102,8 @@ int gb200_render_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* prob
 // ---------------------------------------------------------------- forward-mode traces (gb200_dual.cu)
 int gb200_trace_dual_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* problems, const gb200_dual_ic* ics, int32_t norm_mode,
                            const gb200_plunging_table* const* pls, gb200_dual_out* outs) {
+    if (problems)
+        for (int b = 0; b < nbatch; ++b) { int rc_ = reject_image_order(ctx, &problems[b], "gb200_trace_dual"); if (rc_) return rc_; }
     if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
     if (nbatch < 1 || !problems || !ics || !outs) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad batch arguments");
     if (norm_mode != GB200_DUAL_NORM_WITH_PARTIALS && norm_mode != GB200_DUAL_NORM_VALUES_ONLY) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad norm_mode");
@@ -1220,6 +1251,7 @@ int gb200_trace_dual_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* 
 
 int gb200_trace_dual(gb200_ctx* ctx, const gb200_problem* p, const gb200_dual_ic* ic, int32_t norm_mode,
                      const gb200_plunging_table* plunging, gb200_dual_out* out) {
+    { int rc_ = reject_image_order(ctx, p, "gb200_trace_dual"); if (rc_) return rc_; }
     if (!p || !ic || !out) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null argument");
     const gb200_plunging_table* pls[1] = {plunging};
     return gb200_trace_dual_batch(ctx, 1, p, ic, norm_mode, pls, out);

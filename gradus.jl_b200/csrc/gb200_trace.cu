@@ -143,8 +143,21 @@ __device__ __noinline__ void gb_hist_add(const GbParams& P, unsigned long long* 
     gb_acc128(&sh_hist[bin], &sh_hist[P.lp_nbins + bin], wlo, whi);
 }
 
+// Equatorial crossings (GB200_PF_EQUATORIAL_CROSSINGS) are counted only by instantiations that need them: GEOM is then a
+// public geometry kind plus GB_GEOM_COUNTING (NONE and THIN_DISC), or GB200_GEOMETRY_THIN_DISC_ORDER, which always counts.
+// Every other instantiation compiles exactly the code it had before the counter existed.
+constexpr int GB_GEOM_COUNTING = 16;
+template <int GEOM> GB_HD constexpr bool gb_counts() { return GEOM >= GB_GEOM_COUNTING || GEOM == GB200_GEOMETRY_THIN_DISC_ORDER; }
+// the disc whose condition the kernel evaluates: the order-n image is the thin disc's wedge
+template <int GEOM> GB_HD constexpr int gb_disc_kind() {
+    return GEOM == GB200_GEOMETRY_THIN_DISC_ORDER ? GB200_GEOMETRY_THIN_DISC : (GEOM >= GB_GEOM_COUNTING ? GEOM - GB_GEOM_COUNTING : GEOM);
+}
+
 template <int METRIC, int GEOM>
 __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(const __grid_constant__ GbParams P) {
+    constexpr bool COUNT = gb_counts<GEOM>();
+    constexpr bool ORDER = GEOM == GB200_GEOMETRY_THIN_DISC_ORDER;
+    constexpr int DISC = gb_disc_kind<GEOM>();
     const unsigned lane = threadIdx.x & 31u;
     const double abstol = P.abstol, reltol = P.reltol;
     const double tstop = P.lam1;
@@ -171,6 +184,10 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
     const int maxit = (int)(P.maxiters < 0x7fffffff ? P.maxiters : 0x7fffffff); // step attempts are counted in 32 bits
     bool exhausted = false;
     unsigned long long tot_acc = 0, tot_rej = 0, tot_flag = 0;
+    // COUNT: equatorial crossings of the accepted steps so far and the sign of cos(theta) at u_prev; ORDER: the image order
+    int crossings = 0;
+    bool cpos_prev = true;
+    const int order = ORDER ? (int)P.gp2 : 0;
     // k2..k6 of the four accelerations and of the r, theta stage velocities: 30 rows; rows 30..33 park the k7
     // accelerations of a lane whose step ended in a disc event until it is finalised.
     __shared__ double sh_k[34][GB_BLOCK];
@@ -204,7 +221,7 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
             // ================= finalise terminated lanes =================
             if (state == LANE_PENDING) {
                 int status = pend_status;
-                if (GEOM != GB200_GEOMETRY_NONE && pend_event) {
+                if (DISC != GB200_GEOMETRY_NONE && pend_event) {
                     kA0.k7 = sh_k[30][threadIdx.x]; kA1.k7 = sh_k[31][threadIdx.x]; kA2.k7 = sh_k[32][threadIdx.x]; kA3.k7 = sh_k[33][threadIdx.x];
                     // ContinuousCallback root find on the dense output (DiffEqBase find_callback_time, LeftRootFind)
                     double C2r, C3r, C4r, C2t, C3t, C4t;
@@ -217,10 +234,10 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                         double s_, c_;
                         if (lo > 0.0) {
                             gb_sincos(dense_eval(th, dt, lo, vth, C2t, C3t, C4t), &s_, &c_);
-                            flo = disc_condition<GEOM>(P, dense_eval(r, dt, lo, vr, C2r, C3r, C4r), s_, c_, hgt);
+                            flo = disc_condition<DISC>(P, dense_eval(r, dt, lo, vr, C2r, C3r, C4r), s_, c_, hgt);
                         } else flo = cprev;
                         gb_sincos(dense_eval(th, dt, hi, vth, C2t, C3t, C4t), &s_, &c_);
-                        fhi = disc_condition<GEOM>(P, dense_eval(r, dt, hi, vr, C2r, C3r, C4r), s_, c_, hgt);
+                        fhi = disc_condition<DISC>(P, dense_eval(r, dt, hi, vr, C2r, C3r, C4r), s_, c_, hgt);
                     }
                     if (fhi == 0.0) lo = hi;
                     else {
@@ -235,7 +252,7 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                             if (!(mid > lo && mid < hi)) break;
                             double s_, c_;
                             gb_sincos(dense_eval(th, dt, mid, vth, C2t, C3t, C4t), &s_, &c_);
-                            const double fm = disc_condition<GEOM>(P, dense_eval(r, dt, mid, vr, C2r, C3r, C4r), s_, c_, hgt);
+                            const double fm = disc_condition<DISC>(P, dense_eval(r, dt, mid, vr, C2r, C3r, C4r), s_, c_, hgt);
                             if (fm != 0.0 && (fm > 0.0) == (sprev > 0.0)) {
                                 lo = mid; flo = fm;
                                 if (side == -1) fhi *= 0.5;
@@ -315,6 +332,7 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                         else if (pf == GB200_PF_STATUS) val = (double)status;
                         else if (pf == GB200_PF_AFFINE_TIME) val = tfinal;
                         else if (pf == GB200_PF_RADIUS) val = xe[1] * fabs(sin(xe[2]));
+                        else if (COUNT && pf == GB200_PF_EQUATORIAL_CROSSINGS) val = (double)crossings;
                         P.o_img[k][n] = val;
                     }
                     if (P.o_g || P.lp_bins) { // lineprofile BinningMethod, src/line-profiles.jl:186-194
@@ -349,7 +367,7 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                         lam = P.lam0; ct = ri.x[0]; r = ri.x[1]; th = ri.x[2]; ph = ri.x[3];
                         vt = ri.v[0]; vr = ri.v[1]; vth = ri.v[2]; vph = ri.v[3];
                         area = ri.area;
-                        if (GEOM == GB200_GEOMETRY_DATUM_PLANE && P.ic_kind == GB200_IC_IMPACT_PARAMETERS && P.ex[2])
+                        if (DISC == GB200_GEOMETRY_DATUM_PLANE && P.ic_kind == GB200_IC_IMPACT_PARAMETERS && P.ex[2])
                             hgt = P.ex[2][ray_index_of_slot(P, s)];
 #pragma unroll
                         for (int k = 0; k < 4; ++k) { // GeodesicPoint.x_init / v_init are known now
@@ -367,8 +385,9 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                         // f0 and the Hairer-Wanner initial step (ode_determine_initdt)
                         double acc[4], s_, c_;
                         rhs_accel<METRIC>(P, r, th, vt, vr, vth, vph, acc, s_, c_);
-                        if (GEOM != GB200_GEOMETRY_NONE) cprev = disc_condition<GEOM>(P, r, s_, c_, hgt);
+                        if (DISC != GB200_GEOMETRY_NONE) cprev = disc_condition<DISC>(P, r, s_, c_, hgt);
                         acos_prev = fabs(c_);
+                        if (COUNT) { crossings = 0; cpos_prev = c_ >= 0.0; }
                         const double u0[8] = {ct, r, th, ph, vt, vr, vth, vph};
                         const double f0[8] = {vt, vr, vth, vph, acc[0], acc[1], acc[2], acc[3]};
                         double sk[8], d0 = 0, d1 = 0;
@@ -517,10 +536,12 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
             // ---- callbacks: continuous (disc) first, then discrete (user, chart)
             bool event = false;
             double cnext = 1.0;
-            if (GEOM != GB200_GEOMETRY_NONE) {
-                cnext = disc_condition<GEOM>(P, nr, s_, c_, hgt);
+            if (DISC != GB200_GEOMETRY_NONE) {
+                cnext = disc_condition<DISC>(P, nr, s_, c_, hgt);
                 const double sprev = sgn(cprev);
-                if (accept && sprev != 0.0) {
+                // the order-n image: only an entry into the wedge (sprev > 0) in a step that starts with n crossings is an
+                // event; inside the wedge, before the n-th crossing and after it, the event test and the scan are skipped
+                if (accept && (ORDER ? (sprev > 0.0 && crossings == order) : sprev != 0.0)) {
                     if (sprev * sgn(cnext) <= 0.0) { event = true; ev_lo = 0.0; ev_hi = 1.0; }
                     else {
                         // cheap bound first: |u(Th) - u0| <= |dt| * L * max_j |k_j| with L = max_Th sum_j |b_j(Th)| = 7.5822
@@ -531,14 +552,14 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                         // which the comparisons in scan_needed treat as "cannot skip".
                         const double mth = __hiloint2double(max(mxt, __double2hiint(nvth) & 0x7fffffff) + 1, 0);
                         const double mr = __hiloint2double(max(mxr, __double2hiint(nvr) & 0x7fffffff) + 1, 0);
-                        bool need = sprev < 0.0 || scan_needed<GEOM>(P, r, acos_prev, cprev, adt * 7.5823 * mth, adt * 7.5823 * mr);
+                        bool need = (!ORDER && sprev < 0.0) || scan_needed<DISC>(P, r, acos_prev, cprev, adt * 7.5823 * mth, adt * 7.5823 * mr);
                         double C2r = 0, C3r = 0, C4r = 0, C2t = 0, C3t = 0, C4t = 0;
                         if (need) {
                             dense_coeffs(vth, kT, nvth, C2t, C3t, C4t);
                             dense_coeffs(vr, kR, nvr, C2r, C3r, C4r);
                             const double Bth = adt * (fabs(vth) + fabs(C2t) + fabs(C3t) + fabs(C4t));
                             const double Br = adt * (fabs(vr) + fabs(C2r) + fabs(C3r) + fabs(C4r));
-                            need = sprev < 0.0 || scan_needed<GEOM>(P, r, acos_prev, cprev, Bth, Br);
+                            need = (!ORDER && sprev < 0.0) || scan_needed<DISC>(P, r, acos_prev, cprev, Bth, Br);
                         }
                         if (need) {
 #pragma unroll 1
@@ -546,14 +567,14 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                                 const double Th = (double)i / 7.0;
                                 double si, ci;
                                 gb_sincos(dense_eval(th, dt, Th, vth, C2t, C3t, C4t), &si, &ci);
-                                const double cn = disc_condition<GEOM>(P, dense_eval(r, dt, Th, vr, C2r, C3r, C4r), si, ci, hgt);
+                                const double cn = disc_condition<DISC>(P, dense_eval(r, dt, Th, vr, C2r, C3r, C4r), si, ci, hgt);
                                 if (sprev * cn < 0.0) { event = true; ev_lo = (double)(i - 1) / 7.0; ev_hi = Th; break; }
                             }
                         }
                     }
                 }
             }
-            if (GEOM != GB200_GEOMETRY_NONE && event) { // k2..k6 are in shared memory already; k7 joins them
+            if (DISC != GB200_GEOMETRY_NONE && event) { // k2..k6 are in shared memory already; k7 joins them
                 sh_k[30][threadIdx.x] = kA0.k7; sh_k[31][threadIdx.x] = kA1.k7; sh_k[32][threadIdx.x] = kA2.k7; sh_k[33][threadIdx.x] = kA3.k7;
             }
             int status = GB200_STATUS_NO_STATUS;
@@ -582,6 +603,11 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
             kA0.set(0, advance ? kA0.get(6) : kA0.get(0)); kA1.set(0, advance ? kA1.get(6) : kA1.get(0));
             kA2.set(0, advance ? kA2.get(6) : kA2.get(0)); kA3.set(0, advance ? kA3.get(6) : kA3.get(0));
             cprev = advance ? cnext : cprev; acos_prev = advance ? fabs(c_) : acos_prev;
+            if (COUNT) { // every accepted step counts except one that ends in a disc event (the ray stops at u_prev + a root)
+                const bool cpos = c_ >= 0.0;
+                crossings += (accept && !event && cpos != cpos_prev) ? 1 : 0;
+                cpos_prev = advance ? cpos : cpos_prev;
+            }
             dt = advance ? dtprop : (accept ? dt : dtrej);
         }
     }
@@ -624,9 +650,17 @@ static cudaError_t launch_one(const GbParams& P, int sm_count, cudaStream_t stre
 
 template <int METRIC>
 static cudaError_t launch_geom(const GbParams& P, int sm_count, cudaStream_t stream, int* blocks_out) {
+    bool count = false; // the counting instantiations run only for calls that ask for the crossings
+    for (int k = 0; k < P.npf; ++k) count = count || P.pf[k] == GB200_PF_EQUATORIAL_CROSSINGS;
+    if (count && P.geometry_kind == GB200_GEOMETRY_NONE)
+        return launch_one<METRIC, GB200_GEOMETRY_NONE + GB_GEOM_COUNTING>(P, sm_count, stream, blocks_out);
+    if (count && P.geometry_kind == GB200_GEOMETRY_THIN_DISC)
+        return launch_one<METRIC, GB200_GEOMETRY_THIN_DISC + GB_GEOM_COUNTING>(P, sm_count, stream, blocks_out);
+    if (count && P.geometry_kind != GB200_GEOMETRY_THIN_DISC_ORDER) return cudaErrorInvalidValue; // the host rejects this first
     switch (P.geometry_kind) {
     case GB200_GEOMETRY_NONE: return launch_one<METRIC, GB200_GEOMETRY_NONE>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_THIN_DISC: return launch_one<METRIC, GB200_GEOMETRY_THIN_DISC>(P, sm_count, stream, blocks_out);
+    case GB200_GEOMETRY_THIN_DISC_ORDER: return launch_one<METRIC, GB200_GEOMETRY_THIN_DISC_ORDER>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_SHAKURA_SUNYAEV: return launch_one<METRIC, GB200_GEOMETRY_SHAKURA_SUNYAEV>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_DATUM_PLANE: return launch_one<METRIC, GB200_GEOMETRY_DATUM_PLANE>(P, sm_count, stream, blocks_out);
     case GB200_GEOMETRY_THICK_TABLE: return launch_one<METRIC, GB200_GEOMETRY_THICK_TABLE>(P, sm_count, stream, blocks_out);

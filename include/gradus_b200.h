@@ -68,6 +68,22 @@ extern "C" {
 
 #define GB200_GEOMETRY_TARGET_POINT 5    /* gb200_trace_target only: the distance ContinuousCallback of _make_target_objective,
                                             src/tracing/precision-solvers.jl:473-488 */
+#define GB200_GEOMETRY_THIN_DISC_ORDER 6 /* ImageOrder(ThinDisc(r_in, r_out), n): the order-n image of the thin disc.
+                                            params: inner_radius, outer_radius, n (a non-negative integer stored as a double,
+                                            at most 2^31 - 1; anything else is GB200_ERR_INVALID_ARGUMENT).  The wedge, its
+                                            condition and gtol are GB200_GEOMETRY_THIN_DISC's; only the events differ:
+                                              - an entry into the wedge (condition positive -> non-positive) in a step that starts
+                                                with n equatorial crossings (GB200_PF_EQUATORIAL_CROSSINGS) is an event, handled
+                                                exactly as a ThinDisc event (root find, discrete callbacks on the event state,
+                                                IntersectedWithGeometry);
+                                              - an entry in a step that starts with fewer crossings is passed through (an
+                                                ordinary accepted step); exits from the wedge are never events;
+                                              - once the count exceeds n the disc is inert: the ray ends at its chart, lambda_max
+                                                or callback and is not a hit (its n-th crossing fell outside [r_in, r_out]).
+                                            A ray that hits GB200_GEOMETRY_THIN_DISC with count c takes the same steps and the same
+                                            event step under order c.  Accepted by gb200_trace*, gb200_render*, gb200_lineprofile*
+                                            and gb200_comm_*; gb200_trace_dual*, gb200_trace_target and gb200_trace_path return
+                                            GB200_ERR_UNSUPPORTED */
 
 /* ---- user discrete callback: src/tracing/callbacks.jl:31-39 ------------ */
 #define GB200_CALLBACK_NONE 0
@@ -180,6 +196,13 @@ typedef struct gb200_endpoints {
 #define GB200_PF_AFFINE_TIME 5     /* lambda_max, no filter */
 #define GB200_PF_RADIUS 6          /* r |sin(theta)| of the end point whatever its status (ConstPointFunctions.radius,
                                       src/const-point-functions.jl; the offset root finder reads it, precision-solvers.jl:124) */
+#define GB200_PF_EQUATORIAL_CROSSINGS 7 /* equatorial crossings of the ray, as a double, no filter: the number of accepted steps
+                                      whose start and end states differ in the sign of cos(theta) (cos(theta) >= 0 counts as
+                                      positive), from 0 at the initial state, up to and including the step that ends the ray at
+                                      its chart, lambda_max or a discrete callback.  A step that ends in a disc event does not
+                                      count: a hit reports the count at the start of its event step.  Geometry NONE, THIN_DISC
+                                      and THIN_DISC_ORDER only; any other geometry is GB200_ERR_UNSUPPORTED (in gb200_render,
+                                      gb200_render_batch, gb200_render_device and gb200_comm_render) */
 
 /* ---- emissivity for the binned line profile ---------------------------- */
 #define GB200_EMISSIVITY_POWERLAW 0 /* eps(r) = r^(-index) */

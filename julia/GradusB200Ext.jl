@@ -118,6 +118,25 @@ _geometry(::Nothing) = (Int32(0), (0.0, 0.0, 0.0, 0.0))
 _geometry(d::ThinDisc) = (Int32(1), (Float64(d.inner_radius), Float64(d.outer_radius), 0.0, 0.0))
 _geometry(d::ShakuraSunyaev) = (Int32(2), (Float64(d.Ṁ_Ṁedd), Float64(d.inv_η), Float64(d.inner_radius), 0.0))
 _geometry(d::DatumPlane) = (Int32(3), (Float64(d.height), 0.0, 0.0, 0.0))
+
+"""
+    ImageOrder(d::ThinDisc, n)
+
+The order-n image of a thin disc (n = 0 the direct image, 1 and 2 the first photon-ring subrings): a ray hits it at its
+first entry into the disc's wedge in a step that starts with n equatorial crossings (`equatorial_crossings()`); earlier
+entries pass through and once the count exceeds n the disc is inert (GB200_GEOMETRY_THIN_DISC_ORDER, include/gradus_b200.h).
+Not a type of the reference: it lives in this extension and goes wherever `EnsembleB200` takes a geometry
+(`tracegeodesics`, `rendergeodesics`, `lineprofile_b200`); the transfer-function and target paths refuse it.
+"""
+struct ImageOrder{D}
+    disc::D
+    n::Int
+    function ImageOrder(d::D, n::Integer) where {D<:ThinDisc}
+        n >= 0 || throw(ArgumentError("ImageOrder needs a non-negative order"))
+        new{D}(d, Int(n))
+    end
+end
+_geometry(d::ImageOrder) = (Int32(6), (Float64(d.disc.inner_radius), Float64(d.disc.outer_radius), Float64(d.n), 0.0))
 # thick discs whose height is a closure (`ThickDisc(f)`, `PolishDoughnut`: src/geometry/discs/thick-disc.jl:32-63,
 # polish-doughnut.jl:102-129) cross the ABI as a table (GB200_GEOMETRY_THICK_TABLE); `_install_geometry` uploads it
 _geometry(d::Gradus.AbstractThickAccretionDisc) = begin
@@ -344,7 +363,7 @@ end
 # ---------------------------------------------------------------------------------------------------------------------
 # fused paths
 """
-    B200PointFunction(:redshift | :radius | :shadow | :coordinate_time | :status | :affine_time | :end_radius)
+    B200PointFunction(:redshift | :radius | :shadow | :coordinate_time | :status | :affine_time | :end_radius | :equatorial_crossings)
 
 A point function the device evaluates at the ray end point inside the trace kernel (include/gradus_b200.h, GB200_PF_*):
 `:redshift` = `ConstPointFunctions.redshift(m, x) ∘ ConstPointFunctions.filter_intersected()`, `:radius` =
@@ -354,8 +373,18 @@ A point function the device evaluates at the ray end point inside the trace kern
 struct B200PointFunction
     kind::Int32
 end
-const _PF_KINDS = Dict(:shadow => 0, :redshift => 1, :radius => 2, :coordinate_time => 3, :status => 4, :affine_time => 5, :end_radius => 6)
+const _PF_KINDS = Dict(:shadow => 0, :redshift => 1, :radius => 2, :coordinate_time => 3, :status => 4, :affine_time => 5, :end_radius => 6,
+                       :equatorial_crossings => 7)
 B200PointFunction(s::Symbol) = B200PointFunction(Int32(_PF_KINDS[s]))
+
+"""
+    equatorial_crossings()
+
+The number of accepted integrator steps whose start and end differ in the sign of cos θ, unfiltered
+(GB200_PF_EQUATORIAL_CROSSINGS); a disc hit reports the count at the start of its event step, i.e. its image order.
+`ThinDisc`, `ImageOrder` or no geometry.  Not a point function of the reference.
+"""
+equatorial_crossings() = B200PointFunction(:equatorial_crossings)
 
 const _B200Config{T} = TracingConfiguration{T,M,P,V,G,C,Ch,S,<:EnsembleB200} where {M,P,V,G,C,Ch,S}
 
@@ -504,5 +533,5 @@ function optimize_for_target_b200(target, m::Gradus.AbstractMetric{T}, x0; ensem
     best[2], best[3], best[4], best[1]
 end
 
-export EnsembleB200, B200PointFunction, lineprofile_b200, optimize_for_target_b200
+export EnsembleB200, B200PointFunction, ImageOrder, equatorial_crossings, lineprofile_b200, optimize_for_target_b200
 end # module
