@@ -223,6 +223,16 @@ static int validate_crossings(gb200_ctx* ctx, const gb200_problem* p, const int3
     return GB200_OK;
 }
 
+// 1..GB_MAX_PF point functions of kinds the kernel evaluates; where `images` is given, a non-null image for each
+static int validate_pfs(gb200_ctx* ctx, const int32_t* pfs, int npf, double* const* images) {
+    if (npf < 1 || npf > GB_MAX_PF || !pfs) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 1..%d point functions", GB_MAX_PF);
+    for (int k = 0; k < npf; ++k) {
+        if (pfs[k] < GB200_PF_SHADOW || pfs[k] > GB200_PF_EQUATORIAL_CROSSINGS) return fail(ctx, GB200_ERR_UNSUPPORTED, "point function %d", pfs[k]);
+        if (images && !images[k]) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null image pointer");
+    }
+    return GB200_OK;
+}
+
 static int validate_range(gb200_ctx* ctx, const gb200_ic* ic, const gb200_range* rg) {
     if (!rg) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null range");
     if (rg->count < 0 || rg->first < 0 || rg->stride < 1 || rg->block < 0) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad range");
@@ -241,6 +251,15 @@ static void dd_step(double lo, double hi, int64_t n, double* shi, double* slo) {
     const long double s = ((long double)hi - (long double)lo) / (long double)(n - 1);
     *shi = (double)s;
     *slo = (double)(s - (long double)*shi);
+}
+
+// Rays per image column (render grid) or theta-row (polar and Cartesian planes): the fastest-varying extent of the ray
+// index, whose multiples of GB_TILE_C make the strips of the tiled work order and of the multi-GPU shards.  0 for ray lists.
+static int64_t strip_height(const gb200_ic* ic) {
+    if (ic->kind == GB200_IC_RENDER_GRID) return ic->height;
+    if (ic->kind == GB200_IC_POLAR_PLANE) return ic->width;
+    if (ic->kind == GB200_IC_CARTESIAN_PLANE) return 2 * (ic->height / 2) - 1;
+    return 0;
 }
 
 static void fill_params(const gb200_problem* p, const gb200_ic* ic, const gb200_range* rg, GbParams& P) {
@@ -302,14 +321,8 @@ static void fill_params(const gb200_problem* p, const gb200_ic* ic, const gb200_
     P.first = rg->first; P.count = rg->count; P.stride = rg->stride;
     P.block = rg->block > 0 ? rg->block : 1;
     // 2-D tiled work order when the range is made of whole strips of GB_TILE_C image columns (or theta-rows of the plane)
-    P.tile_h = 0;
-    if (ic->kind != GB200_IC_EXPLICIT && ic->kind != GB200_IC_IMPACT_PARAMETERS && !getenv("GB200_NO_TILING")) {
-        const int64_t h = (ic->kind == GB200_IC_RENDER_GRID) ? ic->height
-                        : (ic->kind == GB200_IC_CARTESIAN_PLANE) ? (2 * (ic->height / 2) - 1) : ic->width; // fastest-varying extent of the ray index
-        const int64_t strip = GB_TILE_C * h;
-        const bool contiguous = (P.stride == 1) || (P.block % strip == 0);
-        if (h % GB_TILE_R == 0 && contiguous && P.first % strip == 0 && P.count % strip == 0) P.tile_h = h;
-    }
+    const int64_t h = strip_height(ic), strip = GB_TILE_C * h;
+    if (h > 0 && h % GB_TILE_R == 0 && (P.stride == 1 || P.block % strip == 0) && P.first % strip == 0 && P.count % strip == 0) P.tile_h = h;
 }
 
 // ---------------------------------------------------------------- device memory
@@ -330,6 +343,22 @@ static int pool_get(gb200_ctx* ctx, size_t slot, size_t bytes, void** out) {
 enum { SL_STATUS = 0, SL_LAMBDA, SL_X0, SL_V0 = SL_X0 + 4, SL_XI0 = SL_V0 + 4, SL_VI0 = SL_XI0 + 4, SL_NACC = SL_VI0 + 4, SL_NREJ, SL_FLAGS,
        SL_IMG0, SL_G = SL_IMG0 + GB_MAX_PF, SL_F, SL_EX0, SL_EV0 = SL_EX0 + 4, SL_BINS = SL_EV0 + 4, SL_PARTIAL, SL_FLUX, SL_EMR, SL_EME,
        SL_PL0, SL_SCRATCH = SL_PL0 + 4, SL_BATCH, SL_BATCH_QUEUE, SL_COUNT };
+
+// The output arrays of gb200_endpoints: f(host array, GbParams field the kernel writes it through, pool slot of a single
+// call) for each, null host arrays included.  Every copy, binding and layout of endpoints goes through this one list.
+template <class F> static void endpoint_arrays(const gb200_endpoints& out, GbParams& P, F&& f) {
+    f(out.status, P.o_status, SL_STATUS);
+    f(out.lambda_max, P.o_lambda, SL_LAMBDA);
+    for (int k = 0; k < 4; ++k) {
+        f(out.x[k], P.o_x[k], SL_X0 + k);
+        f(out.v[k], P.o_v[k], SL_V0 + k);
+        f(out.x_init[k], P.o_x0[k], SL_XI0 + k);
+        f(out.v_init[k], P.o_v0[k], SL_VI0 + k);
+    }
+    f(out.naccept, P.o_naccept, SL_NACC);
+    f(out.nreject, P.o_nreject, SL_NREJ);
+    f(out.flags, P.o_flags, SL_FLAGS);
+}
 
 static int upload(gb200_ctx* ctx, size_t slot, const void* host, size_t bytes, const void** dev) {
     void* d = nullptr;
@@ -419,6 +448,14 @@ static int run_trace(gb200_ctx* ctx, GbParams& P, cudaStream_t stream, bool time
     return GB200_OK;
 }
 
+// add k launches' queue-counter quadruples ([0] ticket queue, [1..3] accepted steps, rejected steps, flagged rays)
+static void add_counters(gb200_ctx* ctx, const unsigned long long* c, size_t k) {
+    for (size_t i = 0; i < k; ++i) {
+        ctx->stats.steps_accepted += (int64_t)c[4 * i + 1]; ctx->stats.steps_rejected += (int64_t)c[4 * i + 2];
+        ctx->stats.flagged += (int64_t)c[4 * i + 3];
+    }
+}
+
 static int finish_stats(gb200_ctx* ctx, int64_t rays) {
     unsigned long long c[4];
     CU(ctx, cudaMemcpyAsync(c, ctx->d_queue, sizeof c, cudaMemcpyDeviceToHost, ctx->cur));
@@ -428,7 +465,16 @@ static int finish_stats(gb200_ctx* ctx, int64_t rays) {
     cudaEventElapsedTime(&k, ctx->ev1, ctx->ev2);
     cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
     ctx->stats.kernel_ms = k; ctx->stats.total_ms = tot; ctx->stats.rays = rays;
-    ctx->stats.steps_accepted = (int64_t)c[1]; ctx->stats.steps_rejected = (int64_t)c[2]; ctx->stats.flagged = (int64_t)c[3];
+    add_counters(ctx, c, 1);
+    return GB200_OK;
+}
+
+static int ensure_streams(gb200_ctx* ctx, size_t n) {
+    while (ctx->pool_streams.size() < n) {
+        cudaStream_t st;
+        CU(ctx, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+        ctx->pool_streams.push_back(st);
+    }
     return GB200_OK;
 }
 
@@ -453,11 +499,7 @@ static int run_pipelined(gb200_ctx* ctx, const gb200_range* rg, const GbParams& 
     cudaStream_t stream = ctx->cur;
     const int64_t unit = pipeline_unit(P);
     const int64_t per = ((rg->count / unit + K - 1) / K) * unit;
-    while (ctx->pool_streams.size() < 2) {
-        cudaStream_t st;
-        CU(ctx, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-        ctx->pool_streams.push_back(st);
-    }
+    int rc = ensure_streams(ctx, 2); if (rc) return rc;
     while (ctx->chunk_events.size() < (size_t)K + 2) {
         cudaEvent_t ev;
         CU(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
@@ -465,7 +507,7 @@ static int run_pipelined(gb200_ctx* ctx, const gb200_range* rg, const GbParams& 
     }
     cudaStream_t alt = ctx->pool_streams[0], copy = ctx->pool_streams[1];
     void* qv = nullptr;
-    int rc = pool_get(ctx, SL_BATCH_QUEUE, sizeof(unsigned long long) * 4 * K, &qv); if (rc) return rc;
+    rc = pool_get(ctx, SL_BATCH_QUEUE, sizeof(unsigned long long) * 4 * K, &qv); if (rc) return rc;
     unsigned long long* queues = (unsigned long long*)qv;
     CU(ctx, cudaMemsetAsync(queues, 0, sizeof(unsigned long long) * 4 * K, stream));
     CU(ctx, cudaEventRecord(ctx->ev1, stream)); // uploads and queue reset done: the other stream may start
@@ -507,9 +549,79 @@ static int run_pipelined(gb200_ctx* ctx, const gb200_range* rg, const GbParams& 
     cudaEventElapsedTime(&kms, ctx->ev1, ctx->ev2);
     cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
     ctx->stats.kernel_ms = kms; ctx->stats.total_ms = tot; ctx->stats.rays = rg->count;
-    for (int c = 0; c < nchunks; ++c) {
-        ctx->stats.steps_accepted += (int64_t)cq[(size_t)c * 4 + 1]; ctx->stats.steps_rejected += (int64_t)cq[(size_t)c * 4 + 2];
-        ctx->stats.flagged += (int64_t)cq[(size_t)c * 4 + 3];
+    add_counters(ctx, cq.data(), (size_t)nchunks);
+    return GB200_OK;
+}
+
+// ---------------------------------------------------------------- batches
+// A batch call lays its items out in one device arena, [inputs of every item | outputs of every item], mirrored byte for
+// byte by the context's pinned staging buffer, so the whole batch costs one H2D and one D2H copy instead of ~20 small
+// ones per item.  An item's layout is written once, as calls of take() on an input and an output Arena, and run in
+// passes: with null bases to size the arena, with the staging buffer to stage the inputs, with the device arena to bind
+// the kernel's pointers, and with the staging buffer again to find the outputs.  So the passes cannot disagree.
+struct Arena {
+    char* base;                  // nullptr: the pass only sizes the arena
+    bool fill = false;           // base is the staging buffer: copy each input's host array into its place
+    size_t used = 0;
+    const double* table[4] = {}; // the plunging table placed last (place_plunging)
+    template <class T> void take(T*& p, int64_t n, const void* src = nullptr) {
+        p = base ? (T*)(base + used) : nullptr;
+        const size_t bytes = sizeof(T) * (size_t)n;
+        if (fill && src) memcpy((void*)p, src, bytes);
+        used += (bytes + 255) & ~(size_t)255;
+    }
+};
+
+// Plunging table of batch item b, bound into P.  Consecutive items with the same table share one copy in the arena.
+static void place_plunging(Arena& in, const gb200_plunging_table* const* pls, int b, GbParams& P) {
+    const gb200_plunging_table* pl = pls ? pls[b] : nullptr;
+    if (!pl || pl->n < 2) return;
+    if (b == 0 || pl != pls[b - 1]) {
+        const double* src[4] = {pl->r, pl->ut, pl->ur, pl->uphi};
+        for (int k = 0; k < 4; ++k) in.take(in.table[k], pl->n, src[k]);
+    }
+    P.pl_n = pl->n;
+    P.pl_r = in.table[0]; P.pl_ut = in.table[1]; P.pl_ur = in.table[2]; P.pl_uphi = in.table[3];
+}
+
+// The output arrays of gb200_dual_out: f(host array, GbDualIO field the kernel writes it through, element count).
+template <class F> static void dual_arrays(const gb200_dual_out& out, GbDualIO& io, int64_t n, int64_t npartials, F&& f) {
+    f(out.status, io.status, n);
+    f(out.lambda_max, io.lambda, n);
+    for (int k = 0; k < 4; ++k) {
+        f(out.x[k], io.x[k], n);
+        f(out.v[k], io.v[k], n);
+    }
+    f(out.g, io.g, n);
+    f(out.dg, io.dg, n * npartials);
+    f(out.rho, io.rho, n);
+    f(out.drho, io.drho, n * npartials);
+    f(out.naccept, io.naccept, n);
+    f(out.nreject, io.nreject, n);
+    f(out.flags, io.flags, n);
+}
+
+static int ensure_stage(gb200_ctx* ctx, size_t total) {
+    if (ctx->stage_cap >= total) return GB200_OK;
+    if (ctx->stage) cudaFreeHost(ctx->stage);
+    ctx->stage = nullptr; ctx->stage_cap = 0;
+    CU(ctx, cudaMallocHost(&ctx->stage, total + 256));
+    ctx->stage_cap = total;
+    return GB200_OK;
+}
+
+// the first nstreams pool streams start after the work enqueued on the context stream so far (ev1)
+static int fan_out(gb200_ctx* ctx, int nstreams) {
+    CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    for (int sidx = 0; sidx < nstreams; ++sidx) CU(ctx, cudaStreamWaitEvent(ctx->pool_streams[(size_t)sidx], ctx->ev1, 0));
+    return GB200_OK;
+}
+
+// join the first nstreams pool streams back into the context stream; ev2 ends recorded on the last of them
+static int fan_in(gb200_ctx* ctx, int nstreams) {
+    for (int sidx = 0; sidx < nstreams; ++sidx) {
+        CU(ctx, cudaEventRecord(ctx->ev2, ctx->pool_streams[(size_t)sidx]));
+        CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev2, 0));
     }
     return GB200_OK;
 }
@@ -639,55 +751,21 @@ static int trace_common(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* 
         rc = pool_get(ctx, SL_G, n * sizeof(double) + 8, &d); if (rc) return rc;
         P.o_closest = (double*)d;
     }
-#define WANT(ptr, slot, type, field)                                               \
-    if (ptr) { rc = pool_get(ctx, slot, n * sizeof(type) + 8, &d); if (rc) return rc; field = (type*)d; }
-    WANT(out->status, SL_STATUS, int32_t, P.o_status)
-    WANT(out->lambda_max, SL_LAMBDA, double, P.o_lambda)
-    for (int k = 0; k < 4; ++k) {
-        WANT(out->x[k], SL_X0 + k, double, P.o_x[k])
-        WANT(out->v[k], SL_V0 + k, double, P.o_v[k])
-        WANT(out->x_init[k], SL_XI0 + k, double, P.o_x0[k])
-        WANT(out->v_init[k], SL_VI0 + k, double, P.o_v0[k])
-    }
-    WANT(out->naccept, SL_NACC, int32_t, P.o_naccept)
-    WANT(out->nreject, SL_NREJ, int32_t, P.o_nreject)
-    WANT(out->flags, SL_FLAGS, int32_t, P.o_flags)
-#undef WANT
-    if (!target && pipeline_eligible(P, rg)) {
-        const GbParams Pf = P;
-        return run_pipelined(ctx, rg, P,
-            [&](GbParams& Pc, int64_t s0) {
-                if (Pf.o_status) Pc.o_status = Pf.o_status + s0;
-                if (Pf.o_lambda) Pc.o_lambda = Pf.o_lambda + s0;
-                for (int k = 0; k < 4; ++k) {
-                    if (Pf.o_x[k]) Pc.o_x[k] = Pf.o_x[k] + s0;
-                    if (Pf.o_v[k]) Pc.o_v[k] = Pf.o_v[k] + s0;
-                    if (Pf.o_x0[k]) Pc.o_x0[k] = Pf.o_x0[k] + s0;
-                    if (Pf.o_v0[k]) Pc.o_v0[k] = Pf.o_v0[k] + s0;
-                }
-                if (Pf.o_naccept) Pc.o_naccept = Pf.o_naccept + s0;
-                if (Pf.o_nreject) Pc.o_nreject = Pf.o_nreject + s0;
-                if (Pf.o_flags) Pc.o_flags = Pf.o_flags + s0;
-            },
-            [&](int64_t s0, int64_t cnt, cudaStream_t copy) -> cudaError_t {
-                cudaError_t e = cudaSuccess;
-#define BACKC(ptr, field, type) \
-    if (e == cudaSuccess && ptr) e = cudaMemcpyAsync(ptr + s0, field + s0, (size_t)cnt * sizeof(type), cudaMemcpyDeviceToHost, copy);
-                BACKC(out->status, Pf.o_status, int32_t)
-                BACKC(out->lambda_max, Pf.o_lambda, double)
-                for (int k = 0; k < 4; ++k) {
-                    BACKC(out->x[k], Pf.o_x[k], double)
-                    BACKC(out->v[k], Pf.o_v[k], double)
-                    BACKC(out->x_init[k], Pf.o_x0[k], double)
-                    BACKC(out->v_init[k], Pf.o_v0[k], double)
-                }
-                BACKC(out->naccept, Pf.o_naccept, int32_t)
-                BACKC(out->nreject, Pf.o_nreject, int32_t)
-                BACKC(out->flags, Pf.o_flags, int32_t)
-#undef BACKC
-                return e;
-            });
-    }
+    endpoint_arrays(*out, P, [&](auto* h, auto*& f, int slot) {
+        if (h && !rc && !(rc = pool_get(ctx, (size_t)slot, n * sizeof(*f) + 8, &d))) f = (decltype(h))d;
+    });
+    if (rc) return rc;
+    // the endpoints of slots [s0, s0 + cnt) to the host
+    auto copy_back = [&](int64_t s0, int64_t cnt, cudaStream_t copy) -> cudaError_t {
+        cudaError_t e = cudaSuccess;
+        endpoint_arrays(*out, P, [&](auto* h, auto* f, int) {
+            if (e == cudaSuccess && h) e = cudaMemcpyAsync(h + s0, f + s0, (size_t)cnt * sizeof(*f), cudaMemcpyDeviceToHost, copy);
+        });
+        return e;
+    };
+    if (!target && pipeline_eligible(P, rg))
+        return run_pipelined(ctx, rg, P, [&](GbParams& Pc, int64_t s0) { endpoint_arrays(*out, Pc, [&](auto*, auto*& f, int) { if (f) f += s0; }); },
+                             copy_back);
     if (target) { // one ray per thread through the generic integrator; no ticket queue, no step counters
         CU(ctx, cudaMemsetAsync(ctx->d_queue, 0, 4 * sizeof(unsigned long long), ctx->stream));
         CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
@@ -696,20 +774,7 @@ static int trace_common(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* 
         ctx->stats.launches += n ? 1 : 0;
         if (n) CU(ctx, cudaMemcpyAsync(closest, P.o_closest, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     } else { rc = run_trace(ctx, P, ctx->stream, true); if (rc) return rc; }
-#define BACK(ptr, field, type) \
-    if (ptr && n) CU(ctx, cudaMemcpyAsync(ptr, field, n * sizeof(type), cudaMemcpyDeviceToHost, ctx->stream));
-    BACK(out->status, P.o_status, int32_t)
-    BACK(out->lambda_max, P.o_lambda, double)
-    for (int k = 0; k < 4; ++k) {
-        BACK(out->x[k], P.o_x[k], double)
-        BACK(out->v[k], P.o_v[k], double)
-        BACK(out->x_init[k], P.o_x0[k], double)
-        BACK(out->v_init[k], P.o_v0[k], double)
-    }
-    BACK(out->naccept, P.o_naccept, int32_t)
-    BACK(out->nreject, P.o_nreject, int32_t)
-    BACK(out->flags, P.o_flags, int32_t)
-#undef BACK
+    if (n) CU(ctx, copy_back(0, rg->count, ctx->stream));
     return finish_stats(ctx, rg->count);
 }
 
@@ -735,113 +800,60 @@ int gb200_trace_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* probl
     }
     { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
     const int nstreams = nbatch < 32 ? nbatch : 32;
-    while ((int)ctx->pool_streams.size() < nstreams) {
-        cudaStream_t st;
-        CU(ctx, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-        ctx->pool_streams.push_back(st);
-    }
-    // One device arena: [explicit ICs of every ensemble | outputs of every ensemble], mirrored by one pinned host
-    // staging buffer, so the whole batch costs one H2D and one D2H copy instead of ~20 small ones per ensemble.
-    auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    struct Off { size_t status, lambda, x[4], v[4], x0[4], v0[4], nacc, nrej, flags, ex[4], ev[4]; };
-    std::vector<Off> off((size_t)nbatch);
-    size_t total = 0;
-    for (int b = 0; b < nbatch; ++b)
+    int rc = ensure_streams(ctx, (size_t)nstreams); if (rc) return rc;
+    // inputs: the explicit ICs; outputs: the endpoint arrays the caller asked for
+    auto layout = [&](int b, Arena& in, Arena& out, GbParams& P) {
         if (ics[b].kind == GB200_IC_EXPLICIT)
-            for (int k = 0; k < 4; ++k) { off[(size_t)b].ex[k] = total; total += al(8 * (size_t)ics[b].n); off[(size_t)b].ev[k] = total; total += al(8 * (size_t)ics[b].n); }
-    const size_t in_bytes = total;
-    for (int b = 0; b < nbatch; ++b) {
-        const size_t n = (size_t)ranges[b].count;
-        Off& o = off[(size_t)b];
-        o.status = total; total += al(4 * n);
-        o.lambda = total; total += al(8 * n);
-        for (int k = 0; k < 4; ++k) { o.x[k] = total; total += al(8 * n); o.v[k] = total; total += al(8 * n);
-                                      o.x0[k] = total; total += al(8 * n); o.v0[k] = total; total += al(8 * n); }
-        o.nacc = total; total += al(4 * n); o.nrej = total; total += al(4 * n); o.flags = total; total += al(4 * n);
-    }
+            for (int k = 0; k < 4; ++k) { in.take(P.ex[k], ics[b].n, ics[b].x[k]); in.take(P.ev[k], ics[b].n, ics[b].v[k]); }
+        endpoint_arrays(outs[b], P, [&](auto* h, auto*& f, int) { if (h) out.take(f, ranges[b].count); });
+    };
+    GbParams S{}; // pointers of the passes over the staging buffer
+    Arena size_in{nullptr}, size_out{nullptr};
+    for (int b = 0; b < nbatch; ++b) layout(b, size_in, size_out, S);
+    const size_t in_bytes = size_in.used, total = in_bytes + size_out.used;
     void* arena_v = nullptr;
-    int rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
+    rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
     char* arena = (char*)arena_v;
-    if (ctx->stage_cap < total) {
-        if (ctx->stage) cudaFreeHost(ctx->stage);
-        ctx->stage = nullptr; ctx->stage_cap = 0;
-        CU(ctx, cudaMallocHost(&ctx->stage, total + 256));
-        ctx->stage_cap = total;
-    }
+    rc = ensure_stage(ctx, total); if (rc) return rc;
     char* stage = (char*)ctx->stage;
     void* qv = nullptr;
     rc = pool_get(ctx, SL_BATCH_QUEUE, sizeof(unsigned long long) * 4 * (size_t)nbatch, &qv); if (rc) return rc;
     unsigned long long* queues = (unsigned long long*)qv;
-    for (int b = 0; b < nbatch; ++b)
-        if (ics[b].kind == GB200_IC_EXPLICIT)
-            for (int k = 0; k < 4; ++k) {
-                memcpy(stage + off[(size_t)b].ex[k], ics[b].x[k], 8 * (size_t)ics[b].n);
-                memcpy(stage + off[(size_t)b].ev[k], ics[b].v[k], 8 * (size_t)ics[b].n);
-            }
+    Arena stage_in{stage, true}, stage_out{stage + in_bytes};
+    for (int b = 0; b < nbatch; ++b) layout(b, stage_in, stage_out, S);
     CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     CU(ctx, cudaMemsetAsync(queues, 0, sizeof(unsigned long long) * 4 * (size_t)nbatch, ctx->stream));
     if (in_bytes) CU(ctx, cudaMemcpyAsync(arena, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    for (int sidx = 0; sidx < nstreams; ++sidx) CU(ctx, cudaStreamWaitEvent(ctx->pool_streams[(size_t)sidx], ctx->ev1, 0));
+    rc = fan_out(ctx, nstreams); if (rc) return rc;
+    Arena dev_in{arena}, dev_out{arena + in_bytes};
     for (int b = 0; b < nbatch; ++b) {
         cudaStream_t st = ctx->pool_streams[(size_t)(b % nstreams)];
-        const gb200_endpoints& out = outs[b];
-        const Off& o = off[(size_t)b];
         GbParams P;
         fill_params(&problems[b], &ics[b], &ranges[b], P);
         { int rcg_ = bind_geometry(ctx, P); if (rcg_) return rcg_; }
-        if (ics[b].kind == GB200_IC_EXPLICIT)
-            for (int k = 0; k < 4; ++k) { P.ex[k] = (const double*)(arena + o.ex[k]); P.ev[k] = (const double*)(arena + o.ev[k]); }
-        if (out.status) P.o_status = (int32_t*)(arena + o.status);
-        if (out.lambda_max) P.o_lambda = (double*)(arena + o.lambda);
-        for (int k = 0; k < 4; ++k) {
-            if (out.x[k]) P.o_x[k] = (double*)(arena + o.x[k]);
-            if (out.v[k]) P.o_v[k] = (double*)(arena + o.v[k]);
-            if (out.x_init[k]) P.o_x0[k] = (double*)(arena + o.x0[k]);
-            if (out.v_init[k]) P.o_v0[k] = (double*)(arena + o.v0[k]);
-        }
-        if (out.naccept) P.o_naccept = (int32_t*)(arena + o.nacc);
-        if (out.nreject) P.o_nreject = (int32_t*)(arena + o.nrej);
-        if (out.flags) P.o_flags = (int32_t*)(arena + o.flags);
+        layout(b, dev_in, dev_out, P);
         P.queue = queues + 4 * (size_t)b;
         P.counters = P.queue + 1;
         int blocks = 0;
         if (ranges[b].count) { CU(ctx, gb200_launch_trace(P, ctx->sm_count, st, &blocks)); ctx->stats.launches += 1; }
     }
-    for (int sidx = 0; sidx < nstreams; ++sidx) { // join the pool back into the context stream
-        CU(ctx, cudaEventRecord(ctx->ev2, ctx->pool_streams[(size_t)sidx]));
-        CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev2, 0));
-    }
+    rc = fan_in(ctx, nstreams); if (rc) return rc;
     std::vector<unsigned long long> c((size_t)nbatch * 4);
     if (total > in_bytes) CU(ctx, cudaMemcpyAsync(stage + in_bytes, arena + in_bytes, total - in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaMemcpyAsync(c.data(), queues, sizeof(unsigned long long) * c.size(), cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
+    Arena host_in{stage}, host_out{stage + in_bytes};
     for (int b = 0; b < nbatch; ++b) { // scatter the staging buffer into the caller's SoA
-        const gb200_endpoints& out = outs[b];
-        const Off& o = off[(size_t)b];
-        const size_t n = (size_t)ranges[b].count;
-        if (out.status) memcpy(out.status, stage + o.status, 4 * n);
-        if (out.lambda_max) memcpy(out.lambda_max, stage + o.lambda, 8 * n);
-        for (int k = 0; k < 4; ++k) {
-            if (out.x[k]) memcpy(out.x[k], stage + o.x[k], 8 * n);
-            if (out.v[k]) memcpy(out.v[k], stage + o.v[k], 8 * n);
-            if (out.x_init[k]) memcpy(out.x_init[k], stage + o.x0[k], 8 * n);
-            if (out.v_init[k]) memcpy(out.v_init[k], stage + o.v0[k], 8 * n);
-        }
-        if (out.naccept) memcpy(out.naccept, stage + o.nacc, 4 * n);
-        if (out.nreject) memcpy(out.nreject, stage + o.nrej, 4 * n);
-        if (out.flags) memcpy(out.flags, stage + o.flags, 4 * n);
+        layout(b, host_in, host_out, S);
+        endpoint_arrays(outs[b], S, [&](auto* h, auto* f, int) { if (h) memcpy(h, f, (size_t)ranges[b].count * sizeof(*f)); });
     }
     float tot = 0, dev = 0;
     cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
     cudaEventElapsedTime(&dev, ctx->ev1, ctx->ev2); // launches only (ev2: the end of the last pool stream), without the two staged copies
     ctx->stats.kernel_ms = dev; ctx->stats.total_ms = tot;
-    for (int b = 0; b < nbatch; ++b) {
-        ctx->stats.rays += ranges[b].count;
-        ctx->stats.steps_accepted += (int64_t)c[(size_t)b * 4 + 1]; ctx->stats.steps_rejected += (int64_t)c[(size_t)b * 4 + 2];
-        ctx->stats.flagged += (int64_t)c[(size_t)b * 4 + 3];
-    }
+    for (int b = 0; b < nbatch; ++b) ctx->stats.rays += ranges[b].count;
+    add_counters(ctx, c.data(), (size_t)nbatch);
     return GB200_OK;
 }
 
@@ -935,11 +947,8 @@ static int render_common(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic*
     if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
     int rc = validate(ctx, p, ic); if (rc) return rc;
     rc = validate_range(ctx, ic, rg); if (rc) return rc;
-    if (npf < 1 || npf > GB_MAX_PF || !pfs || !images) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 1..%d point functions", GB_MAX_PF);
-    for (int k = 0; k < npf; ++k) {
-        if (pfs[k] < GB200_PF_SHADOW || pfs[k] > GB200_PF_EQUATORIAL_CROSSINGS) return fail(ctx, GB200_ERR_UNSUPPORTED, "point function %d", pfs[k]);
-        if (!images[k]) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null image pointer");
-    }
+    if (!images) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 1..%d point functions", GB_MAX_PF);
+    rc = validate_pfs(ctx, pfs, npf, images); if (rc) return rc;
     { int rc_ = begin_call(ctx, stream); if (rc_) return rc_; }
     CU(ctx, cudaEventRecord(ctx->ev0, stream));
     GbParams P;
@@ -991,111 +1000,76 @@ int gb200_render_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* prob
         for (int b = 0; b < nbatch; ++b) { int rc_ = validate_crossings(ctx, &problems[b], pfs, npf); if (rc_) return rc_; }
     if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
     if (nbatch < 1 || !problems || !ics || !ranges || !pfs || !images) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad batch arguments");
-    if (npf < 1 || npf > GB_MAX_PF) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 1..%d point functions", GB_MAX_PF);
-    for (int k = 0; k < npf; ++k)
-        if (pfs[k] < GB200_PF_SHADOW || pfs[k] > GB200_PF_EQUATORIAL_CROSSINGS) return fail(ctx, GB200_ERR_UNSUPPORTED, "point function %d", pfs[k]);
+    int rc = validate_pfs(ctx, pfs, npf, nullptr); if (rc) return rc; // the images are checked per item: empty items need none
     for (int b = 0; b < nbatch; ++b) {
-        int rc = validate(ctx, &problems[b], &ics[b]); if (rc) return rc;
+        rc = validate(ctx, &problems[b], &ics[b]); if (rc) return rc;
         rc = validate_range(ctx, &ics[b], &ranges[b]); if (rc) return rc;
         if (ics[b].kind == GB200_IC_EXPLICIT) return fail(ctx, GB200_ERR_UNSUPPORTED, "explicit initial conditions are batched by gb200_trace_batch");
         for (int k = 0; k < npf; ++k) if (ranges[b].count && !images[(size_t)b * npf + k]) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null image pointer");
     }
     { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
     const int nstreams = nbatch < 32 ? nbatch : 32;
-    while ((int)ctx->pool_streams.size() < nstreams) {
-        cudaStream_t st;
-        CU(ctx, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-        ctx->pool_streams.push_back(st);
-    }
-    // One arena: [impact-parameter lists (+ heights) and plunging tables of every problem | images of every problem],
-    // mirrored by one pinned staging buffer: one H2D and one D2H copy for the whole batch.
-    auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    struct Off { size_t ex[3], pl[4], img[GB_MAX_PF]; };
-    std::vector<Off> off((size_t)nbatch);
-    size_t total = 0;
-    for (int b = 0; b < nbatch; ++b) {
-        Off& o = off[(size_t)b];
+    rc = ensure_streams(ctx, (size_t)nstreams); if (rc) return rc;
+    // inputs: the impact-parameter lists (+ heights) and the plunging table; outputs: the images
+    auto layout = [&](int b, Arena& in, Arena& out, GbParams& P) {
         if (ics[b].kind == GB200_IC_IMPACT_PARAMETERS)
-            for (int k = 0; k < 3; ++k) if (ics[b].x[k]) { o.ex[k] = total; total += al(8 * (size_t)ics[b].n); }
-        if (pls && pls[b] && pls[b]->n >= 2) {
-            if (b > 0 && pls[b] == pls[b - 1]) { for (int k = 0; k < 4; ++k) o.pl[k] = off[(size_t)b - 1].pl[k]; }
-            else for (int k = 0; k < 4; ++k) { o.pl[k] = total; total += al(8 * (size_t)pls[b]->n); }
-        }
-    }
-    const size_t in_bytes = total;
-    for (int b = 0; b < nbatch; ++b)
-        for (int k = 0; k < npf; ++k) { off[(size_t)b].img[k] = total; total += al(8 * (size_t)ranges[b].count); }
+            for (int k = 0; k < 3; ++k) if (ics[b].x[k]) in.take(P.ex[k], ics[b].n, ics[b].x[k]);
+        place_plunging(in, pls, b, P);
+        for (int k = 0; k < npf; ++k) out.take(P.o_img[k], ranges[b].count);
+    };
+    GbParams S{}; // pointers of the passes over the staging buffer and of the items that do not launch
+    Arena size_in{nullptr}, size_out{nullptr};
+    for (int b = 0; b < nbatch; ++b) layout(b, size_in, size_out, S);
+    const size_t in_bytes = size_in.used, total = in_bytes + size_out.used;
     void* arena_v = nullptr;
-    int rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
+    rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
     char* arena = (char*)arena_v;
-    if (ctx->stage_cap < total) {
-        if (ctx->stage) cudaFreeHost(ctx->stage);
-        ctx->stage = nullptr; ctx->stage_cap = 0;
-        CU(ctx, cudaMallocHost(&ctx->stage, total + 256));
-        ctx->stage_cap = total;
-    }
+    rc = ensure_stage(ctx, total); if (rc) return rc;
     char* stage = (char*)ctx->stage;
     void* qv = nullptr;
     rc = pool_get(ctx, SL_BATCH_QUEUE, sizeof(unsigned long long) * 4 * (size_t)nbatch, &qv); if (rc) return rc;
     unsigned long long* queues = (unsigned long long*)qv;
-    for (int b = 0; b < nbatch; ++b) {
-        const Off& o = off[(size_t)b];
-        if (ics[b].kind == GB200_IC_IMPACT_PARAMETERS)
-            for (int k = 0; k < 3; ++k) if (ics[b].x[k]) memcpy(stage + o.ex[k], ics[b].x[k], 8 * (size_t)ics[b].n);
-        if (pls && pls[b] && pls[b]->n >= 2 && !(b > 0 && pls[b] == pls[b - 1])) {
-            const double* src[4] = {pls[b]->r, pls[b]->ut, pls[b]->ur, pls[b]->uphi};
-            for (int k = 0; k < 4; ++k) memcpy(stage + o.pl[k], src[k], 8 * (size_t)pls[b]->n);
-        }
-    }
+    Arena stage_in{stage, true}, stage_out{stage + in_bytes};
+    for (int b = 0; b < nbatch; ++b) layout(b, stage_in, stage_out, S);
     CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     CU(ctx, cudaMemsetAsync(queues, 0, sizeof(unsigned long long) * 4 * (size_t)nbatch, ctx->stream));
     if (in_bytes) CU(ctx, cudaMemcpyAsync(arena, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    for (int sidx = 0; sidx < nstreams; ++sidx) CU(ctx, cudaStreamWaitEvent(ctx->pool_streams[(size_t)sidx], ctx->ev1, 0));
+    rc = fan_out(ctx, nstreams); if (rc) return rc;
     const bool want_isco = needs_isco(pfs, npf, false);
+    Arena dev_in{arena}, dev_out{arena + in_bytes};
     for (int b = 0; b < nbatch; ++b) {
-        if (!ranges[b].count) continue;
+        if (!ranges[b].count) { layout(b, dev_in, dev_out, S); continue; } // the item keeps its place, and its table may be shared
         cudaStream_t st = ctx->pool_streams[(size_t)(b % nstreams)];
-        const Off& o = off[(size_t)b];
         GbParams P;
         fill_params(&problems[b], &ics[b], &ranges[b], P);
         { int rcg_ = bind_geometry(ctx, P); if (rcg_) return rcg_; }
         if (want_isco) { rc = set_isco(ctx, &problems[b], P); if (rc) return rc; }
-        if (ics[b].kind == GB200_IC_IMPACT_PARAMETERS)
-            for (int k = 0; k < 3; ++k) P.ex[k] = ics[b].x[k] ? (const double*)(arena + o.ex[k]) : nullptr;
-        if (pls && pls[b] && pls[b]->n >= 2) {
-            P.pl_n = pls[b]->n;
-            P.pl_r = (const double*)(arena + o.pl[0]); P.pl_ut = (const double*)(arena + o.pl[1]);
-            P.pl_ur = (const double*)(arena + o.pl[2]); P.pl_uphi = (const double*)(arena + o.pl[3]);
-        }
+        layout(b, dev_in, dev_out, P);
         P.npf = npf;
-        for (int k = 0; k < npf; ++k) { P.pf[k] = pfs[k]; P.o_img[k] = (double*)(arena + o.img[k]); }
+        for (int k = 0; k < npf; ++k) P.pf[k] = pfs[k];
         P.queue = queues + 4 * (size_t)b;
         P.counters = P.queue + 1;
         int blocks = 0;
         CU(ctx, gb200_launch_trace(P, ctx->sm_count, st, &blocks));
         ctx->stats.launches += 1;
     }
-    for (int sidx = 0; sidx < nstreams; ++sidx) { // join the pool back into the context stream
-        CU(ctx, cudaEventRecord(ctx->ev2, ctx->pool_streams[(size_t)sidx]));
-        CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev2, 0));
-    }
+    rc = fan_in(ctx, nstreams); if (rc) return rc;
     std::vector<unsigned long long> c((size_t)nbatch * 4);
     if (total > in_bytes) CU(ctx, cudaMemcpyAsync(stage + in_bytes, arena + in_bytes, total - in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaMemcpyAsync(c.data(), queues, sizeof(unsigned long long) * c.size(), cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
-    for (int b = 0; b < nbatch; ++b)
+    Arena host_in{stage}, host_out{stage + in_bytes};
+    for (int b = 0; b < nbatch; ++b) {
+        layout(b, host_in, host_out, S);
         for (int k = 0; k < npf; ++k)
-            if (ranges[b].count) memcpy(images[(size_t)b * npf + k], stage + off[(size_t)b].img[k], 8 * (size_t)ranges[b].count);
+            if (ranges[b].count) memcpy(images[(size_t)b * npf + k], S.o_img[k], 8 * (size_t)ranges[b].count);
+    }
     float tot = 0;
     cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
     ctx->stats.kernel_ms = tot; ctx->stats.total_ms = tot;
-    for (int b = 0; b < nbatch; ++b) {
-        ctx->stats.rays += ranges[b].count;
-        ctx->stats.steps_accepted += (int64_t)c[(size_t)b * 4 + 1]; ctx->stats.steps_rejected += (int64_t)c[(size_t)b * 4 + 2];
-        ctx->stats.flagged += (int64_t)c[(size_t)b * 4 + 3];
-    }
+    for (int b = 0; b < nbatch; ++b) ctx->stats.rays += ranges[b].count;
+    add_counters(ctx, c.data(), (size_t)nbatch);
     return GB200_OK;
 }
 
@@ -1121,127 +1095,58 @@ int gb200_trace_dual_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* 
     }
     { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
     const int nstreams = nbatch < 32 ? nbatch : 32;
-    while ((int)ctx->pool_streams.size() < nstreams) {
-        cudaStream_t st;
-        CU(ctx, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-        ctx->pool_streams.push_back(st);
-    }
-    auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    struct Off { size_t alpha, beta, dalpha, dbeta, height, pl[4], status, lambda, x[4], v[4], g, dg, rho, drho, nacc, nrej, flags; };
-    std::vector<Off> off((size_t)nbatch);
-    size_t total = 0;
-    for (int b = 0; b < nbatch; ++b) {
-        Off& o = off[(size_t)b];
-        const size_t n = (size_t)ics[b].n, nd = (size_t)ics[b].npartials;
-        o.alpha = total; total += al(8 * n); o.beta = total; total += al(8 * n);
-        o.dalpha = total; total += al(8 * n * nd); o.dbeta = total; total += al(8 * n * nd);
-        o.height = total; if (ics[b].height) total += al(8 * n);
-        if (pls && pls[b] && pls[b]->n >= 2) {
-            if (b > 0 && pls[b] == pls[b - 1]) { for (int k = 0; k < 4; ++k) o.pl[k] = off[(size_t)b - 1].pl[k]; }
-            else for (int k = 0; k < 4; ++k) { o.pl[k] = total; total += al(8 * (size_t)pls[b]->n); }
-        }
-    }
-    const size_t in_bytes = total;
-    for (int b = 0; b < nbatch; ++b) {
-        Off& o = off[(size_t)b];
-        const size_t n = (size_t)ics[b].n, nd = (size_t)ics[b].npartials;
-        o.status = total; total += al(4 * n); o.lambda = total; total += al(8 * n);
-        for (int k = 0; k < 4; ++k) { o.x[k] = total; total += al(8 * n); o.v[k] = total; total += al(8 * n); }
-        o.g = total; total += al(8 * n); o.dg = total; total += al(8 * n * nd);
-        o.rho = total; total += al(8 * n); o.drho = total; total += al(8 * n * nd);
-        o.nacc = total; total += al(4 * n); o.nrej = total; total += al(4 * n); o.flags = total; total += al(4 * n);
-    }
-    void* arena_v = nullptr;
-    int rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
-    char* arena = (char*)arena_v;
-    if (ctx->stage_cap < total) {
-        if (ctx->stage) cudaFreeHost(ctx->stage);
-        ctx->stage = nullptr; ctx->stage_cap = 0;
-        CU(ctx, cudaMallocHost(&ctx->stage, total + 256));
-        ctx->stage_cap = total;
-    }
-    char* stage = (char*)ctx->stage;
-    for (int b = 0; b < nbatch; ++b) {
-        const Off& o = off[(size_t)b];
+    int rc = ensure_streams(ctx, (size_t)nstreams); if (rc) return rc;
+    // inputs: the seeded impact parameters (+ heights) and the plunging table; outputs: the arrays the caller asked for
+    auto layout = [&](int b, Arena& in, Arena& out, GbParams& P, GbDualIO& io) {
         const gb200_dual_ic& d = ics[b];
-        const size_t n = (size_t)d.n, nd = (size_t)d.npartials;
-        if (n) {
-            memcpy(stage + o.alpha, d.alpha, 8 * n); memcpy(stage + o.beta, d.beta, 8 * n);
-            memcpy(stage + o.dalpha, d.dalpha, 8 * n * nd); memcpy(stage + o.dbeta, d.dbeta, 8 * n * nd);
-            if (d.height) memcpy(stage + o.height, d.height, 8 * n);
-        }
-        if (pls && pls[b] && pls[b]->n >= 2 && !(b > 0 && pls[b] == pls[b - 1])) {
-            const double* src[4] = {pls[b]->r, pls[b]->ut, pls[b]->ur, pls[b]->uphi};
-            for (int k = 0; k < 4; ++k) memcpy(stage + o.pl[k], src[k], 8 * (size_t)pls[b]->n);
-        }
-    }
+        in.take(io.alpha, d.n, d.alpha); in.take(io.beta, d.n, d.beta);
+        in.take(io.dalpha, d.n * d.npartials, d.dalpha); in.take(io.dbeta, d.n * d.npartials, d.dbeta);
+        if (d.height) in.take(io.height, d.n, d.height);
+        place_plunging(in, pls, b, P);
+        dual_arrays(outs[b], io, d.n, d.npartials, [&](auto* h, auto*& f, int64_t n) { if (h) out.take(f, n); });
+    };
+    GbParams S{}; // pointers of the passes over the staging buffer and of the items that do not launch
+    GbDualIO Sio{};
+    Arena size_in{nullptr}, size_out{nullptr};
+    for (int b = 0; b < nbatch; ++b) layout(b, size_in, size_out, S, Sio);
+    const size_t in_bytes = size_in.used, total = in_bytes + size_out.used;
+    void* arena_v = nullptr;
+    rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
+    char* arena = (char*)arena_v;
+    rc = ensure_stage(ctx, total); if (rc) return rc;
+    char* stage = (char*)ctx->stage;
+    Arena stage_in{stage, true}, stage_out{stage + in_bytes};
+    for (int b = 0; b < nbatch; ++b) layout(b, stage_in, stage_out, S, Sio);
     CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     if (in_bytes) CU(ctx, cudaMemcpyAsync(arena, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    for (int sidx = 0; sidx < nstreams; ++sidx) CU(ctx, cudaStreamWaitEvent(ctx->pool_streams[(size_t)sidx], ctx->ev1, 0));
+    rc = fan_out(ctx, nstreams); if (rc) return rc;
+    Arena dev_in{arena}, dev_out{arena + in_bytes};
     for (int b = 0; b < nbatch; ++b) {
         const gb200_dual_ic& d = ics[b];
-        if (d.n == 0) continue;
-        const gb200_dual_out& out = outs[b];
-        const Off& o = off[(size_t)b];
+        if (d.n == 0) { layout(b, dev_in, dev_out, S, Sio); continue; } // the item keeps its place, and its table may be shared
         gb200_range rg{0, d.n, 1, 1};
         GbParams P;
         fill_params(&problems[b], &fake[(size_t)b], &rg, P);
         { int rcg_ = bind_geometry(ctx, P); if (rcg_) return rcg_; }
-        if (out.g) { rc = set_isco(ctx, &problems[b], P); if (rc) return rc; }
-        if (pls && pls[b] && pls[b]->n >= 2) {
-            P.pl_n = pls[b]->n;
-            P.pl_r = (const double*)(arena + o.pl[0]); P.pl_ut = (const double*)(arena + o.pl[1]);
-            P.pl_ur = (const double*)(arena + o.pl[2]); P.pl_uphi = (const double*)(arena + o.pl[3]);
-        }
+        if (outs[b].g) { rc = set_isco(ctx, &problems[b], P); if (rc) return rc; }
+        if (outs[b].dg && !outs[b].g) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "dg needs g");
         GbDualIO io;
         memset(&io, 0, sizeof io);
         io.n = d.n; io.npartials = d.npartials; io.norm_partials = (norm_mode == GB200_DUAL_NORM_WITH_PARTIALS) ? 1 : 0;
-        io.alpha = (const double*)(arena + o.alpha); io.beta = (const double*)(arena + o.beta);
-        io.dalpha = (const double*)(arena + o.dalpha); io.dbeta = (const double*)(arena + o.dbeta);
-        io.height = d.height ? (const double*)(arena + o.height) : nullptr;
-        if (out.status) io.status = (int32_t*)(arena + o.status);
-        if (out.lambda_max) io.lambda = (double*)(arena + o.lambda);
-        for (int k = 0; k < 4; ++k) {
-            if (out.x[k]) io.x[k] = (double*)(arena + o.x[k]);
-            if (out.v[k]) io.v[k] = (double*)(arena + o.v[k]);
-        }
-        if (out.g) io.g = (double*)(arena + o.g);
-        if (out.dg) { if (!out.g) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "dg needs g"); io.dg = (double*)(arena + o.dg); }
-        if (out.rho) io.rho = (double*)(arena + o.rho);
-        if (out.drho) io.drho = (double*)(arena + o.drho);
-        if (out.naccept) io.naccept = (int32_t*)(arena + o.nacc);
-        if (out.nreject) io.nreject = (int32_t*)(arena + o.nrej);
-        if (out.flags) io.flags = (int32_t*)(arena + o.flags);
+        layout(b, dev_in, dev_out, P, io);
         CU(ctx, gb200_launch_dual(P, io, ctx->pool_streams[(size_t)(b % nstreams)]));
         ctx->stats.launches += 1;
         ctx->stats.rays += d.n;
     }
-    for (int sidx = 0; sidx < nstreams; ++sidx) {
-        CU(ctx, cudaEventRecord(ctx->ev2, ctx->pool_streams[(size_t)sidx]));
-        CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev2, 0));
-    }
+    rc = fan_in(ctx, nstreams); if (rc) return rc;
     if (total > in_bytes) CU(ctx, cudaMemcpyAsync(stage + in_bytes, arena + in_bytes, total - in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
+    Arena host_in{stage}, host_out{stage + in_bytes};
     for (int b = 0; b < nbatch; ++b) {
-        const gb200_dual_out& out = outs[b];
-        const Off& o = off[(size_t)b];
-        const size_t n = (size_t)ics[b].n, nd = (size_t)ics[b].npartials;
-        if (!n) continue;
-        if (out.status) memcpy(out.status, stage + o.status, 4 * n);
-        if (out.lambda_max) memcpy(out.lambda_max, stage + o.lambda, 8 * n);
-        for (int k = 0; k < 4; ++k) {
-            if (out.x[k]) memcpy(out.x[k], stage + o.x[k], 8 * n);
-            if (out.v[k]) memcpy(out.v[k], stage + o.v[k], 8 * n);
-        }
-        if (out.g) memcpy(out.g, stage + o.g, 8 * n);
-        if (out.dg) memcpy(out.dg, stage + o.dg, 8 * n * nd);
-        if (out.rho) memcpy(out.rho, stage + o.rho, 8 * n);
-        if (out.drho) memcpy(out.drho, stage + o.drho, 8 * n * nd);
-        if (out.naccept) memcpy(out.naccept, stage + o.nacc, 4 * n);
-        if (out.nreject) memcpy(out.nreject, stage + o.nrej, 4 * n);
-        if (out.flags) memcpy(out.flags, stage + o.flags, 4 * n);
+        layout(b, host_in, host_out, S, Sio);
+        if (ics[b].n)
+            dual_arrays(outs[b], Sio, ics[b].n, ics[b].npartials, [&](auto* h, auto* f, int64_t n) { if (h) memcpy(h, f, (size_t)n * sizeof(*f)); });
     }
     float tot = 0;
     cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
@@ -1255,6 +1160,13 @@ int gb200_trace_dual(gb200_ctx* ctx, const gb200_problem* p, const gb200_dual_ic
     if (!p || !ic || !out) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null argument");
     const gb200_plunging_table* pls[1] = {plunging};
     return gb200_trace_dual_batch(ctx, 1, p, ic, norm_mode, pls, out);
+}
+
+// the binned line profile to the caller: flux ./ sum(flux) (line-profiles.jl:197), or the raw sums for a multi-rank caller
+static void normalise_flux(const std::vector<double>& h, const gb200_lineprofile_opts* opts, double* flux) {
+    double tot = 0;
+    for (double v : h) tot += v;
+    for (size_t b = 0; b < h.size(); ++b) flux[b] = opts->normalise ? h[b] / tot : h[b];
 }
 
 static int lineprofile_common(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic, const gb200_range* rg, const gb200_emissivity* em,
@@ -1311,9 +1223,7 @@ static int lineprofile_common(gb200_ctx* ctx, const gb200_problem* p, const gb20
         std::vector<double> h((size_t)nbins);
         CU(ctx, cudaMemcpyAsync(h.data(), dflux, sizeof(double) * nbins, cudaMemcpyDeviceToHost, stream));
         CU(ctx, cudaStreamSynchronize(stream));
-        double tot = 0;
-        for (int b = 0; b < nbins; ++b) tot += h[(size_t)b];
-        for (int b = 0; b < nbins; ++b) flux[b] = opts->normalise ? h[(size_t)b] / tot : h[(size_t)b]; // flux ./ sum(flux), line-profiles.jl:197
+        normalise_flux(h, opts, flux);
     }
     if (async) { ctx->stats.rays = rg->count; return end_async_call(ctx, stream); }
     return finish_stats(ctx, rg->count);
@@ -1376,11 +1286,7 @@ struct gb200_comm {
 
 // rank d's share of the rays: whole strips of four image columns / theta-rows, strip d, d + n, ... (DESIGN.md section 6)
 static gb200_range shard_range(const gb200_ic* ic, int d, int n) {
-    int64_t h = 0;
-    if (ic->kind == GB200_IC_RENDER_GRID) h = ic->height;
-    else if (ic->kind == GB200_IC_POLAR_PLANE) h = ic->width;
-    else if (ic->kind == GB200_IC_CARTESIAN_PLANE) h = 2 * (ic->height / 2) - 1;
-    const int64_t strip = GB_TILE_C * h;
+    const int64_t strip = GB_TILE_C * strip_height(ic);
     if (n == 1) return gb200_range{0, ic->n, 1, 1};
     if (strip > 0 && ic->n % strip == 0) {
         const int64_t nstrips = ic->n / strip;
@@ -1468,9 +1374,7 @@ int gb200_comm_lineprofile(gb200_comm* c, const gb200_problem* p, const gb200_ic
         CU(c->ctx[(size_t)d], cudaSetDevice(c->ctx[(size_t)d]->device));
         CU(c->ctx[(size_t)d], cudaStreamSynchronize(c->ctx[(size_t)d]->stream));
     }
-    double tot = 0;
-    for (int b = 0; b < nbins; ++b) tot += h[(size_t)b];
-    for (int b = 0; b < nbins; ++b) flux_out[b] = opts->normalise ? h[(size_t)b] / tot : h[(size_t)b];
+    normalise_flux(h, opts, flux_out);
     return GB200_OK;
 }
 
@@ -1491,11 +1395,7 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
         rg = shard_range(ic, d, n);
         if (rg.block < 1) rg.block = 1;
         CU(ctx, cudaSetDevice(ctx->device));
-        while (ctx->pool_streams.size() < 2) {
-            cudaStream_t st;
-            CU(ctx, cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-            ctx->pool_streams.push_back(st);
-        }
+        { int rc = ensure_streams(ctx, 2); if (rc) return rc; }
         dimg[(size_t)d].resize((size_t)npf);
         for (int k = 0; k < npf; ++k) {
             void* dv = nullptr;
@@ -1531,13 +1431,7 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
         const gb200_range& rg = rgs[(size_t)d];
         if (rg.count == 0) continue;
         CU(ctx, cudaSetDevice(ctx->device));
-        const size_t total = sizeof(double) * (size_t)rg.count * (size_t)npf;
-        if (ctx->stage_cap < total) {
-            if (ctx->stage) cudaFreeHost(ctx->stage);
-            ctx->stage = nullptr; ctx->stage_cap = 0;
-            CU(ctx, cudaMallocHost(&ctx->stage, total + 256));
-            ctx->stage_cap = total;
-        }
+        int rc = ensure_stage(ctx, sizeof(double) * (size_t)rg.count * (size_t)npf); if (rc) return rc;
     }
     for (int ch = 0; ch < K; ++ch)
         for (int d = 0; d < n; ++d) {
