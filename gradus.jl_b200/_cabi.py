@@ -26,6 +26,7 @@ GRID_LINEAR, GRID_GEOMETRIC, GRID_INVERSE = 0, 1, 2
 PF_SHADOW, PF_REDSHIFT, PF_DISC_RADIUS, PF_COORDINATE_TIME, PF_STATUS, PF_AFFINE_TIME, PF_RADIUS = 0, 1, 2, 3, 4, 5, 6
 PF_EQUATORIAL_CROSSINGS = 7
 EMISSIVITY_POWERLAW, EMISSIVITY_TABLE = 0, 1
+PROFILE_TIME_NAN_LINEAR, PROFILE_TIME_LINEAR = 0, 1
 FLAG_MAXITERS, FLAG_DT_MIN, FLAG_UNSTABLE = 1, 2, 4
 
 _dp = C.POINTER(C.c_double)
@@ -83,6 +84,17 @@ class LineProfileOpts(C.Structure):
     _fields_ = [("min_re", C.c_double), ("max_re", C.c_double), ("normalise", C.c_int32), ("bin_right_closed", C.c_int32)]
 
 
+class DiscProfile(C.Structure):
+    """gb200_disc_profile: ε(ρ) and the source-to-disc arrival time t(ρ) of the binned lag transfer function."""
+
+    _fields_ = [("emissivity", Emissivity), ("time_kind", C.c_int32), ("n", C.c_int32), ("r", _dp), ("t", _dp)]
+
+
+class LagTransferOpts(C.Structure):
+    _fields_ = [("E0", C.c_double), ("t0", C.c_double), ("energy_lims", C.c_double * 2), ("time_lims", C.c_double * 2),
+                ("N_E", C.c_int32), ("N_t", C.c_int32)]
+
+
 class DualIC(C.Structure):
     """gb200_dual_ic: impact parameters with seeded partials (forward-mode traces)."""
 
@@ -112,6 +124,7 @@ EXPORTED_SYMBOLS = (
     "gb200_render_batch", "gb200_render_device", "gb200_lineprofile_device", "gb200_fp64_peak", "gb200_fp64_issue_probe", "gb200_debug_rhs", "gb200_debug_math", "gb200_debug_math_lo",
     "gb200_trace_dual", "gb200_trace_dual_batch", "gb200_trace_target",
     "gb200_set_cross_section", "gb200_bucket2d", "gb200_comm_init", "gb200_comm_destroy", "gb200_comm_size", "gb200_comm_context", "gb200_comm_lineprofile", "gb200_comm_render",
+    "gb200_lagtransfer", "gb200_comm_lagtransfer",
 )
 
 
@@ -260,6 +273,10 @@ def load():
     lib.gb200_comm_lineprofile.argtypes = [vp, C.POINTER(Problem), C.POINTER(IC), C.POINTER(Emissivity), C.POINTER(PlungingTable), _dp, C.c_int32,
                                            C.POINTER(LineProfileOpts), _dp]
     lib.gb200_comm_render.argtypes = [vp, C.POINTER(Problem), C.POINTER(IC), _ip, C.c_int32, C.POINTER(PlungingTable), C.POINTER(_dp)]
+    lag = [C.POINTER(Problem), C.POINTER(IC), C.POINTER(DiscProfile), C.POINTER(PlungingTable), C.POINTER(LagTransferOpts), _dp, _dp, _dp,
+           C.POINTER(C.c_int64)]
+    lib.gb200_lagtransfer.argtypes = [vp] + lag
+    lib.gb200_comm_lagtransfer.argtypes = [vp] + lag
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)
         if name not in ("gb200_destroy", "gb200_last_error", "gb200_version", "gb200_comm_destroy", "gb200_comm_context"):

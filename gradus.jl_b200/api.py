@@ -1234,11 +1234,20 @@ class PowerLawEmissivity:
 
     index: float = 3.0
 
+    def __call__(self, r):
+        return np.asarray(r, np.float64) ** -float(self.index)
+
 
 @dataclass(frozen=True)
 class TabulatedEmissivity:
+    """ε(r) by linear interpolation in (r, eps), clamped to the ends"""
+
     r: Any
     eps: Any
+
+    def __call__(self, r):
+        rs = np.asarray(self.r, np.float64)
+        return np.interp(np.clip(r, rs[0], rs[-1]), rs, np.asarray(self.eps, np.float64))
 
 
 def lineprofile(bins, emissivity, m, position, d, method=None, *, lambda_max=None, min_re=None, max_re=50.0,

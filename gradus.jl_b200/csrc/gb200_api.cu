@@ -342,7 +342,8 @@ static int pool_get(gb200_ctx* ctx, size_t slot, size_t bytes, void** out) {
 // pool slots
 enum { SL_STATUS = 0, SL_LAMBDA, SL_X0, SL_V0 = SL_X0 + 4, SL_XI0 = SL_V0 + 4, SL_VI0 = SL_XI0 + 4, SL_NACC = SL_VI0 + 4, SL_NREJ, SL_FLAGS,
        SL_IMG0, SL_G = SL_IMG0 + GB_MAX_PF, SL_F, SL_EX0, SL_EV0 = SL_EX0 + 4, SL_BINS = SL_EV0 + 4, SL_PARTIAL, SL_FLUX, SL_EMR, SL_EME,
-       SL_PL0, SL_SCRATCH = SL_PL0 + 4, SL_BATCH, SL_BATCH_QUEUE, SL_COUNT };
+       SL_PL0, SL_SCRATCH = SL_PL0 + 4, SL_BATCH, SL_BATCH_QUEUE,
+       SL_LAG_SAMPLES, SL_LAG_PARTIAL, SL_LAG_SCAL, SL_LAG_CELLS, SL_LAG_OUT, SL_LAG_PROF, SL_COUNT };
 
 // The output arrays of gb200_endpoints: f(host array, GbParams field the kernel writes it through, pool slot of a single
 // call) for each, null host arrays included.  Every copy, binding and layout of endpoints goes through this one list.
@@ -1484,6 +1485,174 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
     cleanup2();
     cleanup();
     return GB200_OK;
+}
+
+// ---------------------------------------------------------------- binned lag-energy transfer function
+static int validate_lims(gb200_ctx* ctx, const double* lims, const char* axis) {
+    if (std::isnan(lims[0]) && std::isnan(lims[1])) return GB200_OK; // automatic: min / max over the hits
+    if (!std::isfinite(lims[0]) || !std::isfinite(lims[1]) || !(lims[0] < lims[1]))
+        return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "%s limits must be finite with lo < hi, or both NaN (got %g, %g)", axis, lims[0], lims[1]);
+    return GB200_OK;
+}
+
+static int validate_ascending(gb200_ctx* ctx, const double* r, int32_t n, const char* what) {
+    if (n < 2 || !r) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "%s needs n >= 2 radii", what);
+    for (int k = 1; k < n; ++k)
+        if (!(r[k] > r[k - 1])) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "%s radii must be strictly ascending (index %d)", what, k);
+    return GB200_OK;
+}
+
+// Everything that can be rejected without tracing, for every device, before the first launch.
+static int validate_lagtransfer(const std::vector<gb200_ctx*>& ctxs, const gb200_problem* p, const gb200_ic* ic, const gb200_disc_profile* pr,
+                                const gb200_lagtransfer_opts* o, const double* time_edges, const double* energy_edges, const double* tf, const int64_t* hits) {
+    gb200_ctx* ctx = ctxs[0];
+    int rc = validate(ctx, p, ic); if (rc) return rc;
+    if (ic->kind != GB200_IC_POLAR_PLANE)
+        return fail(ctx, GB200_ERR_UNSUPPORTED, "the lag transfer function needs a PolarPlane: its r^2 area weight is defined only there");
+    if (!pr || !o || !time_edges || !energy_edges || !tf || !hits) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null argument");
+    if (o->N_E < 2 || o->N_t < 2 || (int64_t)o->N_E * o->N_t > (1 << 26))
+        return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need N_E, N_t >= 2 and N_E * N_t <= 2^26 (got %d x %d)", o->N_E, o->N_t);
+    if (!std::isfinite(o->E0) || !(o->E0 > 0)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "E0 must be positive and finite (got %g)", o->E0);
+    if (!std::isfinite(o->t0)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "t0 must be finite");
+    rc = validate_lims(ctx, o->energy_lims, "energy"); if (rc) return rc;
+    rc = validate_lims(ctx, o->time_lims, "time"); if (rc) return rc;
+    const gb200_emissivity& em = pr->emissivity;
+    if (em.kind == GB200_EMISSIVITY_POWERLAW) {
+        if (!std::isfinite(em.index)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "emissivity index must be finite");
+    } else if (em.kind == GB200_EMISSIVITY_TABLE) {
+        rc = validate_ascending(ctx, em.r, em.n, "emissivity table"); if (rc) return rc;
+        if (!em.eps) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "emissivity table without values");
+    } else return fail(ctx, GB200_ERR_UNSUPPORTED, "emissivity kind %d", em.kind);
+    if (pr->time_kind != GB200_PROFILE_TIME_NAN_LINEAR && pr->time_kind != GB200_PROFILE_TIME_LINEAR)
+        return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "profile time kind %d", pr->time_kind);
+    rc = validate_ascending(ctx, pr->r, pr->n, "arrival-time profile"); if (rc) return rc;
+    if (!pr->t) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "arrival-time profile without times");
+    // what render_common would only find after it has started on the first device
+    double r_isco;
+    if (gb200_isco(p->metric_kind, p->metric_params, &r_isco)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "no ISCO found for this metric (is it a naked singularity?)");
+    for (gb200_ctx* c : ctxs)
+        if (p->geometry_kind == GB200_GEOMETRY_THICK_TABLE && c->cs_n < 2)
+            return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "GB200_GEOMETRY_THICK_TABLE needs a table on device %d: call gb200_set_cross_section first", c->device);
+    return GB200_OK;
+}
+
+// gb200_lagtransfer over the devices of `ctxs` (nccl: one communicator per device when there are several).  Every device
+// traces its strips and forms its samples; the scalars (limits, hit count, max |f|) are all-reduced; every device bins into
+// integer cells with the same edges and scale; the cells are all-reduced and device 0 finishes and copies the result.
+static int lagtransfer_run(const std::vector<gb200_ctx*>& ctxs, const ncclComm_t* nccl, const gb200_problem* p, const gb200_ic* ic,
+                           const gb200_disc_profile* pr, const gb200_plunging_table* pl, const gb200_lagtransfer_opts* o,
+                           double* time_edges, double* energy_edges, double* tf, int64_t* hits) {
+    const int n = (int)ctxs.size();
+    for (gb200_ctx* c : ctxs) c->stats = gb200_stats{};
+    int rc = validate_lagtransfer(ctxs, p, ic, pr, o, time_edges, energy_edges, tf, hits); if (rc) return rc;
+    static const int32_t pfs[4] = {GB200_PF_STATUS, GB200_PF_REDSHIFT, GB200_PF_DISC_RADIUS, GB200_PF_COORDINATE_TIME}; // lagtransfer's
+    const GbLagLimits L{{o->energy_lims[0], o->energy_lims[1]}, {o->time_lims[0], o->time_lims[1]}, o->N_E, o->N_t};
+    const int ncell = o->N_E * o->N_t;
+    struct Dev {
+        int64_t count;
+        double* samples;
+        GbLagScalars* scal;
+        long long* cells; // ncell + 1: the last is the total
+        unsigned* counts;
+        double* out;      // tf (ncell) | eb (N_E) | tb (N_t)
+    };
+    std::vector<Dev> dv((size_t)n);
+    for (int d = 0; d < n; ++d) {
+        gb200_ctx* ctx = ctxs[(size_t)d];
+        Dev& D = dv[(size_t)d];
+        const gb200_range rg = shard_range(ic, d, n);
+        D.count = rg.count;
+        CU(ctx, cudaSetDevice(ctx->device));
+        double* img[4];
+        void* v;
+        for (int k = 0; k < 4; ++k) { rc = pool_get(ctx, SL_IMG0 + k, sizeof(double) * (size_t)rg.count + 8, &v); if (rc) return rc; img[k] = (double*)v; }
+        rc = render_common(ctx, p, ic, &rg, pfs, 4, pl, img, true, ctx->stream, 1); if (rc) return rc;
+        GbParams P;
+        fill_params(p, ic, &rg, P);
+        rc = upload_ic_and_tables(ctx, ic, nullptr, &pr->emissivity, P); if (rc) return rc;
+        rc = pool_get(ctx, SL_LAG_PROF, sizeof(double) * 2 * (size_t)pr->n, &v); if (rc) return rc;
+        const GbLagProfile gp{pr->time_kind, pr->n, (const double*)v, (const double*)v + pr->n};
+        CU(ctx, cudaMemcpyAsync((void*)gp.r, pr->r, sizeof(double) * (size_t)pr->n, cudaMemcpyHostToDevice, ctx->stream));
+        CU(ctx, cudaMemcpyAsync((void*)gp.t, pr->t, sizeof(double) * (size_t)pr->n, cudaMemcpyHostToDevice, ctx->stream));
+        const int nblocks = (int)std::max<int64_t>(1, std::min<int64_t>((rg.count + 255) / 256, (int64_t)ctx->sm_count * 4));
+        rc = pool_get(ctx, SL_LAG_SAMPLES, sizeof(double) * 3 * (size_t)rg.count + 8, &v); if (rc) return rc;
+        D.samples = (double*)v;
+        rc = pool_get(ctx, SL_LAG_PARTIAL, sizeof(GbLagScalars) * (size_t)nblocks, &v); if (rc) return rc;
+        GbLagScalars* partial = (GbLagScalars*)v;
+        rc = pool_get(ctx, SL_LAG_SCAL, sizeof(GbLagScalars), &v); if (rc) return rc;
+        D.scal = (GbLagScalars*)v;
+        CU(ctx, gb200_launch_lag_samples(P, img, gp, o->E0, rg.count, D.samples, partial, nblocks, D.scal, ctx->stream));
+        ctx->stats.launches += 2;
+    }
+    if (n > 1) {
+        NC(g_nccl.GroupStart());
+        for (int d = 0; d < n; ++d) {
+            GbLagScalars* s = dv[(size_t)d].scal;
+            const cudaStream_t st = ctxs[(size_t)d]->stream;
+            ncclResult_t r = g_nccl.AllReduce(s->mn, s->mn, 2, ncclDouble, ncclMin, nccl[d], st);
+            if (r == ncclSuccess) r = g_nccl.AllReduce(s->mx, s->mx, 4, ncclDouble, ncclMax, nccl[d], st);
+            if (r == ncclSuccess) r = g_nccl.AllReduce(&s->hits, &s->hits, 1, ncclInt64, ncclSum, nccl[d], st);
+            if (r != ncclSuccess) { g_nccl.GroupEnd(); return fail(nullptr, GB200_ERR_CUDA, "ncclAllReduce: %s", g_nccl.GetErrorString(r)); }
+        }
+        NC(g_nccl.GroupEnd());
+    }
+    for (int d = 0; d < n; ++d) {
+        gb200_ctx* ctx = ctxs[(size_t)d];
+        Dev& D = dv[(size_t)d];
+        CU(ctx, cudaSetDevice(ctx->device));
+        void* v;
+        rc = pool_get(ctx, SL_LAG_CELLS, sizeof(long long) * (size_t)(ncell + 1) + sizeof(unsigned) * (size_t)ncell, &v); if (rc) return rc;
+        D.cells = (long long*)v;
+        D.counts = (unsigned*)(D.cells + ncell + 1);
+        rc = pool_get(ctx, SL_LAG_OUT, sizeof(double) * (size_t)(ncell + o->N_E + o->N_t), &v); if (rc) return rc;
+        D.out = (double*)v;
+        const int nblocks = (int)std::max<int64_t>(1, std::min<int64_t>((D.count + 255) / 256, (int64_t)ctx->sm_count * 8));
+        CU(ctx, gb200_launch_lag_bin(D.scal, L, D.out + ncell, D.out + ncell + o->N_E, D.samples, D.count, D.cells, D.counts, nblocks, ctx->stream));
+        ctx->stats.launches += D.count > 0 ? 2 : 1;
+    }
+    if (n > 1) {
+        NC(g_nccl.GroupStart());
+        for (int d = 0; d < n; ++d) {
+            const Dev& D = dv[(size_t)d];
+            const cudaStream_t st = ctxs[(size_t)d]->stream;
+            ncclResult_t r = g_nccl.AllReduce(D.cells, D.cells, (size_t)ncell + 1, ncclInt64, ncclSum, nccl[d], st);
+            if (r == ncclSuccess) r = g_nccl.AllReduce(D.counts, D.counts, (size_t)ncell, ncclUint32, ncclSum, nccl[d], st);
+            if (r != ncclSuccess) { g_nccl.GroupEnd(); return fail(nullptr, GB200_ERR_CUDA, "ncclAllReduce: %s", g_nccl.GetErrorString(r)); }
+        }
+        NC(g_nccl.GroupEnd());
+    }
+    gb200_ctx* c0 = ctxs[0];
+    const Dev& D0 = dv[0];
+    GbLagScalars s;
+    CU(c0, cudaSetDevice(c0->device));
+    CU(c0, gb200_launch_lag_finish(D0.cells, D0.counts, ncell, D0.scal, D0.out, c0->stream));
+    c0->stats.launches += 1;
+    CU(c0, cudaMemcpyAsync(tf, D0.out, sizeof(double) * (size_t)ncell, cudaMemcpyDeviceToHost, c0->stream));
+    CU(c0, cudaMemcpyAsync(energy_edges, D0.out + ncell, sizeof(double) * (size_t)o->N_E, cudaMemcpyDeviceToHost, c0->stream));
+    CU(c0, cudaMemcpyAsync(time_edges, D0.out + ncell + o->N_E, sizeof(double) * (size_t)o->N_t, cudaMemcpyDeviceToHost, c0->stream));
+    CU(c0, cudaMemcpyAsync(&s, D0.scal, sizeof s, cudaMemcpyDeviceToHost, c0->stream));
+    for (int d = 0; d < n; ++d) {
+        CU(ctxs[(size_t)d], cudaSetDevice(ctxs[(size_t)d]->device));
+        rc = finish_stats(ctxs[(size_t)d], dv[(size_t)d].count); if (rc) return rc;
+    }
+    if (s.status == GB_LAG_NONFINITE) return fail(c0, GB200_ERR_INVALID_ARGUMENT, "a hit has a non-finite energy, time or flux (a redshift without a velocity field?)");
+    if (s.status == GB_LAG_NO_HITS) return fail(c0, GB200_ERR_INVALID_ARGUMENT, "automatic limits need hits: no ray reached the disc");
+    if (s.status == GB_LAG_DEGENERATE) return fail(c0, GB200_ERR_INVALID_ARGUMENT, "automatic limits need min < max over the hits");
+    for (int j = 0; j < o->N_t; ++j) time_edges[j] -= o->t0;
+    *hits = s.hits;
+    return GB200_OK;
+}
+
+int gb200_lagtransfer(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic, const gb200_disc_profile* pr, const gb200_plunging_table* pl,
+                      const gb200_lagtransfer_opts* opts, double* time_edges, double* energy_edges, double* tf, int64_t* hits) {
+    if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
+    return lagtransfer_run({ctx}, nullptr, p, ic, pr, pl, opts, time_edges, energy_edges, tf, hits);
+}
+
+int gb200_comm_lagtransfer(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic, const gb200_disc_profile* pr, const gb200_plunging_table* pl,
+                           const gb200_lagtransfer_opts* opts, double* time_edges, double* energy_edges, double* tf, int64_t* hits) {
+    if (!c) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null communicator");
+    return lagtransfer_run(c->ctx, c->nccl.data(), p, ic, pr, pl, opts, time_edges, energy_edges, tf, hits);
 }
 
 int gb200_bucket2d(gb200_ctx* ctx, int64_t n, const double* x, const double* y, const double* w, const double* xbins, int32_t nx,

@@ -31,3 +31,29 @@ struct GbDualIO {
 cudaError_t gb200_launch_dual(const GbParams& P, const GbDualIO& io, cudaStream_t stream);
 // closest approach to a target point (optimize_for_target's objective): the generic integrator over the rays of P
 cudaError_t gb200_launch_target(const GbParams& P, cudaStream_t stream);
+
+// binned lag-energy transfer function (gb200_lag.cu; host side gb200_lagtransfer in gb200_api.cu)
+struct GbLagProfile { // t(rho) of gb200_disc_profile on the device
+    int32_t time_kind, n;
+    const double* r;
+    const double* t;
+};
+struct GbLagLimits { // (lo, hi) of each axis, NaN = min / max over the hits; N_E, N_t >= 2
+    double energy[2], time[2];
+    int32_t N_E, N_t;
+};
+enum { GB_LAG_NONFINITE = 1, GB_LAG_NO_HITS = 2, GB_LAG_DEGENERATE = 3 };
+struct GbLagScalars {
+    // reduced over the hits of every device (the NCCL all-reduce works on these three groups)
+    double mn[2];   // min E, min T (finite samples)
+    double mx[4];   // max E, max T, max |f| (finite samples), 1 if any hit has a non-finite E, T or f
+    long long hits;
+    // derived from them by the edges kernel, the same on every device
+    double scale, dedt; // fixed-point scale, (eb[1] - eb[0]) (tb[1] - tb[0])
+    int32_t status;     // 0 or GB_LAG_*
+};
+cudaError_t gb200_launch_lag_samples(const GbParams& P, const double* const* img, const GbLagProfile& pr, double E0, int64_t n, double* samples,
+                                     GbLagScalars* partial, int nblocks, GbLagScalars* scal, cudaStream_t stream);
+cudaError_t gb200_launch_lag_bin(GbLagScalars* scal, const GbLagLimits& L, double* eb, double* tb, const double* samples, int64_t n,
+                                 long long* cells, unsigned* counts, int nblocks, cudaStream_t stream);
+cudaError_t gb200_launch_lag_finish(const long long* cells, const unsigned* counts, int ncell, const GbLagScalars* scal, double* tf, cudaStream_t stream);

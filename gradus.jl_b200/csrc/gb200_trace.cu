@@ -784,12 +784,6 @@ cudaError_t gb200_launch_hist(const double* g, const double* f, int64_t n, const
 // samples are split over GPUs) the weights are accumulated as 64-bit fixed-point integers -- integer addition is
 // associative -- with the scale chosen from sum |w|, so that the quantisation (2^-62 of the total per sample) is far below
 // the rounding of a floating-point sum.  Lanes of a warp that hit the same cell are combined first (__match_any_sync).
-__device__ __forceinline__ int gb_simple_bucket(const double* __restrict__ bins, int nb, double v) {
-    int lo = 0, hi = nb; // first idx with bins[idx] > v, minus 1 (searchsortedlast), clamped to the ends
-    while (lo < hi) { const int mid = (lo + hi) >> 1; if (bins[mid] <= v) lo = mid + 1; else hi = mid; }
-    const int b = lo - 1;
-    return b < 0 ? 0 : (b > nb - 1 ? nb - 1 : b);
-}
 __global__ void __launch_bounds__(256) gb200_bucket2d_kernel(const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ w,
                                                              int64_t n, const double* __restrict__ xb, int nx, const double* __restrict__ yb, int ny,
                                                              double scale, long long* __restrict__ acc) {

@@ -3,9 +3,12 @@
 
 Both legs are endpoint traces on the device: source → disc through `tracecorona` (explicit ICs), observer → disc through
 one fused `gb200_render` over the image plane that returns (status, g, ρ, t) per ray, so no endpoint arrays cross the
-bus.  Binning is the reference's `Buckets.Simple` in two dimensions (slot i takes bins[i] ≤ v < bins[i+1], clamped)."""
+bus.  Binning is the reference's `Buckets.Simple` in two dimensions (slot i takes bins[i] ≤ v < bins[i+1], clamped).
+`binned_lagtransfer` returns what `binflux(lagtransfer(...))` returns with the binning on the device as well
+(`gb200_lagtransfer`), so no per-ray data reaches the host."""
 from __future__ import annotations
 
+import ctypes as C
 from dataclasses import dataclass
 from typing import Callable, Optional
 
@@ -145,6 +148,81 @@ def binflux(tf: LagTransferFunction, profile=None, *, E0=6.4, t0=None, **kwargs)
     F = f / f.sum()
     tb, eb, td = bin_transfer_function(t, tf.g * E0, F, **kwargs)
     return tb - t0, eb, td
+
+
+def _disc_profile_to_c(profile):
+    """-> (gb200_disc_profile, arrays it points into).  Raises TypeError for an ε the device cannot evaluate."""
+    if isinstance(profile, AnalyticRadialDiscProfile):
+        eps, r, t, kind = profile.eps, profile.t.t, profile.t.u, cabi.PROFILE_TIME_NAN_LINEAR
+        if profile.t.default != 0.0:
+            raise TypeError("binned_lagtransfer supports NaNLinearInterpolator's default fallback value 0 only")
+        if not isinstance(eps, (api.PowerLawEmissivity, api.TabulatedEmissivity)):
+            raise TypeError("an emissivity given as a Python callable cannot cross the C ABI: pass PowerLawEmissivity or "
+                            "TabulatedEmissivity, or use binflux(lagtransfer(...), profile)")
+    elif isinstance(profile, corona.RadialDiscProfile):
+        eps, r, t, kind = api.TabulatedEmissivity(profile.radii, profile.eps), profile.radii, profile.t, cabi.PROFILE_TIME_LINEAR
+    else:
+        raise TypeError(f"profile {type(profile).__name__} cannot be binned on the device: use binflux(lagtransfer(...), profile)")
+    keep = [np.ascontiguousarray(r, np.float64), np.ascontiguousarray(t, np.float64)]
+    c = cabi.DiscProfile()
+    if isinstance(eps, api.PowerLawEmissivity):
+        c.emissivity.kind, c.emissivity.index = cabi.EMISSIVITY_POWERLAW, float(eps.index)
+    else:
+        keep += [np.ascontiguousarray(eps.r, np.float64), np.ascontiguousarray(eps.eps, np.float64)]
+        c.emissivity.kind, c.emissivity.n = cabi.EMISSIVITY_TABLE, len(keep[2])
+        c.emissivity.r, c.emissivity.eps = cabi.dptr(keep[2]), cabi.dptr(keep[3])
+    c.time_kind, c.n, c.r, c.t = kind, len(keep[0]), cabi.dptr(keep[0]), cabi.dptr(keep[1])
+    return c, keep
+
+
+def binned_lagtransfer(m, x, d, model, profile=None, *, plane=None, max_t=None, n_samples=10_000, sampler=None, callback="default",
+                       E0=6.4, t0=None, N_E=300, N_t=300, energy_lims=None, time_lims=None, ensemble=None, **solver_opts):
+    """`binflux(lagtransfer(m, x, d, model; ...), profile; E0, t0, N_E, N_t, energy_lims, time_lims)` with the observer→disc
+    leg binned on the device (`gb200_lagtransfer`, or `gb200_comm_lagtransfer` over several devices): no per-ray data
+    reaches the host, and the histogram is summed in fixed point, so it is the same bits on any number of devices.
+    Returns (time edges - t0, energy edges, tf[N_E, N_t], number of observer→disc hits).  `profile=None` is ε = r⁻³ with the
+    coronal arrival times; an `AnalyticRadialDiscProfile` needs a `PowerLawEmissivity` or `TabulatedEmissivity` ε."""
+    x = np.asarray(x, np.float64)
+    if plane is None:
+        plane = api.PolarPlane(api.GeometricGrid(), Nr=800, Ntheta=800, r_max=50.0)
+    if not isinstance(plane, api.PolarPlane):
+        raise ValueError("lagtransfer is implemented for PolarPlane image planes")
+    if profile is not None:
+        _disc_profile_to_c(profile)  # reject what cannot cross the ABI before tracing
+    if max_t is None:
+        max_t = 2 * x[1]
+    if sampler is None:
+        sampler = corona.EvenSampler("both", "golden")
+    if callback == "default":
+        callback = api.domain_upper_hemisphere()
+    if t0 is None:
+        t0 = x[1]
+    ce = corona.tracecorona(m, d, model, lambda_max=max_t, n_samples=n_samples, sampler=sampler, callback=callback,
+                            ensemble=ensemble, **solver_opts)
+    if profile is None:
+        profile = AnalyticRadialDiscProfile.from_corona(api.PowerLawEmissivity(3.0), ce)
+    config = api.tracing_configuration(m, x, plane, d, (0.0, max_t), chart=api.chart_for_metric(m, 1.1 * x[1]),
+                                       callback=callback, ensemble=ensemble, **solver_opts)
+    p, ic = config.to_c()
+    prof, _keep = _disc_profile_to_c(profile)
+    nan = float("nan")
+    opts = cabi.LagTransferOpts(float(E0), float(t0), tuple(energy_lims) if energy_lims is not None else (nan, nan),
+                                tuple(time_lims) if time_lims is not None else (nan, nan), int(N_E), int(N_t))
+    plunging = api._auto_plunging(m, d, config.ensemble, True, None)
+    pl_ref = C.byref(plunging.c) if plunging is not None else None
+    tb, eb, tf, hits = np.zeros(int(N_t)), np.zeros(int(N_E)), np.zeros((int(N_E), int(N_t))), C.c_int64()
+    args = (C.byref(p), C.byref(ic), C.byref(prof), pl_ref, C.byref(opts), cabi.dptr(tb), cabi.dptr(eb), cabi.dptr(tf.reshape(-1)), C.byref(hits))
+    lib = cabi.load()
+    comm = config.ensemble.comm()
+    if comm is not None:
+        api._install_on_comm(comm, config.geometry)
+        cabi.check(lib.gb200_comm_lagtransfer(comm, *args))
+    else:
+        ctx = config.ensemble.ctx(config.ensemble.devices[0])
+        if hasattr(config.geometry, "install"):
+            config.geometry.install(ctx)
+        cabi.check(lib.gb200_lagtransfer(ctx, *args), ctx)
+    return tb, eb, tf, int(hits.value)
 
 
 def continuum_time(m, x, model, **kwargs):

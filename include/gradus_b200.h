@@ -396,6 +396,45 @@ int gb200_trace_dual_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* 
 int gb200_bucket2d(gb200_ctx* ctx, int64_t n, const double* x, const double* y, const double* w,
                    const double* xbins, int32_t nx, const double* ybins, int32_t ny, double* out);
 
+/* ---- binned lag-energy transfer function ------------------------------- */
+/* binflux(lagtransfer(m, x, d, model; plane, ...), profile; E0, t0, N_E, N_t, energy_lims, time_lims)
+   (src/transfer-functions/transfer-functions-2d.jl:100-122,163-242) from the same traces, binned on the device. */
+#define GB200_PROFILE_TIME_NAN_LINEAR 0 /* NaNLinearInterpolator (AnalyticRadialDiscProfile, corona/analytic.jl:1-40) */
+#define GB200_PROFILE_TIME_LINEAR 1     /* linear interpolation (RadialDiscProfile, corona/radial.jl:1-37) */
+
+typedef struct gb200_disc_profile { /* eps(rho) and the source-to-disc arrival time t(rho) */
+    gb200_emissivity emissivity;    /* POWERLAW or TABLE (r strictly ascending), as for gb200_lineprofile */
+    int32_t time_kind;              /* GB200_PROFILE_TIME_*; both clip rho to [r[0], r[n-1]] first */
+    int32_t n;                      /* >= 2 */
+    const double* r;                /* host, strictly ascending */
+    const double* t;
+} gb200_disc_profile;
+
+typedef struct gb200_lagtransfer_opts {
+    double E0;             /* line energy: E = g E0; positive and finite */
+    double t0;             /* subtracted from the returned time edges */
+    double energy_lims[2]; /* (lo, hi) with lo < hi, or both NaN: min and max of E over the hits */
+    double time_lims[2];   /* likewise for T */
+    int32_t N_E, N_t;      /* >= 2 each, N_E * N_t <= 2^26 as gb200_bucket2d */
+} gb200_lagtransfer_opts;
+
+/* Traces every ray of a GB200_IC_POLAR_PLANE `ic` (anything else: GB200_ERR_UNSUPPORTED, the r^2 area weight of
+   unnormalized_areas, image-planes/planes.jl:108-115, is defined only there) with the point functions of lagtransfer
+   (status, redshift, disc radius, coordinate time) and bins its hits -- rays with status IntersectedWithGeometry -- without
+   copying per-ray data to the host:
+     E = g E0,  T = t(rho) + t,  f = g^3 eps(rho) r^2  (r: the ray's polar-plane radius);
+     eb = linspace(E_lo, E_hi, N_E), tb = linspace(T_lo, T_hi, N_t) (edge k = k * step + lo, two roundings, the last = hi);
+     tf[i * N_t + j] = (sum of f over the hits in cell (i, j)) / (sum of f over all hits) / ((eb[1] - eb[0]) (tb[1] - tb[0])),
+   Buckets.Simple in both axes (cell i takes eb[i] <= E < eb[i+1], clamped at both ends), NaN where no hit with f != 0
+   landed.  time_edges = tb - t0 (N_t), energy_edges = eb (N_E), *hits = the number of hits.  f is summed as 64-bit fixed
+   point with scale 2^floor(62 - log2(H max|f|)) (H: hits), so the result does not depend on the order of summation or on
+   the number of devices.  GB200_ERR_INVALID_ARGUMENT also for automatic limits without hits or with min == max, and for
+   a hit whose E, T or f is not finite; these are found after the trace.  Geometry, callback and plunging-table rules are
+   those of gb200_render. */
+int gb200_lagtransfer(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic, const gb200_disc_profile* profile,
+                      const gb200_plunging_table* plunging, const gb200_lagtransfer_opts* opts,
+                      double* time_edges, double* energy_edges, double* tf, int64_t* hits);
+
 /* ---- device-resident variants (inputs/outputs stay in HBM) ------------- */
 /* Same as gb200_render but `d_images[k]` are DEVICE pointers on ctx's device and no
    host copy is made; work is enqueued on `cuda_stream` (a cudaStream_t cast to
@@ -422,9 +461,9 @@ int gb200_lineprofile_device(gb200_ctx* ctx, const gb200_problem* p, const gb200
 /* ---- several GPUs from ONE process (the Julia extension: EnsembleB200(devices)) ---------------------------- */
 /* One context per listed device plus, for more than one device, an NCCL communicator over them (ncclCommInitAll).  NCCL is
    opened at run time (dlopen "libnccl.so.2"): a single-GPU caller does not need it.  Rays are sharded by whole strips of
-   four image columns / theta-rows (strip d, d + ndev, ... on device d); there is no data-path collective except the
+   four image columns / theta-rows (strip d, d + ndev, ... on device d); the data-path collectives are the
    line-profile histogram, which is summed with one ncclAllReduce(sum, nbins doubles) on the devices' own streams
-   (SURVEY 8e).  torchrun-style callers (one process per GPU) use gb200_lineprofile_device + their own all-reduce instead. */
+   (SURVEY 8e), and the lag-energy histogram of gb200_comm_lagtransfer.  torchrun-style callers (one process per GPU) use gb200_lineprofile_device + their own all-reduce instead. */
 typedef struct gb200_comm gb200_comm;
 int gb200_comm_init(const int32_t* devices, int32_t ndev, gb200_comm** out);
 void gb200_comm_destroy(gb200_comm* comm);
@@ -438,6 +477,12 @@ int gb200_comm_lineprofile(gb200_comm* comm, const gb200_problem* p, const gb200
 /* rendergeodesics over all devices: images[k] -> ic->n doubles on the host in ray order (the (H, W) column-major image). */
 int gb200_comm_render(gb200_comm* comm, const gb200_problem* p, const gb200_ic* ic, const int32_t* pointfns, int32_t npf,
                       const gb200_plunging_table* plunging, double* const* images);
+/* gb200_lagtransfer over all devices: each bins its strips; the limits, hit count and max |f| are made global with
+   ncclAllReduce (min, max, sum) before binning, and the integer cells with one ncclAllReduce(sum), so the result is
+   bit-identical to gb200_lagtransfer on one device. */
+int gb200_comm_lagtransfer(gb200_comm* comm, const gb200_problem* p, const gb200_ic* ic, const gb200_disc_profile* profile,
+                           const gb200_plunging_table* plunging, const gb200_lagtransfer_opts* opts,
+                           double* time_edges, double* energy_edges, double* tf, int64_t* hits);
 
 /* Diagnostics: evaluate the device right-hand side (_second_order_ode_f, src/tracing/geodesic-problem.jl:87-92) for
    n states u (row-major n x 8) -> du (n x 8), and the kernel's branch-free elementary functions on n inputs

@@ -95,6 +95,12 @@ end
 struct CLineProfileOpts
     min_re::Float64; max_re::Float64; normalise::Int32; bin_right_closed::Int32
 end
+struct CDiscProfile
+    emissivity::CEmissivity; time_kind::Int32; n::Int32; r::Ptr{Float64}; t::Ptr{Float64}
+end
+struct CLagTransferOpts
+    E0::Float64; t0::Float64; energy_lims::NTuple{2,Float64}; time_lims::NTuple{2,Float64}; N_E::Int32; N_t::Int32
+end
 const NULL4 = ntuple(_ -> Ptr{Float64}(C_NULL), 4)
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -484,6 +490,68 @@ function lineprofile_b200(bins, ε, m::Gradus.AbstractMetric{T}, u, d;
 end
 
 """
+    lagtransfer_b200(m, u, d, r, t; linear_time = false, power_law_index = 3.0, ε = nothing, ensemble = EnsembleB200(),
+                     plane, max_t, E₀ = 6.4, t0 = u[2], N_E = 300, N_t = 300, energy_lims = nothing, time_lims = nothing,
+                     callback, solver_args...)
+
+`binflux(lagtransfer(m, u, d, model; plane, max_t, ...), profile; E₀, t0, N_E, N_t, energy_lims, time_lims)`
+(src/transfer-functions/transfer-functions-2d.jl:100-122,163-242) with the observer→disc leg traced and binned on the
+device (`gb200_lagtransfer`; `gb200_comm_lagtransfer` over several devices, bit-identical).  The profile crosses the ABI
+as data: `r`, `t` are its arrival-time knots (for `AnalyticRadialDiscProfile` the coronal geodesics' ρ sorted ascending and
+their coordinate times, interpolated as its NaN-linear interpolator; `linear_time = true` for `RadialDiscProfile`), `ε`
+a power law (`power_law_index`) or, when `ε = (radii, values)`, a clamped linear table.  Returns
+`(time_edges .- t0, energy_edges, tf, hits)`.  Not run: there is no Julia toolchain where this binding was written; the
+Python mirror `binned_lagtransfer` is the tested form.
+"""
+function lagtransfer_b200(m::Gradus.AbstractMetric{T}, u, d, r, t; linear_time = false, power_law_index = 3.0, ε = nothing,
+                          ensemble::EnsembleB200 = EnsembleB200(), max_t = 2 * u[2],
+                          plane::PolarPlane = PolarPlane(GeometricGrid(); Nr = 800, Nθ = 800, r_max = 50.0),
+                          E₀ = 6.4, t0 = u[2], N_E = 300, N_t = 300, energy_lims = nothing, time_lims = nothing,
+                          callback = Gradus.domain_upper_hemisphere(), solver_args...) where {T}
+    trace = Gradus.TraceGeodesic()
+    chart = Gradus.chart_for_metric(m, 1.1 * u[2])
+    config, solver_opts = Gradus.tracing_configuration(trace, m, u, plane, d, (0.0, max_t); chart = chart, callback = callback,
+                                                       ensemble = ensemble, solver_args...)
+    problem = Gradus.assemble_tracing_problem(trace, config)
+    p = _problem(config, problem.prob; mu = 0.0, solver_opts...)
+    ic = _plane_ic(plane)
+    rv, tv = collect(Float64, r), collect(Float64, t)
+    er = isnothing(ε) ? Float64[] : collect(Float64, ε[1])
+    ev = isnothing(ε) ? Float64[] : collect(Float64, ε[2])
+    tb, eb, tf = zeros(Float64, N_t), zeros(Float64, N_E), zeros(Float64, N_t, N_E) # column-major: tf[j, i] = cell (i, j)
+    hits = Ref{Int64}(0)
+    lims(l) = isnothing(l) ? (NaN, NaN) : (Float64(l[1]), Float64(l[2]))
+    opts = CLagTransferOpts(E₀, t0, lims(energy_lims), lims(time_lims), N_E, N_t)
+    GC.@preserve rv tv er ev tb eb tf begin
+        emis = isnothing(ε) ? CEmissivity(0, 0, Float64(power_law_index), C_NULL, C_NULL) :
+               CEmissivity(1, length(er), 0.0, pointer(er), pointer(ev))
+        prof = CDiscProfile(emis, linear_time ? 1 : 0, length(rv), pointer(rv), pointer(tv))
+        if length(ensemble.devices) == 1
+            ctx = _context(ensemble, 1)
+            _install_geometry(ctx, d)
+            _check(ccall((:gb200_lagtransfer, libgradus_b200), Cint,
+                         (Ptr{Cvoid}, Ref{CProblem}, Ref{CIC}, Ref{CDiscProfile}, Ptr{Cvoid}, Ref{CLagTransferOpts}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ref{Int64}),
+                         ctx, p, ic, prof, C_NULL, opts, tb, eb, tf, hits), ctx)
+        else
+            comm = Ref{Ptr{Cvoid}}(C_NULL)
+            devs = Int32.(ensemble.devices)
+            _check(ccall((:gb200_comm_init, libgradus_b200), Cint, (Ptr{Int32}, Int32, Ref{Ptr{Cvoid}}), devs, length(devs), comm), C_NULL)
+            try
+                for i = 0:length(devs)-1
+                    _install_geometry(ccall((:gb200_comm_context, libgradus_b200), Ptr{Cvoid}, (Ptr{Cvoid}, Int32), comm[], i), d)
+                end
+                _check(ccall((:gb200_comm_lagtransfer, libgradus_b200), Cint,
+                             (Ptr{Cvoid}, Ref{CProblem}, Ref{CIC}, Ref{CDiscProfile}, Ptr{Cvoid}, Ref{CLagTransferOpts}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ref{Int64}),
+                             comm[], p, ic, prof, C_NULL, opts, tb, eb, tf, hits), C_NULL)
+            finally
+                ccall((:gb200_comm_destroy, libgradus_b200), Cvoid, (Ptr{Cvoid},), comm[])
+            end
+        end
+    end
+    tb, eb, permutedims(tf), hits[]
+end
+
+"""
     optimize_for_target_b200(target, m, x0; ensemble, d_tol = 1e-2, max_time = 2x0[2], p0 = (0.0, 0.0), window, grid = 33, kwargs...)
 
 `Gradus.optimize_for_target` (src/tracing/precision-solvers.jl:512-531) with the device under it: instead of one trace per
@@ -533,5 +601,5 @@ function optimize_for_target_b200(target, m::Gradus.AbstractMetric{T}, x0; ensem
     best[2], best[3], best[4], best[1]
 end
 
-export EnsembleB200, B200PointFunction, ImageOrder, equatorial_crossings, lineprofile_b200, optimize_for_target_b200
+export EnsembleB200, B200PointFunction, ImageOrder, equatorial_crossings, lineprofile_b200, lagtransfer_b200, optimize_for_target_b200
 end # module
