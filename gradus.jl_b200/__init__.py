@@ -5,7 +5,7 @@ of the reference's public API that sits on the per-ray integration path:
 
     tracegeodesics   (src/tracing/tracing.jl:66-80)
     rendergeodesics  (src/rendering/rendering.jl:28-54)
-    lineprofile      (src/line-profiles.jl:152-198, BinningMethod)
+    lineprofile      (src/line-profiles.jl:121-198, BinningMethod and TransferFunctionMethod)
 
 with the same argument meaning, defaults and error behaviour, and a new ensemble type
 `EnsembleB200` next to `EnsembleEndpointThreads` (src/Gradus.jl:412).  All compute goes
@@ -36,6 +36,7 @@ from .api import (  # noqa: F401
     ShakuraSunyaev,
     StatusCodes,
     TabulatedEmissivity,
+    TransferFunctionMethod,
     ThickDisc,
     PolishDoughnut,
     ThinDisc,

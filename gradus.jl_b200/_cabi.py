@@ -95,6 +95,23 @@ class LagTransferOpts(C.Structure):
                 ("N_E", C.c_int32), ("N_t", C.c_int32)]
 
 
+class TfBranches(C.Structure):
+    """gb200_tf_branches: one InterpolatingTransferBranches, flattened (branch 2k lower, 2k+1 upper of radius k)."""
+
+    _fields_ = [("n_radii", C.c_int32), ("reserved", C.c_int32), ("r_e", _dp), ("gmin", _dp), ("gmax", _dp),
+                ("off", C.POINTER(C.c_int64)), ("gs", _dp), ("f", _dp), ("t", _dp)]
+
+
+class TfModel(C.Structure):
+    _fields_ = [("table", C.c_int32), ("n_radii", C.c_int32), ("radii", _dp), ("rmin", C.c_double), ("g_scale", C.c_double),
+                ("profile", DiscProfile)]
+
+
+class TfQuadOpts(C.Structure):
+    _fields_ = [("h", C.c_double), ("t0", C.c_double), ("upscale", C.c_int32), ("npoints", C.c_int32), ("nodes", _dp),
+                ("weights", _dp), ("normalise", C.c_int32), ("reserved", C.c_int32)]
+
+
 class DualIC(C.Structure):
     """gb200_dual_ic: impact parameters with seeded partials (forward-mode traces)."""
 
@@ -124,7 +141,7 @@ EXPORTED_SYMBOLS = (
     "gb200_render_batch", "gb200_render_device", "gb200_lineprofile_device", "gb200_fp64_peak", "gb200_fp64_issue_probe", "gb200_debug_rhs", "gb200_debug_math", "gb200_debug_math_lo",
     "gb200_trace_dual", "gb200_trace_dual_batch", "gb200_trace_target",
     "gb200_set_cross_section", "gb200_bucket2d", "gb200_comm_init", "gb200_comm_destroy", "gb200_comm_size", "gb200_comm_context", "gb200_comm_lineprofile", "gb200_comm_render",
-    "gb200_lagtransfer", "gb200_comm_lagtransfer",
+    "gb200_lagtransfer", "gb200_comm_lagtransfer", "gb200_tf_lineprofile", "gb200_tf_lagtransfer",
 )
 
 
@@ -277,6 +294,9 @@ def load():
            C.POINTER(C.c_int64)]
     lib.gb200_lagtransfer.argtypes = [vp] + lag
     lib.gb200_comm_lagtransfer.argtypes = [vp] + lag
+    tfq = [vp, C.c_int32, C.POINTER(TfBranches), C.c_int32, C.POINTER(TfModel), _dp, C.c_int32]
+    lib.gb200_tf_lineprofile.argtypes = tfq + [C.POINTER(TfQuadOpts), _dp]
+    lib.gb200_tf_lagtransfer.argtypes = tfq + [_dp, C.c_int32, C.POINTER(TfQuadOpts), _dp]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)
         if name not in ("gb200_destroy", "gb200_last_error", "gb200_version", "gb200_comm_destroy", "gb200_comm_context"):

@@ -536,6 +536,20 @@ class BinningMethod:
     """src/Gradus.jl:447"""
 
 
+class TransferFunctionMethod:
+    """src/Gradus.jl:448: `lineprofile` by integrating Cunningham transfer functions (src/line-profiles.jl:121-150).  Carries
+    that method's keywords -- `minrₑ` / `min_re`, `maxrₑ` / `max_re`, `numrₑ` / `num_re`, `h` (the quadrature's edge zone
+    in g✶), `n_radii` -- and any keyword of the transfer-function set-up (`N`, `β₀` / `beta0`, `chart`, ...).  The defaults
+    are those of `tf_integration.lineprofile_transfer_functions`."""
+
+    def __init__(self, *, min_re=None, max_re=50.0, num_re=100, h=2e-8, n_radii=1000, **setup):
+        # Python folds a keyword written minrₑ=... to "minre" (NFKC); a dict can still carry "minrₑ"
+        self.min_re = _pop_alias(setup, ("minrₑ", "minre"), min_re)
+        self.max_re = _pop_alias(setup, ("maxrₑ", "maxre"), max_re)
+        self.num_re = _pop_alias(setup, ("numrₑ", "numre"), num_re)
+        self.h, self.n_radii, self.setup = h, n_radii, setup
+
+
 # --------------------------------------------------------------------------- configuration
 @dataclass
 class TracingConfiguration:
@@ -1250,16 +1264,37 @@ class TabulatedEmissivity:
         return np.interp(np.clip(r, rs[0], rs[-1]), rs, np.asarray(self.eps, np.float64))
 
 
-def lineprofile(bins, emissivity, m, position, d, method=None, *, lambda_max=None, min_re=None, max_re=50.0,
+def _lineprofile_transfer_functions(bins, emissivity, m, position, d, method, min_re, max_re, ensemble, setup):
+    """Transfer functions on the device (`tf_integration.transferfunctions`), integrated on the device
+    (`gb200_tf_lineprofile`).  `min_re` / `max_re` given to `lineprofile` replace the method's."""
+    from . import tf_integration as ti
+
+    if not isinstance(emissivity, (PowerLawEmissivity, TabulatedEmissivity)):
+        raise TypeError("an emissivity given as a Python callable cannot cross the C ABI: pass PowerLawEmissivity or "
+                        "TabulatedEmissivity, or use tf_integration.lineprofile_transfer_functions")
+    itb = ti.transferfunctions(m, position, d, min_re=method.min_re if min_re is None else min_re,
+                               max_re=method.max_re if max_re is None else max_re, num_re=method.num_re, ensemble=ensemble,
+                               **{**method.setup, **setup})
+    return ti.integrate_lineprofiles(emissivity, itb, bins, h=method.h, n_radii=method.n_radii, ensemble=ensemble)[0]
+
+
+def lineprofile(bins, emissivity, m, position, d, method=None, *, lambda_max=None, min_re=None, max_re=None,
                 plane=None, callback="default", ensemble=None, bin_right_closed=False, plunging=None, **solver_args):
     """`lineprofile(bins, ε, m, u, d, ::BinningMethod; λ_max, minrₑ, maxrₑ, plane, callback, ...)`
-    (src/line-profiles.jl:152-198).  Returns (bins, flux ./ sum(flux))."""
-    if method is not None and not isinstance(method, BinningMethod):
-        raise ValueError("only BinningMethod() runs on the device (TransferFunctionMethod is a later row)")
+    (src/line-profiles.jl:152-198), or with `TransferFunctionMethod(...)` (src/line-profiles.jl:121-150).  Returns
+    (bins, flux ./ sum(flux))."""
+    if method is not None and not isinstance(method, (BinningMethod, TransferFunctionMethod)):
+        raise ValueError("method must be BinningMethod() or TransferFunctionMethod()")
     lambda_max = _pop_alias(solver_args, ("λ_max",), lambda_max)
     min_re = _pop_alias(solver_args, ("minrₑ",), min_re)
     max_re = _pop_alias(solver_args, ("maxrₑ",), max_re)
     bins = np.ascontiguousarray(bins, np.float64)
+    if isinstance(method, TransferFunctionMethod):
+        if lambda_max is not None or plane is not None or callback != "default" or bin_right_closed or plunging is not None:
+            raise ValueError("λ_max, plane, callback, bin_right_closed and plunging belong to BinningMethod")
+        return bins, _lineprofile_transfer_functions(bins, emissivity, m, position, d, method, min_re, max_re, ensemble, solver_args)
+    if max_re is None:
+        max_re = 50.0
     if lambda_max is None:
         lambda_max = 2 * position[1]
     if min_re is None:

@@ -343,7 +343,7 @@ static int pool_get(gb200_ctx* ctx, size_t slot, size_t bytes, void** out) {
 enum { SL_STATUS = 0, SL_LAMBDA, SL_X0, SL_V0 = SL_X0 + 4, SL_XI0 = SL_V0 + 4, SL_VI0 = SL_XI0 + 4, SL_NACC = SL_VI0 + 4, SL_NREJ, SL_FLAGS,
        SL_IMG0, SL_G = SL_IMG0 + GB_MAX_PF, SL_F, SL_EX0, SL_EV0 = SL_EX0 + 4, SL_BINS = SL_EV0 + 4, SL_PARTIAL, SL_FLUX, SL_EMR, SL_EME,
        SL_PL0, SL_SCRATCH = SL_PL0 + 4, SL_BATCH, SL_BATCH_QUEUE,
-       SL_LAG_SAMPLES, SL_LAG_PARTIAL, SL_LAG_SCAL, SL_LAG_CELLS, SL_LAG_OUT, SL_LAG_PROF, SL_COUNT };
+       SL_LAG_SAMPLES, SL_LAG_PARTIAL, SL_LAG_SCAL, SL_LAG_CELLS, SL_LAG_OUT, SL_LAG_PROF, SL_TFQ_IN, SL_TFQ_OUT, SL_COUNT };
 
 // The output arrays of gb200_endpoints: f(host array, GbParams field the kernel writes it through, pool slot of a single
 // call) for each, null host arrays included.  Every copy, binding and layout of endpoints goes through this one list.
@@ -1502,6 +1502,24 @@ static int validate_ascending(gb200_ctx* ctx, const double* r, int32_t n, const 
     return GB200_OK;
 }
 
+// the emissivity of a gb200_disc_profile and, when `time`, its arrival-time table
+static int validate_disc_profile(gb200_ctx* ctx, const gb200_disc_profile* pr, bool time) {
+    const gb200_emissivity& em = pr->emissivity;
+    int rc;
+    if (em.kind == GB200_EMISSIVITY_POWERLAW) {
+        if (!std::isfinite(em.index)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "emissivity index must be finite");
+    } else if (em.kind == GB200_EMISSIVITY_TABLE) {
+        rc = validate_ascending(ctx, em.r, em.n, "emissivity table"); if (rc) return rc;
+        if (!em.eps) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "emissivity table without values");
+    } else return fail(ctx, GB200_ERR_UNSUPPORTED, "emissivity kind %d", em.kind);
+    if (!time) return GB200_OK;
+    if (pr->time_kind != GB200_PROFILE_TIME_NAN_LINEAR && pr->time_kind != GB200_PROFILE_TIME_LINEAR)
+        return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "profile time kind %d", pr->time_kind);
+    rc = validate_ascending(ctx, pr->r, pr->n, "arrival-time profile"); if (rc) return rc;
+    if (!pr->t) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "arrival-time profile without times");
+    return GB200_OK;
+}
+
 // Everything that can be rejected without tracing, for every device, before the first launch.
 static int validate_lagtransfer(const std::vector<gb200_ctx*>& ctxs, const gb200_problem* p, const gb200_ic* ic, const gb200_disc_profile* pr,
                                 const gb200_lagtransfer_opts* o, const double* time_edges, const double* energy_edges, const double* tf, const int64_t* hits) {
@@ -1516,17 +1534,7 @@ static int validate_lagtransfer(const std::vector<gb200_ctx*>& ctxs, const gb200
     if (!std::isfinite(o->t0)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "t0 must be finite");
     rc = validate_lims(ctx, o->energy_lims, "energy"); if (rc) return rc;
     rc = validate_lims(ctx, o->time_lims, "time"); if (rc) return rc;
-    const gb200_emissivity& em = pr->emissivity;
-    if (em.kind == GB200_EMISSIVITY_POWERLAW) {
-        if (!std::isfinite(em.index)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "emissivity index must be finite");
-    } else if (em.kind == GB200_EMISSIVITY_TABLE) {
-        rc = validate_ascending(ctx, em.r, em.n, "emissivity table"); if (rc) return rc;
-        if (!em.eps) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "emissivity table without values");
-    } else return fail(ctx, GB200_ERR_UNSUPPORTED, "emissivity kind %d", em.kind);
-    if (pr->time_kind != GB200_PROFILE_TIME_NAN_LINEAR && pr->time_kind != GB200_PROFILE_TIME_LINEAR)
-        return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "profile time kind %d", pr->time_kind);
-    rc = validate_ascending(ctx, pr->r, pr->n, "arrival-time profile"); if (rc) return rc;
-    if (!pr->t) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "arrival-time profile without times");
+    rc = validate_disc_profile(ctx, pr, true); if (rc) return rc;
     // what render_common would only find after it has started on the first device
     double r_isco;
     if (gb200_isco(p->metric_kind, p->metric_params, &r_isco)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "no ISCO found for this metric (is it a naked singularity?)");
@@ -1653,6 +1661,179 @@ int gb200_comm_lagtransfer(gb200_comm* c, const gb200_problem* p, const gb200_ic
                            const gb200_lagtransfer_opts* opts, double* time_edges, double* energy_edges, double* tf, int64_t* hits) {
     if (!c) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null communicator");
     return lagtransfer_run(c->ctx, c->nccl.data(), p, ic, pr, pl, opts, time_edges, energy_edges, tf, hits);
+}
+
+// ---------------------------------------------------------------- quadrature of Cunningham transfer functions
+static bool finite_ascending(const double* x, int64_t n, bool strict) {
+    for (int64_t k = 0; k < n; ++k) {
+        if (!std::isfinite(x[k])) return false;
+        if (k > 0 && (strict ? !(x[k] > x[k - 1]) : !(x[k] >= x[k - 1]))) return false;
+    }
+    return true;
+}
+
+static int validate_tf_quad(gb200_ctx* ctx, bool lag, int32_t ntables, const gb200_tf_branches* tables, int32_t nmodels,
+                            const gb200_tf_model* models, const double* g_grid, int32_t ngrid, const double* t_grid, int32_t nt,
+                            const gb200_tf_quad_opts* o, const double* out) {
+    if (!tables || !models || !g_grid || !o || !out || (lag && !t_grid)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null argument");
+    if (ntables < 1 || nmodels < 1) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need ntables, nmodels >= 1 (got %d, %d)", ntables, nmodels);
+    if (ngrid < 2 || ngrid > 65535 * 128) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 2 <= ngrid <= %d (got %d)", 65535 * 128, ngrid);
+    if (!finite_ascending(g_grid, ngrid, true)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "g_grid must be finite and strictly ascending");
+    if (lag && nt < 1) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need nt >= 1 (got %d)", nt);
+    if (lag && !finite_ascending(t_grid, nt, true)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "t_grid must be finite and strictly ascending");
+    if (!(o->h > 0.0 && o->h < 0.5)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 0 < h < 0.5 (got %g)", o->h);
+    if (o->upscale < 1) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need upscale >= 1 (got %d)", o->upscale);
+    if (o->npoints < 1 || o->npoints > 32 || !o->nodes || !o->weights)
+        return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "need 1..32 Gauss points with nodes and weights (got %d)", o->npoints);
+    for (int k = 0; k < o->npoints; ++k)
+        if (!std::isfinite(o->nodes[k]) || !std::isfinite(o->weights[k])) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "Gauss nodes and weights must be finite");
+    if (o->normalise != 0 && o->normalise != 1) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "normalise must be 0 or 1");
+    if (lag && !std::isfinite(o->t0)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "t0 must be finite");
+    for (int i = 0; i < ntables; ++i) {
+        const gb200_tf_branches& T = tables[i];
+        if (T.n_radii < 2 || !T.r_e || !T.gmin || !T.gmax || !T.off || !T.gs || !T.f || !T.t)
+            return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "table %d: need n_radii >= 2 and every array", i);
+        if (!finite_ascending(T.r_e, T.n_radii, true)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "table %d: r_e must be finite and strictly ascending", i);
+        for (int k = 0; k < T.n_radii; ++k)
+            if (!std::isfinite(T.gmin[k]) || !std::isfinite(T.gmax[k]) || !(T.gmin[k] < T.gmax[k]))
+                return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "table %d, radius %d: need finite gmin < gmax", i, k);
+        if (T.off[0] != 0) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "table %d: off[0] must be 0", i);
+        for (int b = 0; b < 2 * T.n_radii; ++b) {
+            const int64_t n = T.off[b + 1] - T.off[b];
+            if (n < 2 || n > INT32_MAX) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "table %d, branch %d: need at least 2 knots (got %lld)", i, b, (long long)n);
+            if (!finite_ascending(T.gs + T.off[b], n, false)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "table %d, branch %d: g* knots must be finite and ascending", i, b);
+        }
+    }
+    for (int m = 0; m < nmodels; ++m) {
+        const gb200_tf_model& M = models[m];
+        if (M.table < 0 || M.table >= ntables) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "model %d: table index %d out of range [0, %d)", m, M.table, ntables);
+        if (M.n_radii < 2 || !M.radii) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "model %d: need n_radii >= 2 (got %d)", m, M.n_radii);
+        if (!finite_ascending(M.radii, M.n_radii, true)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "model %d: radii must be finite and strictly ascending", m);
+        if (!std::isfinite(M.rmin)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "model %d: rmin must be finite", m);
+        if (!std::isfinite(M.g_scale) || !(M.g_scale > 0.0)) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "model %d: g_scale must be positive and finite", m);
+        int rc = validate_disc_profile(ctx, &M.profile, lag); if (rc) return rc;
+    }
+    return GB200_OK;
+}
+
+// Both entry points: every array of the call is packed into the pinned staging buffer and crosses in one copy; the result
+// comes back in one.
+static int tf_quad_run(gb200_ctx* ctx, bool lag, int32_t ntables, const gb200_tf_branches* tables, int32_t nmodels,
+                       const gb200_tf_model* models, const double* g_grid, int32_t ngrid, const double* t_grid, int32_t nt,
+                       const gb200_tf_quad_opts* o, double* out) {
+    if (!ctx) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null context");
+    ctx->stats = gb200_stats{};
+    int rc = validate_tf_quad(ctx, lag, ntables, tables, nmodels, models, g_grid, ngrid, t_grid, nt, o, out); if (rc) return rc;
+    if (!lag) nt = 1;
+    std::vector<GbTfTable> tabs((size_t)ntables);
+    std::vector<GbTfModel> mods((size_t)nmodels);
+    int64_t nrad = 0, noff = 0, nknot = 0, nann = 0, nprof = 0;
+    for (int i = 0; i < ntables; ++i) {
+        tabs[(size_t)i] = GbTfTable{tables[i].n_radii, nrad, noff};
+        nrad += tables[i].n_radii;
+        noff += 2 * (int64_t)tables[i].n_radii + 1;
+        nknot += tables[i].off[2 * tables[i].n_radii];
+    }
+    for (int m = 0; m < nmodels; ++m) {
+        const gb200_tf_model& M = models[m];
+        const gb200_emissivity& em = M.profile.emissivity;
+        GbTfModel& G = mods[(size_t)m];
+        G = GbTfModel{M.table, M.n_radii, nann, M.rmin, M.g_scale, em.kind, em.kind == GB200_EMISSIVITY_TABLE ? em.n : 0, em.index, nprof,
+                      M.profile.time_kind, lag ? M.profile.n : 0, 0};
+        nann += M.n_radii;
+        nprof += 2 * (int64_t)G.emis_n;
+        G.time0 = nprof;
+        nprof += 2 * (int64_t)G.time_n;
+    }
+    // staging layout, every array 256-byte aligned
+    size_t used = 0;
+    auto place = [&](size_t bytes) { const size_t at = used; used += (bytes + 255) & ~(size_t)255; return at; };
+    const size_t at_tab = place(sizeof(GbTfTable) * tabs.size()), at_mod = place(sizeof(GbTfModel) * mods.size());
+    const size_t at_re = place(8 * (size_t)nrad), at_gmin = place(8 * (size_t)nrad), at_gmax = place(8 * (size_t)nrad);
+    const size_t at_off = place(8 * (size_t)noff), at_gs = place(8 * (size_t)nknot), at_f = place(8 * (size_t)nknot), at_t = place(8 * (size_t)nknot);
+    const size_t at_radii = place(8 * (size_t)nann), at_prof = place(8 * (size_t)nprof), at_g = place(8 * (size_t)ngrid);
+    const size_t at_tg = place(8 * (size_t)(lag ? nt : 0)), at_x = place(8 * (size_t)o->npoints), at_w = place(8 * (size_t)o->npoints);
+    const size_t nout = (size_t)nmodels * (size_t)ngrid * (size_t)nt;
+    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
+    void *din, *dout;
+    rc = pool_get(ctx, SL_TFQ_IN, used, &din); if (rc) return rc;
+    rc = pool_get(ctx, SL_TFQ_OUT, sizeof(double) * nout, &dout); if (rc) return rc;
+    CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    rc = ensure_stage(ctx, used); if (rc) return rc;
+    char* st = (char*)ctx->stage;
+    memcpy(st + at_tab, tabs.data(), sizeof(GbTfTable) * tabs.size());
+    memcpy(st + at_mod, mods.data(), sizeof(GbTfModel) * mods.size());
+    for (int i = 0; i < ntables; ++i) {
+        const gb200_tf_branches& T = tables[i];
+        const GbTfTable& G = tabs[(size_t)i];
+        memcpy(st + at_re + 8 * G.radius0, T.r_e, 8 * (size_t)T.n_radii);
+        memcpy(st + at_gmin + 8 * G.radius0, T.gmin, 8 * (size_t)T.n_radii);
+        memcpy(st + at_gmax + 8 * G.radius0, T.gmax, 8 * (size_t)T.n_radii);
+    }
+    int64_t k0 = 0;
+    for (int i = 0; i < ntables; ++i) { // offsets become knot indices of the whole call
+        const gb200_tf_branches& T = tables[i];
+        int64_t* off = (int64_t*)(st + at_off) + tabs[(size_t)i].off0;
+        const int64_t nk = T.off[2 * T.n_radii];
+        for (int b = 0; b <= 2 * T.n_radii; ++b) off[b] = k0 + T.off[b];
+        memcpy(st + at_gs + 8 * k0, T.gs, 8 * (size_t)nk);
+        memcpy(st + at_f + 8 * k0, T.f, 8 * (size_t)nk);
+        memcpy(st + at_t + 8 * k0, T.t, 8 * (size_t)nk);
+        k0 += nk;
+    }
+    for (int m = 0; m < nmodels; ++m) {
+        const gb200_tf_model& M = models[m];
+        const GbTfModel& G = mods[(size_t)m];
+        memcpy(st + at_radii + 8 * G.radius0, M.radii, 8 * (size_t)M.n_radii);
+        double* prof = (double*)(st + at_prof);
+        if (G.emis_n) {
+            memcpy(prof + G.emis0, M.profile.emissivity.r, 8 * (size_t)G.emis_n);
+            memcpy(prof + G.emis0 + G.emis_n, M.profile.emissivity.eps, 8 * (size_t)G.emis_n);
+        }
+        if (G.time_n) {
+            memcpy(prof + G.time0, M.profile.r, 8 * (size_t)G.time_n);
+            memcpy(prof + G.time0 + G.time_n, M.profile.t, 8 * (size_t)G.time_n);
+        }
+    }
+    memcpy(st + at_g, g_grid, 8 * (size_t)ngrid);
+    if (lag) memcpy(st + at_tg, t_grid, 8 * (size_t)nt);
+    memcpy(st + at_x, o->nodes, 8 * (size_t)o->npoints);
+    memcpy(st + at_w, o->weights, 8 * (size_t)o->npoints);
+    CU(ctx, cudaMemcpyAsync(din, st, used, cudaMemcpyHostToDevice, ctx->stream));
+    char* d = (char*)din;
+    GbTfArgs A;
+    A.tables = (const GbTfTable*)(d + at_tab); A.models = (const GbTfModel*)(d + at_mod);
+    A.r_e = (const double*)(d + at_re); A.gmin = (const double*)(d + at_gmin); A.gmax = (const double*)(d + at_gmax);
+    A.off = (const int64_t*)(d + at_off);
+    A.gs = (const double*)(d + at_gs); A.f = (const double*)(d + at_f); A.t = (const double*)(d + at_t);
+    A.radii = (const double*)(d + at_radii); A.prof = (const double*)(d + at_prof);
+    A.g_grid = (const double*)(d + at_g); A.t_grid = lag ? (const double*)(d + at_tg) : nullptr;
+    A.nodes = (const double*)(d + at_x); A.weights = (const double*)(d + at_w);
+    A.nmodels = nmodels; A.ngrid = ngrid; A.nt = nt; A.upscale = o->upscale; A.npoints = o->npoints; A.normalise = o->normalise;
+    A.h = o->h; A.t0 = lag ? o->t0 : 0.0;
+    A.out = (double*)dout;
+    int launches = 0;
+    CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    CU(ctx, gb200_launch_tf_quad(A, lag, ctx->stream, &launches));
+    CU(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(out, dout, sizeof(double) * nout, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    float k = 0, tot = 0;
+    cudaEventElapsedTime(&k, ctx->ev1, ctx->ev2);
+    cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
+    ctx->stats.kernel_ms = k; ctx->stats.total_ms = tot; ctx->stats.launches = launches;
+    return GB200_OK;
+}
+
+int gb200_tf_lineprofile(gb200_ctx* ctx, int32_t ntables, const gb200_tf_branches* tables, int32_t nmodels, const gb200_tf_model* models,
+                         const double* g_grid, int32_t ngrid, const gb200_tf_quad_opts* opts, double* out) {
+    return tf_quad_run(ctx, false, ntables, tables, nmodels, models, g_grid, ngrid, nullptr, 0, opts, out);
+}
+
+int gb200_tf_lagtransfer(gb200_ctx* ctx, int32_t ntables, const gb200_tf_branches* tables, int32_t nmodels, const gb200_tf_model* models,
+                         const double* g_grid, int32_t ngrid, const double* t_grid, int32_t nt, const gb200_tf_quad_opts* opts, double* out) {
+    return tf_quad_run(ctx, true, ntables, tables, nmodels, models, g_grid, ngrid, t_grid, nt, opts, out);
 }
 
 int gb200_bucket2d(gb200_ctx* ctx, int64_t n, const double* x, const double* y, const double* w, const double* xbins, int32_t nx,

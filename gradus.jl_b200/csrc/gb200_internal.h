@@ -57,3 +57,37 @@ cudaError_t gb200_launch_lag_samples(const GbParams& P, const double* const* img
 cudaError_t gb200_launch_lag_bin(GbLagScalars* scal, const GbLagLimits& L, double* eb, double* tb, const double* samples, int64_t n,
                                  long long* cells, unsigned* counts, int nblocks, cudaStream_t stream);
 cudaError_t gb200_launch_lag_finish(const long long* cells, const unsigned* counts, int ncell, const GbLagScalars* scal, double* tf, cudaStream_t stream);
+
+// line profiles and lag-energy transfer functions from Cunningham transfer functions (gb200_tfquad.cu; host side
+// gb200_tf_lineprofile / gb200_tf_lagtransfer in gb200_api.cu).  All arrays live in one device arena.
+struct GbTfTable { // one gb200_tf_branches
+    int32_t n_radii;
+    int64_t radius0; // its radius 0 in r_e / gmin / gmax
+    int64_t off0;    // its off[0] in off; off holds knot indices into gs / f / t of the whole call
+};
+struct GbTfModel { // one gb200_tf_model
+    int32_t table, n_radii;
+    int64_t radius0; // its first annulus in radii
+    double rmin, g_scale;
+    int32_t emis_kind, emis_n; // emissivity table: r at prof[emis0], eps at prof[emis0 + emis_n]
+    double emis_index;
+    int64_t emis0;
+    int32_t time_kind, time_n; // arrival-time table: r at prof[time0], t at prof[time0 + time_n]
+    int64_t time0;
+};
+struct GbTfArgs {
+    const GbTfTable* tables;
+    const GbTfModel* models;
+    const double *r_e, *gmin, *gmax;
+    const int64_t* off;
+    const double *gs, *f, *t;
+    const double* radii;
+    const double* prof;
+    const double* g_grid;
+    const double* t_grid; // lag only
+    const double *nodes, *weights;
+    int32_t nmodels, ngrid, nt, upscale, npoints, normalise;
+    double h, t0;
+    double* out; // nmodels x ngrid (x nt)
+};
+cudaError_t gb200_launch_tf_quad(const GbTfArgs& A, bool lag, cudaStream_t stream, int* launches);

@@ -18,38 +18,6 @@ namespace {
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kThreads = 256;
 
-// NaNLinearInterpolator (interpolations.jl:1-30) on an abscissa clipped to the knots, with the host's order of operations
-// (w = (x - x1) / (x2 - x1), (1 - w) y1 + w y2, no fused multiply-add) so that T matches the host bit for bit
-__device__ double lag_time_nan_linear(const GbLagProfile& pr, double x) {
-    const int n = pr.n;
-    x = fmin(fmax(x, pr.r[0]), pr.r[n - 1]);
-    int lo = 0, hi = n - 1; // last index with r[idx] <= x, clamped to [0, n - 2]
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (pr.r[mid] <= x) lo = mid; else hi = mid; }
-    const double x1 = pr.r[lo], x2 = pr.r[lo + 1], y1 = pr.t[lo], y2 = pr.t[lo + 1];
-    const double w = (x - x1) / (x2 - x1);
-    const double y = __dadd_rn(__dmul_rn(1.0 - w, y1), __dmul_rn(w, y2));
-    if (y == y) return y;
-    const double near = w < 0.5 ? y1 : y2; // NaN knots: the nearer neighbour, else the interpolator's default 0
-    return near == near ? near : 0.0;
-}
-
-// np.interp (numpy's arr_interp) on an abscissa clipped to the knots: slope (y[j+1] - y[j]) / (x[j+1] - x[j]) times
-// (x - x[j]) plus y[j], knot values exactly at the knots
-__device__ double lag_time_linear(const GbLagProfile& pr, double x) {
-    const int n = pr.n;
-    x = fmin(fmax(x, pr.r[0]), pr.r[n - 1]);
-    int lo = 0, hi = n; // last index with r[idx] <= x
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (pr.r[mid] <= x) lo = mid; else hi = mid; }
-    if (lo == n - 1 || pr.r[lo] == x) return pr.t[lo];
-    const double slope = (pr.t[lo + 1] - pr.t[lo]) / (pr.r[lo + 1] - pr.r[lo]);
-    double y = __dadd_rn(__dmul_rn(slope, x - pr.r[lo]), pr.t[lo]);
-    if (y != y) {
-        y = __dadd_rn(__dmul_rn(slope, x - pr.r[lo + 1]), pr.t[lo + 1]);
-        if (y != y && pr.t[lo] == pr.t[lo + 1]) y = pr.t[lo];
-    }
-    return y;
-}
-
 // numpy.linspace(lo, hi, N)[k]: k * step + lo with step = (hi - lo) / (N - 1), two roundings, the last edge exactly hi
 __device__ double lag_edge(double lo, double hi, int N, int k) {
     if (k == N - 1) return hi;
@@ -100,7 +68,7 @@ __global__ void __launch_bounds__(kThreads) gb200_lag_samples_kernel(const GbPar
             ray_initial_state(P, ray_index_of_slot(P, i), ri);
             const double gi = g[i], r = rho[i];
             E = gi * E0;
-            T = (pr.time_kind == GB200_PROFILE_TIME_NAN_LINEAR ? lag_time_nan_linear(pr, r) : lag_time_linear(pr, r)) + t[i];
+            T = (pr.time_kind == GB200_PROFILE_TIME_NAN_LINEAR ? gb_nan_linear_clipped(pr.r, pr.t, pr.n, r) : gb_interp_clipped(pr.r, pr.t, pr.n, r)) + t[i];
             f = pow(gi, 3.0) * emissivity_eval(P, r) * ri.area; // g .^ 3 is libm pow on the host, not g * g * g
             if (isfinite(E) && isfinite(T) && isfinite(f)) {
                 s.mn[0] = fmin(s.mn[0], E); s.mx[0] = fmax(s.mx[0], E);

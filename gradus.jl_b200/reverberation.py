@@ -150,27 +150,35 @@ def binflux(tf: LagTransferFunction, profile=None, *, E0=6.4, t0=None, **kwargs)
     return tb - t0, eb, td
 
 
-def _disc_profile_to_c(profile):
-    """-> (gb200_disc_profile, arrays it points into).  Raises TypeError for an ε the device cannot evaluate."""
+def _emissivity_to_c(eps, c: cabi.DiscProfile, keep: list, host="binflux(lagtransfer(...), profile)"):
+    """Fill c.emissivity from a PowerLawEmissivity or TabulatedEmissivity (its arrays appended to `keep`); anything else
+    raises TypeError naming the host function that evaluates it instead."""
+    if isinstance(eps, api.PowerLawEmissivity):
+        c.emissivity.kind, c.emissivity.index = cabi.EMISSIVITY_POWERLAW, float(eps.index)
+    elif isinstance(eps, api.TabulatedEmissivity):
+        r, e = np.ascontiguousarray(eps.r, np.float64), np.ascontiguousarray(eps.eps, np.float64)
+        keep += [r, e]
+        c.emissivity.kind, c.emissivity.n = cabi.EMISSIVITY_TABLE, len(r)
+        c.emissivity.r, c.emissivity.eps = cabi.dptr(r), cabi.dptr(e)
+    else:
+        raise TypeError("an emissivity given as a Python callable cannot cross the C ABI: pass PowerLawEmissivity or "
+                        f"TabulatedEmissivity, or use {host}")
+
+
+def _disc_profile_to_c(profile, host="binflux(lagtransfer(...), profile)"):
+    """-> (gb200_disc_profile, arrays it points into).  Raises TypeError for an ε the device cannot evaluate, naming `host`,
+    the host function that can."""
     if isinstance(profile, AnalyticRadialDiscProfile):
         eps, r, t, kind = profile.eps, profile.t.t, profile.t.u, cabi.PROFILE_TIME_NAN_LINEAR
         if profile.t.default != 0.0:
-            raise TypeError("binned_lagtransfer supports NaNLinearInterpolator's default fallback value 0 only")
-        if not isinstance(eps, (api.PowerLawEmissivity, api.TabulatedEmissivity)):
-            raise TypeError("an emissivity given as a Python callable cannot cross the C ABI: pass PowerLawEmissivity or "
-                            "TabulatedEmissivity, or use binflux(lagtransfer(...), profile)")
+            raise TypeError("the device supports NaNLinearInterpolator's default fallback value 0 only")
     elif isinstance(profile, corona.RadialDiscProfile):
         eps, r, t, kind = api.TabulatedEmissivity(profile.radii, profile.eps), profile.radii, profile.t, cabi.PROFILE_TIME_LINEAR
     else:
-        raise TypeError(f"profile {type(profile).__name__} cannot be binned on the device: use binflux(lagtransfer(...), profile)")
+        raise TypeError(f"profile {type(profile).__name__} cannot be evaluated on the device: use {host}")
     keep = [np.ascontiguousarray(r, np.float64), np.ascontiguousarray(t, np.float64)]
     c = cabi.DiscProfile()
-    if isinstance(eps, api.PowerLawEmissivity):
-        c.emissivity.kind, c.emissivity.index = cabi.EMISSIVITY_POWERLAW, float(eps.index)
-    else:
-        keep += [np.ascontiguousarray(eps.r, np.float64), np.ascontiguousarray(eps.eps, np.float64)]
-        c.emissivity.kind, c.emissivity.n = cabi.EMISSIVITY_TABLE, len(keep[2])
-        c.emissivity.r, c.emissivity.eps = cabi.dptr(keep[2]), cabi.dptr(keep[3])
+    _emissivity_to_c(eps, c, keep, host)
     c.time_kind, c.n, c.r, c.t = kind, len(keep[0]), cabi.dptr(keep[0]), cabi.dptr(keep[1])
     return c, keep
 

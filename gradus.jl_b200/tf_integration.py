@@ -12,12 +12,14 @@ The transfer functions themselves (all radii in lock step) come from `transfer_f
 the quadrature below is the reference's host-side arithmetic, vectorised over the energy bins of one annulus."""
 from __future__ import annotations
 
+import ctypes as C
 import math
 from dataclasses import dataclass
 from typing import Callable, Optional, Sequence
 
 import numpy as np
 
+from . import _cabi as cabi
 from . import api
 from . import transfer_functions as tf
 
@@ -315,3 +317,142 @@ def integrate_lagtransfer(profile, itb: InterpolatingTransferBranches, g_grid, t
     if total > 0:
         out = out / total
     return out
+
+
+# --------------------------------------------------------------------------- many models on the device
+@dataclass
+class PackedBranches:
+    """An InterpolatingTransferBranches as the flat arrays of `gb200_tf_branches`: branch 2k is the lower, 2k+1 the upper
+    branch of radius k, with knots gs[off[b]:off[b+1]] and values f, t there."""
+
+    r_e: np.ndarray
+    gmin: np.ndarray
+    gmax: np.ndarray
+    off: np.ndarray
+    gs: np.ndarray
+    f: np.ndarray
+    t: np.ndarray
+
+    def to_c(self):
+        return cabi.TfBranches(len(self.r_e), 0, cabi.dptr(self.r_e), cabi.dptr(self.gmin), cabi.dptr(self.gmax),
+                               self.off.ctypes.data_as(C.POINTER(C.c_int64)), cabi.dptr(self.gs), cabi.dptr(self.f), cabi.dptr(self.t))
+
+
+def pack_branches(itb: InterpolatingTransferBranches) -> PackedBranches:
+    """Flatten `itb` for the device.  Every branch must be a `NaNLinearInterpolator` with the default fallback 0 (what
+    `interpolate_branches` makes), and f and t of a branch must share their knots."""
+    gs, f, t, off = [], [], [], [0]
+    for br in itb.branches:
+        for fb, tb in ((br.lower_f, br.lower_t), (br.upper_f, br.upper_t)):
+            for fn in (fb, tb):
+                if not isinstance(fn, NaNLinearInterpolator) or fn.default != 0.0:
+                    raise TypeError("only NaNLinearInterpolator branches with default 0 can be integrated on the device: "
+                                    "use integrate_lineprofile / integrate_lagtransfer")
+            if not np.array_equal(fb.t, tb.t):
+                raise ValueError(f"the f and t branches at r_e = {br.r_e} do not share their knots")
+            gs.append(fb.t)
+            f.append(fb.u)
+            t.append(tb.u)
+            off.append(off[-1] + fb.t.size)
+    cat = lambda parts: np.ascontiguousarray(np.concatenate(parts), np.float64)  # noqa: E731
+    return PackedBranches(np.ascontiguousarray(itb.radii, np.float64), np.ascontiguousarray(itb.gmin, np.float64),
+                          np.ascontiguousarray(itb.gmax, np.float64), np.array(off, np.int64), cat(gs), cat(f), cat(t))
+
+
+def _per_model(values: dict):
+    """Broadcast the per-model arguments (a scalar, or a sequence of one or of n values) to one list per argument."""
+    lists = {k: list(v) if isinstance(v, (list, tuple, np.ndarray)) else [v] for k, v in values.items()}
+    n = max(len(v) for v in lists.values())
+    for k, v in lists.items():
+        if len(v) not in (1, n):
+            raise ValueError(f"{k}: {len(v)} values for {n} models")
+    return n, {k: v * n if len(v) == 1 else v for k, v in lists.items()}
+
+
+def _ascending(name, a):
+    a = np.ascontiguousarray(a, np.float64)
+    if a.ndim != 1 or a.size < 1 or not np.all(np.isfinite(a)) or not np.all(np.diff(a) > 0):
+        raise ValueError(f"{name} must be a finite, strictly ascending 1-D grid")
+    return a
+
+
+def _device_quadrature(lag, profiles, itbs, g_grid, t_grid, *, table_of, rmin, rmax, g_scale, h, n_radii, g_grid_upscale,
+                       quadrature_points, t0, ensemble):
+    from .reverberation import _disc_profile_to_c, _emissivity_to_c
+
+    itbs = [itbs] if isinstance(itbs, InterpolatingTransferBranches) else list(itbs)
+    packed = [pack_branches(itb) for itb in itbs]
+    if isinstance(profiles, (list, tuple)) and len(profiles) == 0:
+        raise ValueError("no emission models")
+    n, per = _per_model({"profiles": profiles if isinstance(profiles, (list, tuple)) else [profiles],
+                         "table_of": list(range(len(itbs))) if table_of is None else table_of,
+                         "rmin": rmin, "rmax": rmax, "g_scale": g_scale, "n_radii": n_radii})
+    host = "integrate_lagtransfer" if lag else "integrate_lineprofile"
+    g_grid = _ascending("g_grid", g_grid)
+    if g_grid.size < 2:
+        raise ValueError("g_grid needs at least two edges")
+    if lag:
+        t_grid = _ascending("t_grid", t_grid)
+    if not 1 <= int(quadrature_points) <= 32:
+        raise ValueError(f"quadrature_points must be in 1..32 (got {quadrature_points})")
+    if int(g_grid_upscale) < 1:
+        raise ValueError(f"g_grid_upscale must be >= 1 (got {g_grid_upscale})")
+    if not 0 < h < 0.5:
+        raise ValueError(f"h must lie in (0, 0.5) (got {h})")
+    models, keep = (cabi.TfModel * n)(), []
+    for k in range(n):
+        tab = per["table_of"][k]
+        if int(tab) != tab or not 0 <= tab < len(itbs):
+            raise ValueError(f"model {k}: table index {tab} out of range for {len(itbs)} tables")
+        nr = per["n_radii"][k]
+        if int(nr) != nr or nr < 2:
+            raise ValueError(f"model {k}: n_radii must be an integer >= 2 (got {nr})")
+        itb = itbs[int(tab)]
+        lo = itb.inner_radius() if per["rmin"][k] is None else float(per["rmin"][k])
+        hi = itb.outer_radius() if per["rmax"][k] is None else float(per["rmax"][k])
+        if not lo < hi:
+            raise ValueError(f"model {k}: need rmin < rmax (got {lo}, {hi})")
+        radii = np.ascontiguousarray((geometric_grid if lag else inverse_grid)(lo, hi, int(nr)), np.float64)
+        if lag:
+            prof, pk = _disc_profile_to_c(per["profiles"][k], host)
+        else:
+            prof, pk = cabi.DiscProfile(), []
+            _emissivity_to_c(per["profiles"][k], prof, pk, host)
+        keep += [radii, pk]
+        models[k] = cabi.TfModel(int(tab), int(nr), cabi.dptr(radii), lo, float(per["g_scale"][k]), prof)
+    X, W = (np.ascontiguousarray(a, np.float64) for a in _gauss(int(quadrature_points)))
+    opts = cabi.TfQuadOpts(float(h), float(t0), int(g_grid_upscale), int(quadrature_points), cabi.dptr(X), cabi.dptr(W), 1, 0)
+    tables = (cabi.TfBranches * len(packed))(*[p.to_c() for p in packed])
+    ens = ensemble if ensemble is not None else api.default_ensemble()
+    ctx = ens.ctx(ens.devices[0])
+    lib = cabi.load()
+    if lag:
+        out = np.zeros((n, g_grid.size, t_grid.size))
+        cabi.check(lib.gb200_tf_lagtransfer(ctx, len(packed), tables, n, models, cabi.dptr(g_grid), g_grid.size, cabi.dptr(t_grid),
+                                            t_grid.size, C.byref(opts), cabi.dptr(out.reshape(-1))), ctx)
+    else:
+        out = np.zeros((n, g_grid.size))
+        cabi.check(lib.gb200_tf_lineprofile(ctx, len(packed), tables, n, models, cabi.dptr(g_grid), g_grid.size, C.byref(opts),
+                                            cabi.dptr(out.reshape(-1))), ctx)
+    return out
+
+
+def integrate_lineprofiles(emissivities, itbs, g_grid, *, table_of=None, rmin=None, rmax=None, g_scale=1.0, h=1e-8,
+                           n_radii=1000, g_grid_upscale=1, quadrature_points=7, ensemble=None):
+    """`integrate_lineprofile` for many emission models in one device call (`gb200_tf_lineprofile`): row k of the returned
+    (nmodels, len(g_grid)) array is `integrate_lineprofile(emissivities[k], itbs[table_of[k]], g_grid, rmin=rmin[k], ...)`.
+    `emissivities`, `table_of` (default: model k uses table k), `rmin`, `rmax`, `g_scale` and `n_radii` are per model and
+    broadcast; an emissivity is a `PowerLawEmissivity` or a `TabulatedEmissivity`."""
+    return _device_quadrature(False, emissivities, itbs, g_grid, None, table_of=table_of, rmin=rmin, rmax=rmax, g_scale=g_scale,
+                              h=h, n_radii=n_radii, g_grid_upscale=g_grid_upscale, quadrature_points=quadrature_points, t0=0.0,
+                              ensemble=ensemble)
+
+
+def integrate_lagtransfers(profiles, itbs, g_grid, t_grid, *, t0=0.0, table_of=None, rmin=None, rmax=None, g_scale=1.0, h=1e-8,
+                           n_radii=1000, g_grid_upscale=1, quadrature_points=7, ensemble=None):
+    """`integrate_lagtransfer` for many emission models in one device call (`gb200_tf_lagtransfer`): returns an
+    (nmodels, len(g_grid), len(t_grid)) array.  Profiles are `AnalyticRadialDiscProfile`s with a `PowerLawEmissivity` or
+    `TabulatedEmissivity` ε, or `RadialDiscProfile`s; per-model arguments broadcast as in `integrate_lineprofiles`."""
+    return _device_quadrature(True, profiles, itbs, g_grid, t_grid, table_of=table_of, rmin=rmin, rmax=rmax, g_scale=g_scale, h=h,
+                              n_radii=n_radii, g_grid_upscale=g_grid_upscale, quadrature_points=quadrature_points, t0=t0,
+                              ensemble=ensemble)

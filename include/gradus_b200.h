@@ -435,6 +435,53 @@ int gb200_lagtransfer(gb200_ctx* ctx, const gb200_problem* p, const gb200_ic* ic
                       const gb200_plunging_table* plunging, const gb200_lagtransfer_opts* opts,
                       double* time_edges, double* energy_edges, double* tf, int64_t* hits);
 
+/* ---- line profiles and lag-energy transfer functions from Cunningham transfer functions ---- */
+/* integrate_lineprofile / integrate_lagtransfer (src/transfer-functions/integration.jl:158-207, 233-279, 322-442) for many
+   emission models at once.  One table is an InterpolatingTransferBranches (transfer-functions-2d.jl:1-88) as the host holds
+   it after interpolate_branches: branch 2k is the lower, 2k+1 the upper branch of radius k, with knots
+   [off[b], off[b+1]) of gs / f / t (g* non-decreasing, >= 2 knots).  f and t are NaNLinearInterpolators with default 0:
+   NaN knots are allowed, evaluation extrapolates linearly beyond the ends. */
+typedef struct gb200_tf_branches {
+    int32_t n_radii;                 /* >= 2, r_e strictly ascending */
+    int32_t reserved;
+    const double *r_e, *gmin, *gmax; /* n_radii each, finite gmin < gmax */
+    const int64_t* off;              /* 2 n_radii + 1, off[0] = 0 */
+    const double *gs, *f, *t;        /* off[2 n_radii] knots each */
+} gb200_tf_branches;
+
+typedef struct gb200_tf_model {
+    int32_t table;              /* index into tables[] */
+    int32_t n_radii;            /* annuli, >= 2 */
+    const double* radii;        /* host, strictly ascending: inverse_grid (line profile) or geometric_grid (lag) of (rmin, rmax) */
+    double rmin;                /* r_prev of the first annulus is rmin - (radii[1] - rmin), as on the host */
+    double g_scale;             /* bins are g_grid / g_scale; positive and finite */
+    gb200_disc_profile profile; /* emissivity for both calls (POWERLAW: r^-index, TABLE: numpy.interp of the clipped radius);
+                                   the arrival-time table is read by gb200_tf_lagtransfer only */
+} gb200_tf_model;
+
+typedef struct gb200_tf_quad_opts {
+    double h;                      /* edge zone in g*, 0 < h < 0.5 */
+    double t0;                     /* gb200_tf_lagtransfer: subtracted from the profile's arrival time */
+    int32_t upscale;               /* g_grid_upscale >= 1: sub-bins per bin */
+    int32_t npoints;               /* Gauss-Legendre points, 1..32 */
+    const double *nodes, *weights; /* npoints each: the rule on [-1, 1] (numpy leggauss / FastGaussQuadrature) */
+    int32_t normalise;             /* 1: _normalize! (divide bin j by g[j] + g[j+1], then by the total); 0: raw sums */
+    int32_t reserved;
+} gb200_tf_quad_opts;
+
+/* out[m * ngrid + j]: the line profile of model m, bin j = [g_grid[j], g_grid[j+1]) (the last entry is 0, as on the host).
+   Each (model, bin) is one device thread that walks the annuli in the host's order, so every result is independent of the
+   other models of the call.  Every argument is checked before the first launch (GB200_ERR_INVALID_ARGUMENT). */
+int gb200_tf_lineprofile(gb200_ctx* ctx, int32_t ntables, const gb200_tf_branches* tables, int32_t nmodels,
+                         const gb200_tf_model* models, const double* g_grid, int32_t ngrid, const gb200_tf_quad_opts* opts,
+                         double* out);
+/* out[(m * ngrid + j) * nt + k]: the lag-energy transfer function of model m, energy bin j, time bin k, where a branch's
+   contribution lands in the first k with t_grid[k] >= its time (numpy.searchsorted, side left) and is dropped past the
+   end.  t_grid: nt >= 1, strictly ascending. */
+int gb200_tf_lagtransfer(gb200_ctx* ctx, int32_t ntables, const gb200_tf_branches* tables, int32_t nmodels,
+                         const gb200_tf_model* models, const double* g_grid, int32_t ngrid, const double* t_grid, int32_t nt,
+                         const gb200_tf_quad_opts* opts, double* out);
+
 /* ---- device-resident variants (inputs/outputs stay in HBM) ------------- */
 /* Same as gb200_render but `d_images[k]` are DEVICE pointers on ctx's device and no
    host copy is made; work is enqueued on `cuda_stream` (a cudaStream_t cast to

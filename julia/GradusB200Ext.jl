@@ -101,6 +101,17 @@ end
 struct CLagTransferOpts
     E0::Float64; t0::Float64; energy_lims::NTuple{2,Float64}; time_lims::NTuple{2,Float64}; N_E::Int32; N_t::Int32
 end
+struct CTfBranches
+    n_radii::Int32; reserved::Int32; r_e::Ptr{Float64}; gmin::Ptr{Float64}; gmax::Ptr{Float64}; off::Ptr{Int64}
+    gs::Ptr{Float64}; f::Ptr{Float64}; t::Ptr{Float64}
+end
+struct CTfModel
+    table::Int32; n_radii::Int32; radii::Ptr{Float64}; rmin::Float64; g_scale::Float64; profile::CDiscProfile
+end
+struct CTfQuadOpts
+    h::Float64; t0::Float64; upscale::Int32; npoints::Int32; nodes::Ptr{Float64}; weights::Ptr{Float64}; normalise::Int32
+    reserved::Int32
+end
 const NULL4 = ntuple(_ -> Ptr{Float64}(C_NULL), 4)
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -551,6 +562,123 @@ function lagtransfer_b200(m::Gradus.AbstractMetric{T}, u, d, r, t; linear_time =
     tb, eb, permutedims(tf), hits[]
 end
 
+# ---------------------------------------------------------------------------------------------------------------------
+# quadrature of Cunningham transfer functions, many emission models per call
+
+# An InterpolatingTransferBranches as the flat arrays of gb200_tf_branches: branch 2k is the lower, 2k+1 the upper branch
+# of radius k; every branch a NaNLinearInterpolator (fields t, u) with default 0, f and t on the same knots.
+function _pack_branches(itb)
+    rs, gmin, gmax, off, gs, f, t = Float64[], Float64[], Float64[], Int64[0], Float64[], Float64[], Float64[]
+    for br in sort(collect(itb.branches); by = b -> b.rₑ)
+        push!(rs, br.rₑ); push!(gmin, br.gmin); push!(gmax, br.gmax)
+        for (fb, tb) in ((br.lower_f, br.lower_t), (br.upper_f, br.upper_t))
+            all(x -> x isa Gradus.NaNLinearInterpolator && iszero(x.default), (fb, tb)) ||
+                throw(ArgumentError("only NaNLinearInterpolator branches with default 0 can be integrated on the device"))
+            fb.t == tb.t || throw(ArgumentError("the f and t branches at rₑ = $(br.rₑ) do not share their knots"))
+            append!(gs, fb.t); append!(f, fb.u); append!(t, tb.u); push!(off, length(gs))
+        end
+    end
+    (rs, gmin, gmax, off, gs, f, t)
+end
+
+_per_model(v, n) = v isa AbstractVector ? (length(v) == n ? v : throw(ArgumentError("$(length(v)) values for $n models"))) : fill(v, n)
+
+# ε: a power-law index (a Number) or a clamped linear table (radii, values); profile time: (r, t) knots, NaN-linear
+# (AnalyticRadialDiscProfile) or linear (`linear_time`, RadialDiscProfile)
+function _c_disc_profile(ε, r, t, linear_time, keep)
+    emis = if ε isa Number
+        CEmissivity(0, 0, Float64(ε), C_NULL, C_NULL)
+    else
+        er, ev = collect(Float64, ε[1]), collect(Float64, ε[2])
+        push!(keep, er, ev)
+        CEmissivity(1, length(er), 0.0, pointer(er), pointer(ev))
+    end
+    rv, tv = collect(Float64, r), collect(Float64, t)
+    push!(keep, rv, tv)
+    CDiscProfile(emis, linear_time ? 1 : 0, length(rv), isempty(rv) ? C_NULL : pointer(rv), isempty(tv) ? C_NULL : pointer(tv))
+end
+
+function _tf_quadrature(lag, itbs, g_grid, t_grid, profiles, n; table_of, rmin, rmax, g_scale, h, n_radii, g_grid_upscale,
+                        quadrature_points, t0, ensemble)
+    itbs = itbs isa AbstractVector ? itbs : [itbs]
+    packed = [_pack_branches(itb) for itb in itbs]
+    table_of = isnothing(table_of) ? _per_model(collect(1:length(itbs)), n) : _per_model(table_of, n)
+    rmin, rmax, g_scale, n_radii = _per_model(rmin, n), _per_model(rmax, n), _per_model(g_scale, n), _per_model(n_radii, n)
+    X, W = Gradus.FastGaussQuadrature.gausslegendre(quadrature_points)
+    g, tg = collect(Float64, g_grid), collect(Float64, t_grid)
+    keep = Any[]
+    out = lag ? zeros(Float64, length(tg), length(g), n) : zeros(Float64, length(g), n) # column-major of the C layout
+    GC.@preserve packed keep X W g tg begin
+        tables = [CTfBranches(length(p[1]), 0, pointer(p[1]), pointer(p[2]), pointer(p[3]), pointer(p[4]), pointer(p[5]),
+                              pointer(p[6]), pointer(p[7])) for p in packed]
+        models = map(1:n) do k
+            itb = itbs[table_of[k]]
+            lo = isnothing(rmin[k]) ? minimum(b.rₑ for b in itb.branches) : Float64(rmin[k])
+            hi = isnothing(rmax[k]) ? maximum(b.rₑ for b in itb.branches) : Float64(rmax[k])
+            radii = collect(Float64, lag ? Gradus._geometric_grid(lo, hi, n_radii[k]) : Gradus._inverse_grid(lo, hi, n_radii[k]))
+            push!(keep, radii)
+            CTfModel(table_of[k] - 1, n_radii[k], pointer(radii), lo, g_scale[k], profiles(k, keep))
+        end
+        opts = CTfQuadOpts(h, t0, g_grid_upscale, quadrature_points, pointer(X), pointer(W), 1, 0)
+        ctx = _context(ensemble, 1)
+        if lag
+            _check(ccall((:gb200_tf_lagtransfer, libgradus_b200), Cint,
+                         (Ptr{Cvoid}, Int32, Ptr{CTfBranches}, Int32, Ptr{CTfModel}, Ptr{Float64}, Int32, Ptr{Float64}, Int32,
+                          Ref{CTfQuadOpts}, Ptr{Float64}),
+                         ctx, length(tables), tables, n, models, g, length(g), tg, length(tg), opts, out), ctx)
+        else
+            _check(ccall((:gb200_tf_lineprofile, libgradus_b200), Cint,
+                         (Ptr{Cvoid}, Int32, Ptr{CTfBranches}, Int32, Ptr{CTfModel}, Ptr{Float64}, Int32, Ref{CTfQuadOpts}, Ptr{Float64}),
+                         ctx, length(tables), tables, n, models, g, length(g), opts, out), ctx)
+        end
+    end
+    lag ? permutedims(out, (2, 1, 3)) : out
+end
+
+"""
+    integrate_lineprofile_b200(itbs, g_grid; ε = 3.0, table_of = nothing, rmin = nothing, rmax = nothing, g_scale = 1.0,
+                               h = 1e-8, n_radii = 1000, g_grid_upscale = 1, quadrature_points = 7, ensemble = EnsembleB200())
+
+`integrate_lineprofile(ε, itb, g_grid; rmin, rmax, h, n_radii, g_grid_upscale, ...)`
+(src/transfer-functions/integration.jl:233-254, 322-357) for many emission models in one device call
+(`gb200_tf_lineprofile`).  `itbs`: one `InterpolatingTransferBranches` or a vector of them; `ε` (a power-law index or a
+`(radii, values)` table), `table_of` (1-based; default model k uses table k), `rmin`, `rmax`, `g_scale` and `n_radii` are
+per model, a vector with one entry per model or one value for all.  Returns a `length(g_grid)` × nmodels matrix of
+normalised profiles.  Not run: there is no Julia toolchain where this binding was written; the Python mirror
+`integrate_lineprofiles` is the tested form.
+"""
+function integrate_lineprofile_b200(itbs, g_grid; ε = 3.0, table_of = nothing, rmin = nothing, rmax = nothing, g_scale = 1.0,
+                                    h = 1e-8, n_radii = 1000, g_grid_upscale = 1, quadrature_points = 7,
+                                    ensemble::EnsembleB200 = EnsembleB200())
+    n = maximum(v -> v isa AbstractVector ? length(v) : 1, (table_of, rmin, rmax, g_scale, n_radii,
+                                                            ε isa AbstractVector ? ε : nothing))
+    isnothing(table_of) && itbs isa AbstractVector && (n = max(n, length(itbs)))
+    εs = _per_model(ε isa AbstractVector ? ε : [ε for _ = 1:n], n)
+    _tf_quadrature(false, itbs, g_grid, Float64[], (k, keep) -> _c_disc_profile(εs[k], Float64[], Float64[], false, keep), n;
+                   table_of, rmin, rmax, g_scale, h, n_radii, g_grid_upscale, quadrature_points, t0 = 0.0, ensemble)
+end
+
+"""
+    integrate_lagtransfer_b200(itbs, g_grid, t_grid, profiles; t0 = 0.0, table_of = nothing, rmin = nothing, rmax = nothing,
+                               g_scale = 1.0, h = 1e-8, n_radii = 1000, g_grid_upscale = 1, quadrature_points = 7,
+                               ensemble = EnsembleB200())
+
+`integrate_lagtransfer(profile, itb, g_grid, t_grid; t0, n_radii, rmin, rmax, ...)`
+(src/transfer-functions/integration.jl:256-279, 359-442) for many emission models in one device call
+(`gb200_tf_lagtransfer`).  `profiles`: a vector of named tuples `(r, t, linear_time = false, ε = 3.0)`, the profile's
+arrival-time knots as in `lagtransfer_b200`; the other per-model keywords as in `integrate_lineprofile_b200`.  Returns a
+`length(g_grid)` × `length(t_grid)` × nmodels array.  Not run: there is no Julia toolchain where this binding was written;
+the Python mirror `integrate_lagtransfers` is the tested form.
+"""
+function integrate_lagtransfer_b200(itbs, g_grid, t_grid, profiles::AbstractVector; t0 = 0.0, table_of = nothing, rmin = nothing,
+                                    rmax = nothing, g_scale = 1.0, h = 1e-8, n_radii = 1000, g_grid_upscale = 1,
+                                    quadrature_points = 7, ensemble::EnsembleB200 = EnsembleB200())
+    n = length(profiles)
+    prof(k, keep) = (p = profiles[k]; _c_disc_profile(get(p, :ε, 3.0), p.r, p.t, get(p, :linear_time, false), keep))
+    _tf_quadrature(true, itbs, g_grid, t_grid, prof, n; table_of, rmin, rmax, g_scale, h, n_radii, g_grid_upscale,
+                   quadrature_points, t0, ensemble)
+end
+
 """
     optimize_for_target_b200(target, m, x0; ensemble, d_tol = 1e-2, max_time = 2x0[2], p0 = (0.0, 0.0), window, grid = 33, kwargs...)
 
@@ -601,5 +729,6 @@ function optimize_for_target_b200(target, m::Gradus.AbstractMetric{T}, x0; ensem
     best[2], best[3], best[4], best[1]
 end
 
-export EnsembleB200, B200PointFunction, ImageOrder, equatorial_crossings, lineprofile_b200, lagtransfer_b200, optimize_for_target_b200
+export EnsembleB200, B200PointFunction, ImageOrder, equatorial_crossings, lineprofile_b200, lagtransfer_b200, optimize_for_target_b200,
+       integrate_lineprofile_b200, integrate_lagtransfer_b200
 end # module
