@@ -37,9 +37,8 @@ struct gb200_ctx {
     gb200_stats stats{};
     std::vector<DevBuf> pool;
     unsigned long long* d_queue = nullptr; // [0] queue, [1..3] counters
-    double fp64_peak = 0.0;
-    std::vector<cudaStream_t> pool_streams; // gb200_trace_batch, gb200_render_batch, pipelined gb200_render
-    std::vector<cudaEvent_t> chunk_events;  // pipelined gb200_render: one per chunk
+    std::vector<cudaStream_t> pool_streams; // batch calls, pipelined gb200_render, gb200_comm_render's copies
+    std::vector<cudaEvent_t> chunk_events;  // pipelined gb200_render and gb200_comm_render: per chunk
     void* stage = nullptr;                  // pinned host staging for gb200_trace_batch
     size_t stage_cap = 0;
     // An asynchronous call (gb200_render_device / gb200_lineprofile_device with async != 0) returns while its kernels still
@@ -413,10 +412,16 @@ static int upload_ic_and_tables(gb200_ctx* ctx, const gb200_ic* ic, const gb200_
     return GB200_OK;
 }
 
+static int check_table(gb200_ctx* ctx, int32_t geometry_kind) {
+    if (geometry_kind == GB200_GEOMETRY_THICK_TABLE && ctx->cs_n < 2)
+        return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "GB200_GEOMETRY_THICK_TABLE needs a table: call gb200_set_cross_section first");
+    return GB200_OK;
+}
+
 // GB200_GEOMETRY_THICK_TABLE: point the launch at the context's cross-section table
 static int bind_geometry(gb200_ctx* ctx, GbParams& P) {
+    { int rc_ = check_table(ctx, P.geometry_kind); if (rc_) return rc_; }
     if (P.geometry_kind != GB200_GEOMETRY_THICK_TABLE) return GB200_OK;
-    if (ctx->cs_n < 2) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "GB200_GEOMETRY_THICK_TABLE needs a table: call gb200_set_cross_section first");
     P.cs_n = ctx->cs_n; P.cs_rho = ctx->d_cs; P.cs_h = ctx->d_cs + ctx->cs_n;
     P.gp0 = ctx->cs_max;
     return GB200_OK;
@@ -479,6 +484,15 @@ static int ensure_streams(gb200_ctx* ctx, size_t n) {
     return GB200_OK;
 }
 
+static int ensure_events(gb200_ctx* ctx, size_t n) {
+    while (ctx->chunk_events.size() < n) {
+        cudaEvent_t ev;
+        CU(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        ctx->chunk_events.push_back(ev);
+    }
+    return GB200_OK;
+}
+
 // ---------------------------------------------------------------- pipelined host-output launches
 // Large host-output calls are pipelined: the range is cut into chunks of whole tile strips, the chunk kernels alternate
 // between two streams (the next chunk's CTAs take over the SMs as the previous chunk drains, so there is no idle tail
@@ -501,11 +515,7 @@ static int run_pipelined(gb200_ctx* ctx, const gb200_range* rg, const GbParams& 
     const int64_t unit = pipeline_unit(P);
     const int64_t per = ((rg->count / unit + K - 1) / K) * unit;
     int rc = ensure_streams(ctx, 2); if (rc) return rc;
-    while (ctx->chunk_events.size() < (size_t)K + 2) {
-        cudaEvent_t ev;
-        CU(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-        ctx->chunk_events.push_back(ev);
-    }
+    rc = ensure_events(ctx, (size_t)K + 2); if (rc) return rc;
     cudaStream_t alt = ctx->pool_streams[0], copy = ctx->pool_streams[1];
     void* qv = nullptr;
     rc = pool_get(ctx, SL_BATCH_QUEUE, sizeof(unsigned long long) * 4 * K, &qv); if (rc) return rc;
@@ -624,6 +634,99 @@ static int fan_in(gb200_ctx* ctx, int nstreams) {
         CU(ctx, cudaEventRecord(ctx->ev2, ctx->pool_streams[(size_t)sidx]));
         CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev2, 0));
     }
+    return GB200_OK;
+}
+
+// The sequence of every batch call, after its validation: lay the items out, stage the inputs, launch the items with rays
+// round-robin on up to 32 pool streams, copy the outputs back and scatter them.  The call supplies
+//   rays(b)                        item b's ray count (an empty item keeps its place in the layout but does not launch),
+//   layout(b, in, out, P, io)      item b's inputs and outputs, as take() calls on the two Arenas,
+//   setup(b, P, io) -> rc          the parameters of an item with rays, before its layout binds the device pointers,
+//   launch(P, io, stream) -> err   its kernel,
+//   scatter(b, P, io)              item b's outputs from the staging buffer to the caller, P and io pointing into it.
+// With `queues`, every item gets its own ticket queue and step counters, reset before the launches and added to the stats.
+// Set-up stays interleaved with the launches: a non-Kerr ISCO costs milliseconds of host time, during which the items
+// already launched run.  stats: launches, rays and counters; kernel_ms = total_ms = the whole call.
+template <class Rays, class Layout, class Setup, class Launch, class Scatter>
+static int run_batch(gb200_ctx* ctx, int nbatch, bool queues, Rays&& rays, Layout&& layout, Setup&& setup, Launch&& launch, Scatter&& scatter) {
+    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
+    const int nstreams = nbatch < 32 ? nbatch : 32;
+    int rc = ensure_streams(ctx, (size_t)nstreams); if (rc) return rc;
+    GbParams S{}; // pointers of the passes over the staging buffer and of the items that do not launch
+    GbDualIO Sio{};
+    Arena size_in{nullptr}, size_out{nullptr};
+    for (int b = 0; b < nbatch; ++b) layout(b, size_in, size_out, S, Sio);
+    const size_t in_bytes = size_in.used, total = in_bytes + size_out.used;
+    void* arena_v = nullptr;
+    rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
+    char* arena = (char*)arena_v;
+    rc = ensure_stage(ctx, total); if (rc) return rc;
+    char* stage = (char*)ctx->stage;
+    unsigned long long* qs = nullptr;
+    const size_t qbytes = queues ? sizeof(unsigned long long) * 4 * (size_t)nbatch : 0;
+    if (queues) { void* qv = nullptr; rc = pool_get(ctx, SL_BATCH_QUEUE, qbytes, &qv); if (rc) return rc; qs = (unsigned long long*)qv; }
+    Arena stage_in{stage, true}, stage_out{stage + in_bytes};
+    for (int b = 0; b < nbatch; ++b) layout(b, stage_in, stage_out, S, Sio);
+    CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    if (queues) CU(ctx, cudaMemsetAsync(qs, 0, qbytes, ctx->stream));
+    if (in_bytes) CU(ctx, cudaMemcpyAsync(arena, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    rc = fan_out(ctx, nstreams); if (rc) return rc;
+    Arena dev_in{arena}, dev_out{arena + in_bytes};
+    for (int b = 0; b < nbatch; ++b) {
+        if (!rays(b)) { layout(b, dev_in, dev_out, S, Sio); continue; } // the item keeps its place, and its table may be shared
+        GbParams P;
+        GbDualIO io;
+        memset(&io, 0, sizeof io);
+        if ((rc = setup(b, P, io))) break;
+        layout(b, dev_in, dev_out, P, io);
+        if (queues) { P.queue = qs + 4 * (size_t)b; P.counters = P.queue + 1; }
+        const cudaError_t e = launch(P, io, ctx->pool_streams[(size_t)(b % nstreams)]);
+        if (e != cudaSuccess) { rc = fail(ctx, GB200_ERR_CUDA, "launch of batch item %d: %s", b, cudaGetErrorString(e)); break; }
+        ctx->stats.launches += 1;
+    }
+    const int joined = fan_in(ctx, nstreams);
+    if (rc) { // the items launched so far end before the error returns: the next call stages into the same arena
+        if (!joined) cudaStreamSynchronize(ctx->stream);
+        return rc;
+    }
+    if (joined) return joined;
+    std::vector<unsigned long long> c(qbytes / sizeof(unsigned long long));
+    if (total > in_bytes) CU(ctx, cudaMemcpyAsync(stage + in_bytes, arena + in_bytes, total - in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    if (queues) CU(ctx, cudaMemcpyAsync(c.data(), qs, qbytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    Arena host_in{stage}, host_out{stage + in_bytes};
+    for (int b = 0; b < nbatch; ++b) {
+        layout(b, host_in, host_out, S, Sio);
+        if (rays(b)) scatter(b, S, Sio);
+        ctx->stats.rays += rays(b);
+    }
+    float tot = 0;
+    cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
+    ctx->stats.kernel_ms = tot; ctx->stats.total_ms = tot;
+    add_counters(ctx, c.data(), c.size() / 4);
+    return GB200_OK;
+}
+
+// gb200_fp64_peak and gb200_fp64_issue_probe: launch(d, blocks, iters) runs blocks x 256 threads of 64 FMAs per iteration;
+// the rate is the best of repetitions 1..3 (repetition 0 warms up)
+template <class Launch> static int fp64_rate(gb200_ctx* ctx, Launch&& launch, double* tflops_out) {
+    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
+    void* d;
+    int rc = pool_get(ctx, SL_SCRATCH, 64, &d); if (rc) return rc;
+    const int blocks = ctx->sm_count * 8, iters = 20000;
+    double best = 0;
+    for (int rep = 0; rep < 4; ++rep) {
+        CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+        CU(ctx, launch((double*)d, blocks, iters));
+        CU(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
+        CU(ctx, cudaStreamSynchronize(ctx->stream));
+        float ms = 0;
+        cudaEventElapsedTime(&ms, ctx->ev1, ctx->ev2);
+        const double tf = 2.0 * 64.0 * (double)iters * 256.0 * (double)blocks / (ms * 1e-3) / 1e12;
+        if (rep > 0 && tf > best) best = tf;
+    }
+    *tflops_out = best;
     return GB200_OK;
 }
 
@@ -799,62 +902,26 @@ int gb200_trace_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* probl
         rc = validate_range(ctx, &ics[b], &ranges[b]); if (rc) return rc;
         if (ics[b].kind == GB200_IC_IMPACT_PARAMETERS) return fail(ctx, GB200_ERR_UNSUPPORTED, "impact-parameter lists are not batched; use gb200_trace / gb200_render");
     }
-    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
-    const int nstreams = nbatch < 32 ? nbatch : 32;
-    int rc = ensure_streams(ctx, (size_t)nstreams); if (rc) return rc;
-    // inputs: the explicit ICs; outputs: the endpoint arrays the caller asked for
-    auto layout = [&](int b, Arena& in, Arena& out, GbParams& P) {
-        if (ics[b].kind == GB200_IC_EXPLICIT)
-            for (int k = 0; k < 4; ++k) { in.take(P.ex[k], ics[b].n, ics[b].x[k]); in.take(P.ev[k], ics[b].n, ics[b].v[k]); }
-        endpoint_arrays(outs[b], P, [&](auto* h, auto*& f, int) { if (h) out.take(f, ranges[b].count); });
-    };
-    GbParams S{}; // pointers of the passes over the staging buffer
-    Arena size_in{nullptr}, size_out{nullptr};
-    for (int b = 0; b < nbatch; ++b) layout(b, size_in, size_out, S);
-    const size_t in_bytes = size_in.used, total = in_bytes + size_out.used;
-    void* arena_v = nullptr;
-    rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
-    char* arena = (char*)arena_v;
-    rc = ensure_stage(ctx, total); if (rc) return rc;
-    char* stage = (char*)ctx->stage;
-    void* qv = nullptr;
-    rc = pool_get(ctx, SL_BATCH_QUEUE, sizeof(unsigned long long) * 4 * (size_t)nbatch, &qv); if (rc) return rc;
-    unsigned long long* queues = (unsigned long long*)qv;
-    Arena stage_in{stage, true}, stage_out{stage + in_bytes};
-    for (int b = 0; b < nbatch; ++b) layout(b, stage_in, stage_out, S);
-    CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    CU(ctx, cudaMemsetAsync(queues, 0, sizeof(unsigned long long) * 4 * (size_t)nbatch, ctx->stream));
-    if (in_bytes) CU(ctx, cudaMemcpyAsync(arena, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    rc = fan_out(ctx, nstreams); if (rc) return rc;
-    Arena dev_in{arena}, dev_out{arena + in_bytes};
-    for (int b = 0; b < nbatch; ++b) {
-        cudaStream_t st = ctx->pool_streams[(size_t)(b % nstreams)];
-        GbParams P;
-        fill_params(&problems[b], &ics[b], &ranges[b], P);
-        { int rcg_ = bind_geometry(ctx, P); if (rcg_) return rcg_; }
-        layout(b, dev_in, dev_out, P);
-        P.queue = queues + 4 * (size_t)b;
-        P.counters = P.queue + 1;
-        int blocks = 0;
-        if (ranges[b].count) { CU(ctx, gb200_launch_trace(P, ctx->sm_count, st, &blocks)); ctx->stats.launches += 1; }
-    }
-    rc = fan_in(ctx, nstreams); if (rc) return rc;
-    std::vector<unsigned long long> c((size_t)nbatch * 4);
-    if (total > in_bytes) CU(ctx, cudaMemcpyAsync(stage + in_bytes, arena + in_bytes, total - in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaMemcpyAsync(c.data(), queues, sizeof(unsigned long long) * c.size(), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    Arena host_in{stage}, host_out{stage + in_bytes};
-    for (int b = 0; b < nbatch; ++b) { // scatter the staging buffer into the caller's SoA
-        layout(b, host_in, host_out, S);
-        endpoint_arrays(outs[b], S, [&](auto* h, auto* f, int) { if (h) memcpy(h, f, (size_t)ranges[b].count * sizeof(*f)); });
-    }
-    float tot = 0, dev = 0;
-    cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
+    for (int b = 0; b < nbatch; ++b) { int rc = check_table(ctx, problems[b].geometry_kind); if (rc) return rc; }
+    int rc = run_batch(ctx, nbatch, true, [&](int b) { return ranges[b].count; },
+        // inputs: the explicit ICs; outputs: the endpoint arrays the caller asked for
+        [&](int b, Arena& in, Arena& out, GbParams& P, GbDualIO&) {
+            if (ics[b].kind == GB200_IC_EXPLICIT)
+                for (int k = 0; k < 4; ++k) { in.take(P.ex[k], ics[b].n, ics[b].x[k]); in.take(P.ev[k], ics[b].n, ics[b].v[k]); }
+            endpoint_arrays(outs[b], P, [&](auto* h, auto*& f, int) { if (h) out.take(f, ranges[b].count); });
+        },
+        [&](int b, GbParams& P, GbDualIO&) {
+            fill_params(&problems[b], &ics[b], &ranges[b], P);
+            return bind_geometry(ctx, P);
+        },
+        [&](GbParams& P, GbDualIO&, cudaStream_t st) { int blocks = 0; return gb200_launch_trace(P, ctx->sm_count, st, &blocks); },
+        [&](int b, GbParams& S, GbDualIO&) { // the staging buffer into the caller's SoA
+            endpoint_arrays(outs[b], S, [&](auto* h, auto* f, int) { if (h) memcpy(h, f, (size_t)ranges[b].count * sizeof(*f)); });
+        });
+    if (rc) return rc;
+    float dev = 0;
     cudaEventElapsedTime(&dev, ctx->ev1, ctx->ev2); // launches only (ev2: the end of the last pool stream), without the two staged copies
-    ctx->stats.kernel_ms = dev; ctx->stats.total_ms = tot;
-    for (int b = 0; b < nbatch; ++b) ctx->stats.rays += ranges[b].count;
-    add_counters(ctx, c.data(), (size_t)nbatch);
+    ctx->stats.kernel_ms = dev;
     return GB200_OK;
 }
 
@@ -1008,70 +1075,28 @@ int gb200_render_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* prob
         if (ics[b].kind == GB200_IC_EXPLICIT) return fail(ctx, GB200_ERR_UNSUPPORTED, "explicit initial conditions are batched by gb200_trace_batch");
         for (int k = 0; k < npf; ++k) if (ranges[b].count && !images[(size_t)b * npf + k]) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null image pointer");
     }
-    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
-    const int nstreams = nbatch < 32 ? nbatch : 32;
-    rc = ensure_streams(ctx, (size_t)nstreams); if (rc) return rc;
-    // inputs: the impact-parameter lists (+ heights) and the plunging table; outputs: the images
-    auto layout = [&](int b, Arena& in, Arena& out, GbParams& P) {
-        if (ics[b].kind == GB200_IC_IMPACT_PARAMETERS)
-            for (int k = 0; k < 3; ++k) if (ics[b].x[k]) in.take(P.ex[k], ics[b].n, ics[b].x[k]);
-        place_plunging(in, pls, b, P);
-        for (int k = 0; k < npf; ++k) out.take(P.o_img[k], ranges[b].count);
-    };
-    GbParams S{}; // pointers of the passes over the staging buffer and of the items that do not launch
-    Arena size_in{nullptr}, size_out{nullptr};
-    for (int b = 0; b < nbatch; ++b) layout(b, size_in, size_out, S);
-    const size_t in_bytes = size_in.used, total = in_bytes + size_out.used;
-    void* arena_v = nullptr;
-    rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
-    char* arena = (char*)arena_v;
-    rc = ensure_stage(ctx, total); if (rc) return rc;
-    char* stage = (char*)ctx->stage;
-    void* qv = nullptr;
-    rc = pool_get(ctx, SL_BATCH_QUEUE, sizeof(unsigned long long) * 4 * (size_t)nbatch, &qv); if (rc) return rc;
-    unsigned long long* queues = (unsigned long long*)qv;
-    Arena stage_in{stage, true}, stage_out{stage + in_bytes};
-    for (int b = 0; b < nbatch; ++b) layout(b, stage_in, stage_out, S);
-    CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    CU(ctx, cudaMemsetAsync(queues, 0, sizeof(unsigned long long) * 4 * (size_t)nbatch, ctx->stream));
-    if (in_bytes) CU(ctx, cudaMemcpyAsync(arena, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    rc = fan_out(ctx, nstreams); if (rc) return rc;
+    for (int b = 0; b < nbatch; ++b) if (ranges[b].count) { rc = check_table(ctx, problems[b].geometry_kind); if (rc) return rc; }
     const bool want_isco = needs_isco(pfs, npf, false);
-    Arena dev_in{arena}, dev_out{arena + in_bytes};
-    for (int b = 0; b < nbatch; ++b) {
-        if (!ranges[b].count) { layout(b, dev_in, dev_out, S); continue; } // the item keeps its place, and its table may be shared
-        cudaStream_t st = ctx->pool_streams[(size_t)(b % nstreams)];
-        GbParams P;
-        fill_params(&problems[b], &ics[b], &ranges[b], P);
-        { int rcg_ = bind_geometry(ctx, P); if (rcg_) return rcg_; }
-        if (want_isco) { rc = set_isco(ctx, &problems[b], P); if (rc) return rc; }
-        layout(b, dev_in, dev_out, P);
-        P.npf = npf;
-        for (int k = 0; k < npf; ++k) P.pf[k] = pfs[k];
-        P.queue = queues + 4 * (size_t)b;
-        P.counters = P.queue + 1;
-        int blocks = 0;
-        CU(ctx, gb200_launch_trace(P, ctx->sm_count, st, &blocks));
-        ctx->stats.launches += 1;
-    }
-    rc = fan_in(ctx, nstreams); if (rc) return rc;
-    std::vector<unsigned long long> c((size_t)nbatch * 4);
-    if (total > in_bytes) CU(ctx, cudaMemcpyAsync(stage + in_bytes, arena + in_bytes, total - in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaMemcpyAsync(c.data(), queues, sizeof(unsigned long long) * c.size(), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    Arena host_in{stage}, host_out{stage + in_bytes};
-    for (int b = 0; b < nbatch; ++b) {
-        layout(b, host_in, host_out, S);
-        for (int k = 0; k < npf; ++k)
-            if (ranges[b].count) memcpy(images[(size_t)b * npf + k], S.o_img[k], 8 * (size_t)ranges[b].count);
-    }
-    float tot = 0;
-    cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
-    ctx->stats.kernel_ms = tot; ctx->stats.total_ms = tot;
-    for (int b = 0; b < nbatch; ++b) ctx->stats.rays += ranges[b].count;
-    add_counters(ctx, c.data(), (size_t)nbatch);
-    return GB200_OK;
+    return run_batch(ctx, nbatch, true, [&](int b) { return ranges[b].count; },
+        // inputs: the impact-parameter lists (+ heights) and the plunging table; outputs: the images
+        [&](int b, Arena& in, Arena& out, GbParams& P, GbDualIO&) {
+            if (ics[b].kind == GB200_IC_IMPACT_PARAMETERS)
+                for (int k = 0; k < 3; ++k) if (ics[b].x[k]) in.take(P.ex[k], ics[b].n, ics[b].x[k]);
+            place_plunging(in, pls, b, P);
+            for (int k = 0; k < npf; ++k) out.take(P.o_img[k], ranges[b].count);
+        },
+        [&](int b, GbParams& P, GbDualIO&) {
+            fill_params(&problems[b], &ics[b], &ranges[b], P);
+            int rc_ = bind_geometry(ctx, P); if (rc_) return rc_;
+            if (want_isco) { rc_ = set_isco(ctx, &problems[b], P); if (rc_) return rc_; }
+            P.npf = npf;
+            for (int k = 0; k < npf; ++k) P.pf[k] = pfs[k];
+            return GB200_OK;
+        },
+        [&](GbParams& P, GbDualIO&, cudaStream_t st) { int blocks = 0; return gb200_launch_trace(P, ctx->sm_count, st, &blocks); },
+        [&](int b, GbParams& S, GbDualIO&) {
+            for (int k = 0; k < npf; ++k) memcpy(images[(size_t)b * npf + k], S.o_img[k], 8 * (size_t)ranges[b].count);
+        });
 }
 
 // ---------------------------------------------------------------- forward-mode traces (gb200_dual.cu)
@@ -1094,65 +1119,33 @@ int gb200_trace_dual_batch(gb200_ctx* ctx, int32_t nbatch, const gb200_problem* 
         int rc = validate(ctx, &problems[b], &f); if (rc) return rc;
         if (d.height && problems[b].geometry_kind != GB200_GEOMETRY_DATUM_PLANE) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "per-ray heights need GB200_GEOMETRY_DATUM_PLANE");
     }
-    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
-    const int nstreams = nbatch < 32 ? nbatch : 32;
-    int rc = ensure_streams(ctx, (size_t)nstreams); if (rc) return rc;
-    // inputs: the seeded impact parameters (+ heights) and the plunging table; outputs: the arrays the caller asked for
-    auto layout = [&](int b, Arena& in, Arena& out, GbParams& P, GbDualIO& io) {
-        const gb200_dual_ic& d = ics[b];
-        in.take(io.alpha, d.n, d.alpha); in.take(io.beta, d.n, d.beta);
-        in.take(io.dalpha, d.n * d.npartials, d.dalpha); in.take(io.dbeta, d.n * d.npartials, d.dbeta);
-        if (d.height) in.take(io.height, d.n, d.height);
-        place_plunging(in, pls, b, P);
-        dual_arrays(outs[b], io, d.n, d.npartials, [&](auto* h, auto*& f, int64_t n) { if (h) out.take(f, n); });
-    };
-    GbParams S{}; // pointers of the passes over the staging buffer and of the items that do not launch
-    GbDualIO Sio{};
-    Arena size_in{nullptr}, size_out{nullptr};
-    for (int b = 0; b < nbatch; ++b) layout(b, size_in, size_out, S, Sio);
-    const size_t in_bytes = size_in.used, total = in_bytes + size_out.used;
-    void* arena_v = nullptr;
-    rc = pool_get(ctx, SL_BATCH, total + 256, &arena_v); if (rc) return rc;
-    char* arena = (char*)arena_v;
-    rc = ensure_stage(ctx, total); if (rc) return rc;
-    char* stage = (char*)ctx->stage;
-    Arena stage_in{stage, true}, stage_out{stage + in_bytes};
-    for (int b = 0; b < nbatch; ++b) layout(b, stage_in, stage_out, S, Sio);
-    CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    if (in_bytes) CU(ctx, cudaMemcpyAsync(arena, stage, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    rc = fan_out(ctx, nstreams); if (rc) return rc;
-    Arena dev_in{arena}, dev_out{arena + in_bytes};
     for (int b = 0; b < nbatch; ++b) {
-        const gb200_dual_ic& d = ics[b];
-        if (d.n == 0) { layout(b, dev_in, dev_out, S, Sio); continue; } // the item keeps its place, and its table may be shared
-        gb200_range rg{0, d.n, 1, 1};
-        GbParams P;
-        fill_params(&problems[b], &fake[(size_t)b], &rg, P);
-        { int rcg_ = bind_geometry(ctx, P); if (rcg_) return rcg_; }
-        if (outs[b].g) { rc = set_isco(ctx, &problems[b], P); if (rc) return rc; }
+        if (!ics[b].n) continue;
+        int rc = check_table(ctx, problems[b].geometry_kind); if (rc) return rc;
         if (outs[b].dg && !outs[b].g) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "dg needs g");
-        GbDualIO io;
-        memset(&io, 0, sizeof io);
-        io.n = d.n; io.npartials = d.npartials; io.norm_partials = (norm_mode == GB200_DUAL_NORM_WITH_PARTIALS) ? 1 : 0;
-        layout(b, dev_in, dev_out, P, io);
-        CU(ctx, gb200_launch_dual(P, io, ctx->pool_streams[(size_t)(b % nstreams)]));
-        ctx->stats.launches += 1;
-        ctx->stats.rays += d.n;
     }
-    rc = fan_in(ctx, nstreams); if (rc) return rc;
-    if (total > in_bytes) CU(ctx, cudaMemcpyAsync(stage + in_bytes, arena + in_bytes, total - in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaEventRecord(ctx->ev3, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    Arena host_in{stage}, host_out{stage + in_bytes};
-    for (int b = 0; b < nbatch; ++b) {
-        layout(b, host_in, host_out, S, Sio);
-        if (ics[b].n)
+    return run_batch(ctx, nbatch, false, [&](int b) { return ics[b].n; },
+        // inputs: the seeded impact parameters (+ heights) and the plunging table; outputs: the arrays the caller asked for
+        [&](int b, Arena& in, Arena& out, GbParams& P, GbDualIO& io) {
+            const gb200_dual_ic& d = ics[b];
+            in.take(io.alpha, d.n, d.alpha); in.take(io.beta, d.n, d.beta);
+            in.take(io.dalpha, d.n * d.npartials, d.dalpha); in.take(io.dbeta, d.n * d.npartials, d.dbeta);
+            if (d.height) in.take(io.height, d.n, d.height);
+            place_plunging(in, pls, b, P);
+            dual_arrays(outs[b], io, d.n, d.npartials, [&](auto* h, auto*& f, int64_t n) { if (h) out.take(f, n); });
+        },
+        [&](int b, GbParams& P, GbDualIO& io) {
+            const gb200_range rg{0, ics[b].n, 1, 1};
+            fill_params(&problems[b], &fake[(size_t)b], &rg, P);
+            int rc_ = bind_geometry(ctx, P); if (rc_) return rc_;
+            if (outs[b].g) { rc_ = set_isco(ctx, &problems[b], P); if (rc_) return rc_; }
+            io.n = ics[b].n; io.npartials = ics[b].npartials; io.norm_partials = (norm_mode == GB200_DUAL_NORM_WITH_PARTIALS) ? 1 : 0;
+            return GB200_OK;
+        },
+        [&](GbParams& P, GbDualIO& io, cudaStream_t st) { return gb200_launch_dual(P, io, st); },
+        [&](int b, GbParams&, GbDualIO& Sio) {
             dual_arrays(outs[b], Sio, ics[b].n, ics[b].npartials, [&](auto* h, auto* f, int64_t n) { if (h) memcpy(h, f, (size_t)n * sizeof(*f)); });
-    }
-    float tot = 0;
-    cudaEventElapsedTime(&tot, ctx->ev0, ctx->ev3);
-    ctx->stats.kernel_ms = tot; ctx->stats.total_ms = tot;
-    return GB200_OK;
+        });
 }
 
 int gb200_trace_dual(gb200_ctx* ctx, const gb200_problem* p, const gb200_dual_ic* ic, int32_t norm_mode,
@@ -1276,14 +1269,34 @@ static std::mutex g_nccl_mutex;
 struct gb200_comm {
     std::vector<gb200_ctx*> ctx;
     std::vector<ncclComm_t> nccl; // empty when ndev == 1 and NCCL is unavailable
-    std::vector<double*> d_flux;  // per device: nbins doubles
-    int flux_cap = 0;
 };
 #define NC(call)                                                                                                         \
     do {                                                                                                                 \
         ncclResult_t r__ = (call);                                                                                       \
         if (r__ != ncclSuccess) return fail(nullptr, GB200_ERR_CUDA, "%s: %s", #call, g_nccl.GetErrorString(r__));       \
     } while (0)
+
+// One in-place all-reduce of a device buffer
+struct NcclReduce {
+    void* buf;
+    size_t count;
+    ncclDataType_t type;
+    ncclRedOp_t op;
+};
+
+// ops[d]: the all-reduces of device d, enqueued on its context's stream; all of them run as one NCCL group.  Nothing to do
+// on one device.
+static int all_reduce(const std::vector<gb200_ctx*>& ctxs, const ncclComm_t* nccl, const std::vector<std::vector<NcclReduce>>& ops) {
+    if (ctxs.size() < 2) return GB200_OK;
+    NC(g_nccl.GroupStart());
+    for (size_t d = 0; d < ctxs.size(); ++d)
+        for (const NcclReduce& o : ops[d]) {
+            ncclResult_t r = g_nccl.AllReduce(o.buf, o.buf, o.count, o.type, o.op, nccl[d], ctxs[d]->stream);
+            if (r != ncclSuccess) { g_nccl.GroupEnd(); return fail(nullptr, GB200_ERR_CUDA, "ncclAllReduce: %s", g_nccl.GetErrorString(r)); }
+        }
+    NC(g_nccl.GroupEnd());
+    return GB200_OK;
+}
 
 // rank d's share of the rays: whole strips of four image columns / theta-rows, strip d, d + n, ... (DESIGN.md section 6)
 static gb200_range shard_range(const gb200_ic* ic, int d, int n) {
@@ -1328,7 +1341,6 @@ int gb200_comm_init(const int32_t* devices, int32_t ndev, gb200_comm** out) {
 void gb200_comm_destroy(gb200_comm* c) {
     if (!c) return;
     for (size_t d = 0; d < c->ctx.size(); ++d) {
-        if (d < c->d_flux.size() && c->d_flux[d]) { cudaSetDevice(c->ctx[d]->device); cudaFree(c->d_flux[d]); }
         if (d < c->nccl.size() && c->nccl[d]) g_nccl.CommDestroy(c->nccl[d]);
         gb200_destroy(c->ctx[d]);
     }
@@ -1342,35 +1354,24 @@ int gb200_comm_lineprofile(gb200_comm* c, const gb200_problem* p, const gb200_ic
                            const double* bins, int32_t nbins, const gb200_lineprofile_opts* opts, double* flux_out) {
     if (!c || !ic || !opts || !flux_out) return fail(nullptr, GB200_ERR_INVALID_ARGUMENT, "null argument");
     const int n = (int)c->ctx.size();
-    if (c->flux_cap < nbins) {
-        c->d_flux.resize((size_t)n, nullptr);
-        for (int d = 0; d < n; ++d) {
-            CU(c->ctx[(size_t)d], cudaSetDevice(c->ctx[(size_t)d]->device));
-            if (c->d_flux[(size_t)d]) cudaFree(c->d_flux[(size_t)d]);
-            CU(c->ctx[(size_t)d], cudaMalloc(&c->d_flux[(size_t)d], sizeof(double) * (size_t)nbins));
-        }
-        c->flux_cap = nbins;
-    }
     // every device traces its strips and bins them into its own raw histogram (asynchronous launches, one host thread) ...
+    std::vector<std::vector<NcclReduce>> sums((size_t)n);
     for (int d = 0; d < n; ++d) {
         gb200_ctx* ctx = c->ctx[(size_t)d];
         gb200_range rg = shard_range(ic, d, n);
-        int rc = lineprofile_common(ctx, p, ic, &rg, em, pl, bins, nbins, opts, c->d_flux[(size_t)d], true, ctx->stream, 1);
+        void* flux = nullptr;
+        CU(ctx, cudaSetDevice(ctx->device));
+        int rc = pool_get(ctx, SL_FLUX, sizeof(double) * (size_t)nbins, &flux);
+        if (!rc) rc = lineprofile_common(ctx, p, ic, &rg, em, pl, bins, nbins, opts, (double*)flux, true, ctx->stream, 1);
         if (rc) return fail(nullptr, rc, "device %d: %s", ctx->device, ctx->err.c_str());
+        sums[(size_t)d] = {{flux, (size_t)nbins, ncclDouble, ncclSum}};
     }
     // ... one all-reduce over NVLink sums them in place on every device's own stream ...
-    if (n > 1) {
-        NC(g_nccl.GroupStart());
-        for (int d = 0; d < n; ++d) {
-            ncclResult_t r = g_nccl.AllReduce(c->d_flux[(size_t)d], c->d_flux[(size_t)d], (size_t)nbins, ncclDouble, ncclSum, c->nccl[(size_t)d], c->ctx[(size_t)d]->stream);
-            if (r != ncclSuccess) { g_nccl.GroupEnd(); return fail(nullptr, GB200_ERR_CUDA, "ncclAllReduce: %s", g_nccl.GetErrorString(r)); }
-        }
-        NC(g_nccl.GroupEnd());
-    }
+    { int rc_ = all_reduce(c->ctx, c->nccl.data(), sums); if (rc_) return rc_; }
     // ... and device 0 hands the sum to the host, which normalises it (flux ./ sum(flux), line-profiles.jl:197)
     std::vector<double> h((size_t)nbins);
     CU(c->ctx[0], cudaSetDevice(c->ctx[0]->device));
-    CU(c->ctx[0], cudaMemcpyAsync(h.data(), c->d_flux[0], sizeof(double) * (size_t)nbins, cudaMemcpyDeviceToHost, c->ctx[0]->stream));
+    CU(c->ctx[0], cudaMemcpyAsync(h.data(), sums[0][0].buf, sizeof(double) * (size_t)nbins, cudaMemcpyDeviceToHost, c->ctx[0]->stream));
     for (int d = 0; d < n; ++d) {
         CU(c->ctx[(size_t)d], cudaSetDevice(c->ctx[(size_t)d]->device));
         CU(c->ctx[(size_t)d], cudaStreamSynchronize(c->ctx[(size_t)d]->stream));
@@ -1386,9 +1387,8 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
     const int K = 4; // chunks per device: a chunk's images travel to the host while the next chunks compute
     std::vector<gb200_range> rgs((size_t)n);
     std::vector<std::vector<double*>> dimg((size_t)n);
-    std::vector<std::vector<cudaEvent_t>> done((size_t)n);
+    std::vector<int> nch((size_t)n, 0); // chunks of device d: their kernels end at chunk_events[ch], their copies at [K + ch]
     std::vector<int64_t> per((size_t)n, 0);
-    auto cleanup = [&]() { for (auto& v : done) for (auto e : v) cudaEventDestroy(e); };
     // all launches first (asynchronous, one host thread): the devices compute concurrently
     for (int d = 0; d < n; ++d) {
         gb200_ctx* ctx = c->ctx[(size_t)d];
@@ -1396,12 +1396,12 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
         rg = shard_range(ic, d, n);
         if (rg.block < 1) rg.block = 1;
         CU(ctx, cudaSetDevice(ctx->device));
-        { int rc = ensure_streams(ctx, 2); if (rc) return rc; }
+        { int rc = ensure_streams(ctx, 2); if (!rc) rc = ensure_events(ctx, 2 * K); if (rc) return rc; }
         dimg[(size_t)d].resize((size_t)npf);
         for (int k = 0; k < npf; ++k) {
             void* dv = nullptr;
             int rc = pool_get(ctx, SL_IMG0 + k, sizeof(double) * (size_t)rg.count + 8, &dv);
-            if (rc) { cleanup(); return fail(nullptr, rc, "device %d: %s", ctx->device, ctx->err.c_str()); }
+            if (rc) return fail(nullptr, rc, "device %d: %s", ctx->device, ctx->err.c_str());
             dimg[(size_t)d][(size_t)k] = (double*)dv;
         }
         if (rg.count == 0) continue;
@@ -1413,11 +1413,8 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
             double* sub_img[GB_MAX_PF];
             for (int k = 0; k < npf; ++k) sub_img[k] = dimg[(size_t)d][(size_t)k] + s0;
             int rc = render_common(ctx, p, ic, &sub, pfs, npf, pl, sub_img, true, ctx->stream, 1);
-            if (rc) { cleanup(); return fail(nullptr, rc, "device %d: %s", ctx->device, ctx->err.c_str()); }
-            cudaEvent_t ev;
-            CU(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            done[(size_t)d].push_back(ev);
-            CU(ctx, cudaEventRecord(ev, ctx->stream));
+            if (rc) return fail(nullptr, rc, "device %d: %s", ctx->device, ctx->err.c_str());
+            CU(ctx, cudaEventRecord(ctx->chunk_events[(size_t)nch[(size_t)d]++], ctx->stream));
         }
     }
     // Results travel chunk by chunk: a contiguous copy into the device's pinned staging buffer on its copy stream (truly
@@ -1425,8 +1422,6 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
     // the caller's (pageable) images -- strip b of a device sits at ray first + b * stride * block.  A strided copy
     // straight into pageable memory is staged by the driver on the calling thread and serialises the devices (measured:
     // 8 GPUs 15.1 ms for the 2048 x 2048 render whose kernels take 5.3 ms).
-    std::vector<std::vector<cudaEvent_t>> copied((size_t)n);
-    auto cleanup2 = [&]() { for (auto& v : copied) for (auto e : v) cudaEventDestroy(e); };
     for (int d = 0; d < n; ++d) {
         gb200_ctx* ctx = c->ctx[(size_t)d];
         const gb200_range& rg = rgs[(size_t)d];
@@ -1436,31 +1431,28 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
     }
     for (int ch = 0; ch < K; ++ch)
         for (int d = 0; d < n; ++d) {
-            if ((size_t)ch >= done[(size_t)d].size()) continue;
+            if (ch >= nch[(size_t)d]) continue;
             gb200_ctx* ctx = c->ctx[(size_t)d];
             const gb200_range& rg = rgs[(size_t)d];
             const int64_t s0 = (int64_t)ch * per[(size_t)d], cnt = std::min(per[(size_t)d], rg.count - s0);
             CU(ctx, cudaSetDevice(ctx->device));
             cudaStream_t copy = ctx->pool_streams[1];
-            CU(ctx, cudaStreamWaitEvent(copy, done[(size_t)d][(size_t)ch], 0));
+            CU(ctx, cudaStreamWaitEvent(copy, ctx->chunk_events[(size_t)ch], 0));
             for (int k = 0; k < npf; ++k)
                 CU(ctx, cudaMemcpyAsync((double*)ctx->stage + (size_t)k * (size_t)rg.count + s0, dimg[(size_t)d][(size_t)k] + s0,
                                         sizeof(double) * (size_t)cnt, cudaMemcpyDeviceToHost, copy));
-            cudaEvent_t ev;
-            CU(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            copied[(size_t)d].push_back(ev);
-            CU(ctx, cudaEventRecord(ev, copy));
+            CU(ctx, cudaEventRecord(ctx->chunk_events[(size_t)(K + ch)], copy));
         }
     std::vector<cudaError_t> terr((size_t)n, cudaSuccess);
     std::vector<std::thread> workers;
     for (int d = 0; d < n; ++d) {
-        if (copied[(size_t)d].empty()) continue;
+        if (!nch[(size_t)d]) continue;
         workers.emplace_back([&, d]() {
             gb200_ctx* ctx = c->ctx[(size_t)d];
             const gb200_range& rg = rgs[(size_t)d];
             const size_t blk = (size_t)rg.block;
-            for (size_t ch = 0; ch < copied[(size_t)d].size(); ++ch) {
-                const cudaError_t e = cudaEventSynchronize(copied[(size_t)d][ch]);
+            for (int ch = 0; ch < nch[(size_t)d]; ++ch) {
+                const cudaError_t e = cudaEventSynchronize(ctx->chunk_events[(size_t)(K + ch)]);
                 if (e != cudaSuccess) { terr[(size_t)d] = e; return; }
                 const int64_t s0 = (int64_t)ch * per[(size_t)d], cnt = std::min(per[(size_t)d], rg.count - s0);
                 for (int k = 0; k < npf; ++k) {
@@ -1477,13 +1469,11 @@ int gb200_comm_render(gb200_comm* c, const gb200_problem* p, const gb200_ic* ic,
     for (auto& w : workers) w.join();
     for (int d = 0; d < n; ++d) {
         gb200_ctx* ctx = c->ctx[(size_t)d];
-        if (terr[(size_t)d] != cudaSuccess) { cleanup(); cleanup2(); return fail(nullptr, GB200_ERR_CUDA, "device %d: %s", ctx->device, cudaGetErrorString(terr[(size_t)d])); }
+        if (terr[(size_t)d] != cudaSuccess) return fail(nullptr, GB200_ERR_CUDA, "device %d: %s", ctx->device, cudaGetErrorString(terr[(size_t)d]));
         CU(ctx, cudaSetDevice(ctx->device));
         if (ctx->pool_streams.size() >= 2) CU(ctx, cudaStreamSynchronize(ctx->pool_streams[1]));
         CU(ctx, cudaStreamSynchronize(ctx->stream));
     }
-    cleanup2();
-    cleanup();
     return GB200_OK;
 }
 
@@ -1592,18 +1582,9 @@ static int lagtransfer_run(const std::vector<gb200_ctx*>& ctxs, const ncclComm_t
         CU(ctx, gb200_launch_lag_samples(P, img, gp, o->E0, rg.count, D.samples, partial, nblocks, D.scal, ctx->stream));
         ctx->stats.launches += 2;
     }
-    if (n > 1) {
-        NC(g_nccl.GroupStart());
-        for (int d = 0; d < n; ++d) {
-            GbLagScalars* s = dv[(size_t)d].scal;
-            const cudaStream_t st = ctxs[(size_t)d]->stream;
-            ncclResult_t r = g_nccl.AllReduce(s->mn, s->mn, 2, ncclDouble, ncclMin, nccl[d], st);
-            if (r == ncclSuccess) r = g_nccl.AllReduce(s->mx, s->mx, 4, ncclDouble, ncclMax, nccl[d], st);
-            if (r == ncclSuccess) r = g_nccl.AllReduce(&s->hits, &s->hits, 1, ncclInt64, ncclSum, nccl[d], st);
-            if (r != ncclSuccess) { g_nccl.GroupEnd(); return fail(nullptr, GB200_ERR_CUDA, "ncclAllReduce: %s", g_nccl.GetErrorString(r)); }
-        }
-        NC(g_nccl.GroupEnd());
-    }
+    std::vector<std::vector<NcclReduce>> ops;
+    for (const Dev& D : dv) ops.push_back({{D.scal->mn, 2, ncclDouble, ncclMin}, {D.scal->mx, 4, ncclDouble, ncclMax}, {&D.scal->hits, 1, ncclInt64, ncclSum}});
+    rc = all_reduce(ctxs, nccl, ops); if (rc) return rc;
     for (int d = 0; d < n; ++d) {
         gb200_ctx* ctx = ctxs[(size_t)d];
         Dev& D = dv[(size_t)d];
@@ -1618,17 +1599,9 @@ static int lagtransfer_run(const std::vector<gb200_ctx*>& ctxs, const ncclComm_t
         CU(ctx, gb200_launch_lag_bin(D.scal, L, D.out + ncell, D.out + ncell + o->N_E, D.samples, D.count, D.cells, D.counts, nblocks, ctx->stream));
         ctx->stats.launches += D.count > 0 ? 2 : 1;
     }
-    if (n > 1) {
-        NC(g_nccl.GroupStart());
-        for (int d = 0; d < n; ++d) {
-            const Dev& D = dv[(size_t)d];
-            const cudaStream_t st = ctxs[(size_t)d]->stream;
-            ncclResult_t r = g_nccl.AllReduce(D.cells, D.cells, (size_t)ncell + 1, ncclInt64, ncclSum, nccl[d], st);
-            if (r == ncclSuccess) r = g_nccl.AllReduce(D.counts, D.counts, (size_t)ncell, ncclUint32, ncclSum, nccl[d], st);
-            if (r != ncclSuccess) { g_nccl.GroupEnd(); return fail(nullptr, GB200_ERR_CUDA, "ncclAllReduce: %s", g_nccl.GetErrorString(r)); }
-        }
-        NC(g_nccl.GroupEnd());
-    }
+    ops.clear();
+    for (const Dev& D : dv) ops.push_back({{D.cells, (size_t)ncell + 1, ncclInt64, ncclSum}, {D.counts, (size_t)ncell, ncclUint32, ncclSum}});
+    rc = all_reduce(ctxs, nccl, ops); if (rc) return rc;
     gb200_ctx* c0 = ctxs[0];
     const Dev& D0 = dv[0];
     GbLagScalars s;
@@ -1745,70 +1718,51 @@ static int tf_quad_run(gb200_ctx* ctx, bool lag, int32_t ntables, const gb200_tf
         G.time0 = nprof;
         nprof += 2 * (int64_t)G.time_n;
     }
-    // staging layout, every array 256-byte aligned
-    size_t used = 0;
-    auto place = [&](size_t bytes) { const size_t at = used; used += (bytes + 255) & ~(size_t)255; return at; };
-    const size_t at_tab = place(sizeof(GbTfTable) * tabs.size()), at_mod = place(sizeof(GbTfModel) * mods.size());
-    const size_t at_re = place(8 * (size_t)nrad), at_gmin = place(8 * (size_t)nrad), at_gmax = place(8 * (size_t)nrad);
-    const size_t at_off = place(8 * (size_t)noff), at_gs = place(8 * (size_t)nknot), at_f = place(8 * (size_t)nknot), at_t = place(8 * (size_t)nknot);
-    const size_t at_radii = place(8 * (size_t)nann), at_prof = place(8 * (size_t)nprof), at_g = place(8 * (size_t)ngrid);
-    const size_t at_tg = place(8 * (size_t)(lag ? nt : 0)), at_x = place(8 * (size_t)o->npoints), at_w = place(8 * (size_t)o->npoints);
+    // Every array of the call in one arena, laid out as in the batch calls (Arena).  The tables' and the models' arrays are
+    // concatenated, so the fill pass copies them piece by piece, the branch offsets becoming knot indices of the whole call.
+    GbTfArgs A{};
+    auto layout = [&](Arena& a) {
+        a.take(A.tables, ntables, tabs.data()); a.take(A.models, nmodels, mods.data());
+        a.take(A.r_e, nrad); a.take(A.gmin, nrad); a.take(A.gmax, nrad);
+        a.take(A.off, noff); a.take(A.gs, nknot); a.take(A.f, nknot); a.take(A.t, nknot);
+        a.take(A.radii, nann); a.take(A.prof, nprof); a.take(A.g_grid, ngrid, g_grid);
+        if (lag) a.take(A.t_grid, nt, t_grid);
+        a.take(A.nodes, o->npoints, o->nodes); a.take(A.weights, o->npoints, o->weights);
+        if (!a.fill) return;
+        auto put = [](const auto* dst, int64_t at, const void* src, int64_t n) { memcpy((void*)(dst + at), src, sizeof(*dst) * (size_t)n); };
+        int64_t k0 = 0;
+        for (int i = 0; i < ntables; ++i) {
+            const gb200_tf_branches& T = tables[i];
+            const GbTfTable& G = tabs[(size_t)i];
+            put(A.r_e, G.radius0, T.r_e, T.n_radii); put(A.gmin, G.radius0, T.gmin, T.n_radii); put(A.gmax, G.radius0, T.gmax, T.n_radii);
+            int64_t* off = (int64_t*)A.off + G.off0;
+            for (int b = 0; b <= 2 * T.n_radii; ++b) off[b] = k0 + T.off[b];
+            const int64_t nk = T.off[2 * T.n_radii];
+            put(A.gs, k0, T.gs, nk); put(A.f, k0, T.f, nk); put(A.t, k0, T.t, nk);
+            k0 += nk;
+        }
+        for (int m = 0; m < nmodels; ++m) {
+            const gb200_tf_model& M = models[m];
+            const GbTfModel& G = mods[(size_t)m];
+            put(A.radii, G.radius0, M.radii, M.n_radii);
+            if (G.emis_n) { put(A.prof, G.emis0, M.profile.emissivity.r, G.emis_n); put(A.prof, G.emis0 + G.emis_n, M.profile.emissivity.eps, G.emis_n); }
+            if (G.time_n) { put(A.prof, G.time0, M.profile.r, G.time_n); put(A.prof, G.time0 + G.time_n, M.profile.t, G.time_n); }
+        }
+    };
+    Arena size{nullptr};
+    layout(size);
     const size_t nout = (size_t)nmodels * (size_t)ngrid * (size_t)nt;
     { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
     void *din, *dout;
-    rc = pool_get(ctx, SL_TFQ_IN, used, &din); if (rc) return rc;
+    rc = pool_get(ctx, SL_TFQ_IN, size.used, &din); if (rc) return rc;
     rc = pool_get(ctx, SL_TFQ_OUT, sizeof(double) * nout, &dout); if (rc) return rc;
     CU(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    rc = ensure_stage(ctx, used); if (rc) return rc;
-    char* st = (char*)ctx->stage;
-    memcpy(st + at_tab, tabs.data(), sizeof(GbTfTable) * tabs.size());
-    memcpy(st + at_mod, mods.data(), sizeof(GbTfModel) * mods.size());
-    for (int i = 0; i < ntables; ++i) {
-        const gb200_tf_branches& T = tables[i];
-        const GbTfTable& G = tabs[(size_t)i];
-        memcpy(st + at_re + 8 * G.radius0, T.r_e, 8 * (size_t)T.n_radii);
-        memcpy(st + at_gmin + 8 * G.radius0, T.gmin, 8 * (size_t)T.n_radii);
-        memcpy(st + at_gmax + 8 * G.radius0, T.gmax, 8 * (size_t)T.n_radii);
-    }
-    int64_t k0 = 0;
-    for (int i = 0; i < ntables; ++i) { // offsets become knot indices of the whole call
-        const gb200_tf_branches& T = tables[i];
-        int64_t* off = (int64_t*)(st + at_off) + tabs[(size_t)i].off0;
-        const int64_t nk = T.off[2 * T.n_radii];
-        for (int b = 0; b <= 2 * T.n_radii; ++b) off[b] = k0 + T.off[b];
-        memcpy(st + at_gs + 8 * k0, T.gs, 8 * (size_t)nk);
-        memcpy(st + at_f + 8 * k0, T.f, 8 * (size_t)nk);
-        memcpy(st + at_t + 8 * k0, T.t, 8 * (size_t)nk);
-        k0 += nk;
-    }
-    for (int m = 0; m < nmodels; ++m) {
-        const gb200_tf_model& M = models[m];
-        const GbTfModel& G = mods[(size_t)m];
-        memcpy(st + at_radii + 8 * G.radius0, M.radii, 8 * (size_t)M.n_radii);
-        double* prof = (double*)(st + at_prof);
-        if (G.emis_n) {
-            memcpy(prof + G.emis0, M.profile.emissivity.r, 8 * (size_t)G.emis_n);
-            memcpy(prof + G.emis0 + G.emis_n, M.profile.emissivity.eps, 8 * (size_t)G.emis_n);
-        }
-        if (G.time_n) {
-            memcpy(prof + G.time0, M.profile.r, 8 * (size_t)G.time_n);
-            memcpy(prof + G.time0 + G.time_n, M.profile.t, 8 * (size_t)G.time_n);
-        }
-    }
-    memcpy(st + at_g, g_grid, 8 * (size_t)ngrid);
-    if (lag) memcpy(st + at_tg, t_grid, 8 * (size_t)nt);
-    memcpy(st + at_x, o->nodes, 8 * (size_t)o->npoints);
-    memcpy(st + at_w, o->weights, 8 * (size_t)o->npoints);
-    CU(ctx, cudaMemcpyAsync(din, st, used, cudaMemcpyHostToDevice, ctx->stream));
-    char* d = (char*)din;
-    GbTfArgs A;
-    A.tables = (const GbTfTable*)(d + at_tab); A.models = (const GbTfModel*)(d + at_mod);
-    A.r_e = (const double*)(d + at_re); A.gmin = (const double*)(d + at_gmin); A.gmax = (const double*)(d + at_gmax);
-    A.off = (const int64_t*)(d + at_off);
-    A.gs = (const double*)(d + at_gs); A.f = (const double*)(d + at_f); A.t = (const double*)(d + at_t);
-    A.radii = (const double*)(d + at_radii); A.prof = (const double*)(d + at_prof);
-    A.g_grid = (const double*)(d + at_g); A.t_grid = lag ? (const double*)(d + at_tg) : nullptr;
-    A.nodes = (const double*)(d + at_x); A.weights = (const double*)(d + at_w);
+    rc = ensure_stage(ctx, size.used); if (rc) return rc;
+    Arena stage{(char*)ctx->stage, true};
+    layout(stage);
+    CU(ctx, cudaMemcpyAsync(din, ctx->stage, size.used, cudaMemcpyHostToDevice, ctx->stream));
+    Arena dev{(char*)din};
+    layout(dev);
     A.nmodels = nmodels; A.ngrid = ngrid; A.nt = nt; A.upscale = o->upscale; A.npoints = o->npoints; A.normalise = o->normalise;
     A.h = o->h; A.t0 = lag ? o->t0 : 0.0;
     A.out = (double*)dout;
@@ -1890,74 +1844,33 @@ int gb200_debug_rhs(gb200_ctx* ctx, int32_t metric_kind, const double* mp, int64
     return GB200_OK;
 }
 
-int gb200_debug_math(gb200_ctx* ctx, int64_t n, const double* x, double* out5) {
-    if (!ctx || !x || !out5 || n < 1) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad arguments");
+// gb200_debug_math and gb200_debug_math_lo: `width` outputs per input through `launch`
+static int debug_math(gb200_ctx* ctx, int64_t n, const double* x, double* out, int width,
+                      cudaError_t (*launch)(long long, const double*, double*, cudaStream_t)) {
+    if (!ctx || !x || !out || n < 1) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad arguments");
     { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
     void *d_x, *d_o;
     int rc = pool_get(ctx, SL_X0, sizeof(double) * (size_t)n, &d_x); if (rc) return rc;
-    rc = pool_get(ctx, SL_V0, sizeof(double) * 5 * (size_t)n, &d_o); if (rc) return rc;
+    rc = pool_get(ctx, SL_V0, sizeof(double) * width * (size_t)n, &d_o); if (rc) return rc;
     CU(ctx, cudaMemcpyAsync(d_x, x, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, gb200_launch_debug_math(n, (const double*)d_x, (double*)d_o, ctx->stream));
-    CU(ctx, cudaMemcpyAsync(out5, d_o, sizeof(double) * 5 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, launch(n, (const double*)d_x, (double*)d_o, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(out, d_o, sizeof(double) * width * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return GB200_OK;
 }
 
-int gb200_debug_math_lo(gb200_ctx* ctx, int64_t n, const double* x, double* out2) {
-    if (!ctx || !x || !out2 || n < 1) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad arguments");
-    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
-    void *d_x, *d_o;
-    int rc = pool_get(ctx, SL_X0, sizeof(double) * (size_t)n, &d_x); if (rc) return rc;
-    rc = pool_get(ctx, SL_V0, sizeof(double) * 2 * (size_t)n, &d_o); if (rc) return rc;
-    CU(ctx, cudaMemcpyAsync(d_x, x, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    CU(ctx, gb200_launch_debug_math_lo(n, (const double*)d_x, (double*)d_o, ctx->stream));
-    CU(ctx, cudaMemcpyAsync(out2, d_o, sizeof(double) * 2 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    return GB200_OK;
-}
+int gb200_debug_math(gb200_ctx* ctx, int64_t n, const double* x, double* out5) { return debug_math(ctx, n, x, out5, 5, gb200_launch_debug_math); }
+
+int gb200_debug_math_lo(gb200_ctx* ctx, int64_t n, const double* x, double* out2) { return debug_math(ctx, n, x, out2, 2, gb200_launch_debug_math_lo); }
 
 int gb200_fp64_peak(gb200_ctx* ctx, double* tflops_out) {
     if (!ctx || !tflops_out) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "null argument");
-    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
-    void* d;
-    int rc = pool_get(ctx, SL_SCRATCH, 64, &d); if (rc) return rc;
-    const int blocks = ctx->sm_count * 8, iters = 20000;
-    double best = 0;
-    for (int rep = 0; rep < 4; ++rep) {
-        CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-        CU(ctx, gb200_launch_dfma((double*)d, blocks, iters, ctx->stream));
-        CU(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
-        CU(ctx, cudaStreamSynchronize(ctx->stream));
-        float ms = 0;
-        cudaEventElapsedTime(&ms, ctx->ev1, ctx->ev2);
-        const double flop = 2.0 * 64.0 * (double)iters * 256.0 * (double)blocks; // 64 FMAs per iteration per thread
-        const double tf = flop / (ms * 1e-3) / 1e12;
-        if (rep > 0 && tf > best) best = tf;
-    }
-    ctx->fp64_peak = best;
-    *tflops_out = best;
-    return GB200_OK;
+    return fp64_rate(ctx, [&](double* d, int blocks, int iters) { return gb200_launch_dfma(d, blocks, iters, ctx->stream); }, tflops_out);
 }
 
 int gb200_fp64_issue_probe(gb200_ctx* ctx, int32_t mix, double* tflops_out) {
     if (!ctx || !tflops_out || mix < 0 || mix > 5) return fail(ctx, GB200_ERR_INVALID_ARGUMENT, "bad argument");
-    { int rc_ = begin_call(ctx, ctx->stream); if (rc_) return rc_; }
-    void* d;
-    int rc = pool_get(ctx, SL_SCRATCH, 64, &d); if (rc) return rc;
-    const int blocks = ctx->sm_count * 8, iters = 20000;
-    double best = 0;
-    for (int rep = 0; rep < 4; ++rep) {
-        CU(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-        CU(ctx, gb200_launch_dfma_mix((double*)d, blocks, iters, mix, ctx->stream));
-        CU(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
-        CU(ctx, cudaStreamSynchronize(ctx->stream));
-        float ms = 0;
-        cudaEventElapsedTime(&ms, ctx->ev1, ctx->ev2);
-        const double tf = 2.0 * 64.0 * (double)iters * 256.0 * (double)blocks / (ms * 1e-3) / 1e12;
-        if (rep > 0 && tf > best) best = tf;
-    }
-    *tflops_out = best;
-    return GB200_OK;
+    return fp64_rate(ctx, [&](double* d, int blocks, int iters) { return gb200_launch_dfma_mix(d, blocks, iters, mix, ctx->stream); }, tflops_out);
 }
 
 } // extern "C"

@@ -1,7 +1,8 @@
 """The batch entry points against single calls of the same items, bit for bit, for the cases their shared host plumbing
 (one arena per batch, laid out per item, with plunging tables shared between consecutive items) has to get right: partial
 outputs, empty items, mixed initial conditions, shared tables and per-ray heights; and the pipelined single call with
-partial outputs against the one-launch path."""
+partial outputs against the one-launch path.  A batch that fails returns with nothing of it running, and fails before its
+first launch where the host can tell."""
 import ctypes as C
 import math
 
@@ -176,3 +177,77 @@ def test_pipelined_trace_with_partial_outputs_equals_one_launch(ensemble, monkey
     assert [s[1:] for s in st_p] == [s[1:] for s in st_1]
     for got, want in zip(piped, single):
         _same_arrays(got, want, ENDPOINT_FIELDS)
+
+
+def _dual_item(ensemble, n):
+    m = gb.KerrMetric(1.0, 0.9)
+    rng = np.random.default_rng(n)
+    cfg = api.tracing_configuration(m, [0.0, 1e4, math.radians(40.0), 0.0], api.ImpactParameters(np.ones(1), np.ones(1)), gb.DatumPlane(0.0),
+                                    2e4, chart=gb.chart_for_metric(m, 2e4), ensemble=ensemble)
+    return cfg.to_c()[0], None, cabi.DualArrays(rng.uniform(-10, 10, n), rng.uniform(-10, 10, n), np.ones((1, n)), np.zeros((1, n)))
+
+
+def _batch(lib, ctx, call, items):
+    """`items`, [(problem, ic, rays)], as one gb200_<call>_batch; its return code.  rays: a count, or trace_dual's DualArrays."""
+    nb = len(items)
+    problems = (cabi.Problem * nb)(*[p for p, _, _ in items])
+    if call == "trace_dual":
+        return lib.gb200_trace_dual_batch(ctx, nb, problems, (cabi.DualIC * nb)(*[a.ic for _, _, a in items]), cabi.DUAL_NORM_WITH_PARTIALS,
+                                          None, (cabi.DualOut * nb)(*[a.out for _, _, a in items]))
+    ics = (cabi.IC * nb)(*[ic for _, ic, _ in items])
+    ranges = (cabi.Range * nb)(*[cabi.Range(0, n, 1) for _, _, n in items])
+    if call == "trace":
+        outs = [cabi.EndpointArrays(n) for _, _, n in items]
+        return lib.gb200_trace_batch(ctx, nb, problems, ics, ranges, (cabi.Endpoints * nb)(*[o.c for o in outs]))
+    images = [np.zeros(n) for _, _, n in items]
+    return lib.gb200_render_batch(ctx, nb, problems, ics, ranges, cabi.iptr(np.array([cabi.PF_STATUS], np.int32)), 1, None,
+                                  (cabi._dp * nb)(*[cabi.dptr(img) for img in images]))
+
+
+@pytest.mark.parametrize("call, check", [("trace", "table"), ("render", "table"), ("trace_dual", "table"), ("trace_dual", "dg")])
+def test_batch_whose_later_item_fails_a_host_check_launches_nothing(ensemble, call, check):
+    """GB200_GEOMETRY_THICK_TABLE without a cross-section table, or a dual item asking for dg but not g, fails the batch before
+    its first item launches: the stats keep the launch count of the last successful call."""
+    lib = cabi.load()
+    ctx = ensemble.ctx(ensemble.devices[0])
+    cabi.check(lib.gb200_set_cross_section(ctx, None, None, 0), ctx)
+    if call == "trace_dual":
+        good, empty, bad = _dual_item(ensemble, 50), _dual_item(ensemble, 0), _dual_item(ensemble, 40)
+    else:
+        p, ic = (_lamp_post(ensemble, 64) if call == "trace" else common.c1(16, 16, ensemble=ensemble)[3]).to_c()
+        good, empty, bad = (p, ic, ic.n), (p, ic, 0), (cabi.Problem.from_buffer_copy(p), ic, ic.n)
+    if check == "table":
+        bad[0].geometry_kind = cabi.GEOMETRY_THICK_TABLE
+    else:
+        bad[2].out.g = cabi.dptr(None)
+    cabi.check(_batch(lib, ctx, call, [empty]), ctx)
+    assert ensemble.stats().launches == 0
+    assert _batch(lib, ctx, call, [good, bad]) == cabi.ERR_INVALID_ARGUMENT
+    assert (b"GB200_GEOMETRY_THICK_TABLE needs a table" if check == "table" else b"dg needs g") in lib.gb200_last_error(ctx)
+    assert ensemble.stats().launches == 0
+
+
+def test_render_batch_failing_after_a_launch_leaves_nothing_running(ensemble):
+    """A metric without an ISCO is found on the host only when its item's turn comes, after the items before it launched:
+    the batch returns the error once those have finished, so the next batch on the context has its arena to itself."""
+    lib = cabi.load()
+    ctx = ensemble.ctx(ensemble.devices[0])
+    kerr = common.c1(1024, 1024, ensemble=ensemble)[3].to_c()
+    jp = common.render_config(gb.JohannsenPsaltisMetric(1.0, 0.8831, 0.4), [0.0, 1000.0, math.radians(60.0), 0.0], gb.ThinDisc(0.0, 50.0),
+                              2000.0, 16, 16, ensemble=ensemble).to_c()
+    pfs = np.array([cabi.PF_REDSHIFT], np.int32)
+
+    def render(items):
+        nb = len(items)
+        images = [np.zeros(ic.n) for _, ic in items]
+        rc = lib.gb200_render_batch(ctx, nb, (cabi.Problem * nb)(*[p for p, _ in items]), (cabi.IC * nb)(*[ic for _, ic in items]),
+                                    (cabi.Range * nb)(*[cabi.Range(0, ic.n, 1) for _, ic in items]), cabi.iptr(pfs), 1, None,
+                                    (cabi._dp * nb)(*[cabi.dptr(img) for img in images]))
+        return rc, images[0]
+
+    rc, before = render([kerr])
+    cabi.check(rc, ctx)
+    assert render([kerr, jp])[0] == cabi.ERR_INVALID_ARGUMENT and b"no ISCO" in lib.gb200_last_error(ctx)
+    rc, after = render([kerr])
+    cabi.check(rc, ctx)
+    assert np.isfinite(before).any() and np.array_equal(after, before, equal_nan=True)
