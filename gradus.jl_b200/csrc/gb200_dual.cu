@@ -3,8 +3,9 @@
 //                          (alpha, beta)) for the transfer-function solvers, src/tracing/precision-solvers.jl:73-131,401-451
 //   gb200_path_kernel      one geodesic with every accepted step recorded (save_on = true, src/tracing/tracing.jl:66-108)
 // One ray per thread.  These launches carry 10^2..10^5 rays between host-side root-finding rounds: they are latency
-// bound, not throughput bound, and share no code with the throughput kernel of gb200_trace.cu beyond the metric
-// closed forms -- tests/test_gpu_dual.py holds the two integrators to the same end points.
+// bound, not throughput bound: their integrator is not the throughput kernel's of gb200_trace.cu, but the metric closed
+// forms, the disc conditions, the endpoint redshift and the v^t constraint are the same templates of gb200_device.cuh --
+// tests/test_gpu_dual.py holds the two integrators to the same end points.
 #include <cuda_runtime.h>
 #include "gb200_generic.cuh"
 #include "gb200_internal.h"
@@ -42,7 +43,7 @@ __global__ void __launch_bounds__(64) gb200_dual_kernel(const __grid_constant__ 
     if (io.g) {
         const bool hit = res.status == GB200_STATUS_INTERSECTED_WITH_GEOMETRY && res.flags == 0;
         S g_(nan(""));
-        if (hit) g_ = redshift_endpoint_g<S>(P, res.u, res.u + 4, E_obs);
+        if (hit) g_ = redshift_endpoint<-1>(P, res.u, res.u + 4, E_obs);
         io.g[i] = g_.v;
         if (io.dg) for (int k = 0; k < N; ++k) io.dg[(size_t)k * io.n + i] = hit ? g_.d[k] : nan("");
     }
@@ -60,7 +61,7 @@ cudaError_t gb200_launch_dual(const GbParams& P, const GbDualIO& io, cudaStream_
 
 // ---------------------------------------------------------------- closest approach to a target point
 // The objective of optimize_for_target (src/tracing/precision-solvers.jl:452-546) over a set of rays: one ray per thread
-// through the generic integrator with the distance condition (disc_condition_g, GB200_GEOMETRY_TARGET_POINT).
+// through the generic integrator with the distance condition (disc_condition, GB200_GEOMETRY_TARGET_POINT).
 template <int MK>
 __global__ void __launch_bounds__(64) gb200_target_kernel(const __grid_constant__ GbParams P) {
     const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -115,7 +116,7 @@ __global__ void gb200_path_kernel(const __grid_constant__ GbParams P, const doub
         GD<0> s, c, g[5], dr[5], dth[5];
         gd_sincos(u[2], s, c);
         metric_jacobian_kind<GD<0>>(P.metric_kind, P.mp, u[1], s, c, g, dr, dth);
-        u[4] = constrain_vt_g<GD<0>>(g, u[5], u[6], u[7], P.mu);
+        u[4] = constrain_vt(g, u[5], u[6], u[7], P.mu);
     }
     int rows = 0;
     GbPathRecord rec{cap, lam_out, u_out, &rows};

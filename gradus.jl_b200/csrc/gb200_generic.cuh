@@ -1,5 +1,8 @@
-// gb200_generic.cuh -- the integrator of gb200_trace.cu once more, written over a generic scalar: one ray per thread,
-// plain loops, every quantity of the state a dual number GD<N> carrying N partial derivatives (N = 0: plain doubles).
+// gb200_generic.cuh -- a second integrator beside the warp-cooperative one of gb200_trace.cu, written over a generic
+// scalar: one ray per thread, plain loops, every quantity of the state a dual number GD<N> carrying N partial derivatives
+// (N = 0: plain doubles).  The step loop and the right-hand sides are its own; the disc conditions, the endpoint
+// redshift, the v^t constraint and the Tsit5 tableau are gb200_device.cuh's, instantiated on GD<N> (the overloads of
+// gd_sqrt, gd_abs, gd_sin, gd_cos, gd_fmin and gd_fmax below keep each scalar type's own arithmetic).
 //
 // Two users:
 //   * N = 1, 2: the forward-mode traces of the transfer-function solvers.  The reference pushes ForwardDiff duals through
@@ -66,8 +69,7 @@ GD_T bool operator<(const GD<N>& a, double b) { return a.v < b; }
 GD_T bool operator>(const GD<N>& a, double b) { return a.v > b; }
 GD_T bool operator<=(const GD<N>& a, double b) { return a.v <= b; }
 GD_T bool operator>=(const GD<N>& a, double b) { return a.v >= b; }
-GB_HD inline double gd_sqrt(double x) { return sqrt(x); }
-GB_HD inline double gd_abs(double x) { return fabs(x); }
+GD_T bool operator<=(double a, const GD<N>& b) { return a <= b.v; }
 GD_T GD<N> gb_rcp(const GD<N>& a) { return 1.0 / a; } // the generated metric code calls gb_rcp on its scalar type
 GD_T GD<N> gd_sqrt(const GD<N>& a) { GD<N> r; r.v = sqrt(a.v); const double h = 0.5 / r.v; for (int i = 0; i < N; ++i) r.d[i] = h * a.d[i]; return r; }
 GD_T GD<N> gd_abs(const GD<N>& a) { return a.v < 0.0 ? -a : a; }
@@ -81,6 +83,11 @@ GD_T void gd_sincos(const GD<N>& a, GD<N>& s, GD<N>& c) {
     s.v = sv; c.v = cv;
     for (int i = 0; i < N; ++i) { s.d[i] = cv * a.d[i]; c.d[i] = -sv * a.d[i]; }
 }
+GD_T GD<N> gd_sin(const GD<N>& a) { GD<N> s, c; gd_sincos(a, s, c); return s; }
+GD_T GD<N> gd_cos(const GD<N>& a) { GD<N> s, c; gd_sincos(a, s, c); return c; }
+// clamps by compares and selects: a clamped value carries no derivative
+GD_T GD<N> gd_fmin(const GD<N>& a, double b) { return a > b ? GD<N>(b) : a; }
+GD_T GD<N> gd_fmax(const GD<N>& a, double b) { return a < b ? GD<N>(b) : a; }
 // |u| as DiffEqBase's internalnorm sees one dual: sqrt(value^2 + sum partials^2); values only: |value|
 GD_T double gd_norm1(const GD<N>& a, bool partials) {
     if (!partials || N == 0) return fabs(a.v);
@@ -187,120 +194,6 @@ GB_HD inline void rhs_g(const GbParams& P, const GD<N> u[8], GD<N> du[8], GD<N>&
     for (int i = 0; i < 4; ++i) { du[i] = u[4 + i]; du[4 + i] = acc[i]; }
 }
 
-template <class S>
-GB_HD inline S cross_section_table_g(const double* xs, const double* ys, int n, const S& x) { // cross_section_table over S
-    if (n < 2 || !(x >= xs[0]) || !(x <= xs[n - 1])) return S(-1.0);
-    int lo = 0, hi = n - 1;
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (x >= xs[mid]) lo = mid; else hi = mid; }
-    const S w = (x - xs[lo]) / (xs[lo + 1] - xs[lo]);
-    return (1.0 - w) * ys[lo] + w * ys[lo + 1];
-}
-// distance_to_disc over S, geometry chosen at run time (src/geometry/discs/*.jl, see disc_condition<GEOM>)
-template <class S>
-GB_HD inline S disc_condition_g(const GbParams& P, const S& r, const S& s, const S& c, double hgt, double ph = 0.0) {
-    if (P.geometry_kind == GB200_GEOMETRY_TARGET_POINT) {
-        // distance_callback of _make_target_objective (src/tracing/precision-solvers.jl:473-488): Euclidean distance between
-        // to_cartesian(u) (src/geometry/geometry.jl:13-16) and the target, minus d_tol; gp0..gp2 = target in Cartesian
-        // coordinates, gtol = d_tol.  phi enters as a value (no partials: this kind runs with N = 0 only).
-        double sp, cp;
-        sincos(ph, &sp, &cp);
-        const S rs = r * s;
-        const S dx = rs * cp - P.gp0, dy = rs * sp - P.gp1, dz = r * c - P.gp2;
-        return gd_sqrt(dx * dx + dy * dy + dz * dz) - P.gtol;
-    }
-    if (P.geometry_kind == GB200_GEOMETRY_THIN_DISC) {
-        const S rho = r * gd_abs(s);
-        if (rho < P.gp0 || rho > P.gp1) return S(1.0);
-        return r * gd_abs(c) - P.gtol * gd_abs(r);
-    } else if (P.geometry_kind == GB200_GEOMETRY_SHAKURA_SUNYAEV) {
-        const S rho = r * gd_abs(s);
-        if (rho < P.gp2) return S(1.0);
-        const S h = (3.0 * P.gp1 * P.gp0) * (1.0 - gd_sqrt(P.gp2 / rho));
-        if (h <= 0.0) return S(1.0);
-        return r * gd_abs(c) - h;
-    } else if (P.geometry_kind == GB200_GEOMETRY_DATUM_PLANE) {
-        return r * c - hgt;
-    } else if (P.geometry_kind == GB200_GEOMETRY_THICK_TABLE) {
-        const S h = cross_section_table_g<S>(P.cs_rho, P.cs_h, P.cs_n, r * gd_abs(s));
-        if (h <= 0.0) return S(1.0);
-        return r * gd_abs(c) - h;
-    }
-    return S(1.0);
-}
-
-// ---------------------------------------------------------------- redshift over S (redshift_endpoint<METRIC>)
-template <class S>
-GB_HD inline void circular_fourvelocity_g(const GbParams& P, const S& rho, S& ut_up, S& uph_up) {
-    S g[5], dr[5], dth[5];
-    metric_jacobian_kind<S>(P.metric_kind, P.mp, rho, S(1.0), S(0.0), g, dr, dth);
-    const S D = g[0] * g[3] - g[4] * g[4];
-    const S iD = 1.0 / D;
-    const S gitt = g[3] * iD, giphph = g[0] * iD, gitph = -(g[4] * iD);
-    const S disc = gd_sqrt(dr[4] * dr[4] - dr[0] * dr[3]);
-    const S Om = -(dr[4] - disc) / dr[3];
-    const S A = -(Om * gitt - gitph);
-    const S B = (Om * gitph - giphph);
-    const S denom = B * B * gitt + 2.0 * (A * B * gitph) + A * A * giphph;
-    const double sg = (denom > 0.0) ? 1.0 : ((denom < 0.0) ? -1.0 : 0.0);
-    const S d = -sg * gd_sqrt(1.0 / gd_abs(denom));
-    const S ut = B * d, uph = A * d;
-    ut_up = gitt * ut + gitph * uph;
-    uph_up = gitph * ut + giphph * uph;
-}
-template <class S>
-GB_HD inline S table_lerp_g(const double* xs, const double* ys, int n, const S& x) { // clamped abscissa: no derivative outside
-    S xc = x;
-    if (x < xs[0]) xc = S(xs[0]);
-    if (x > xs[n - 1]) xc = S(xs[n - 1]);
-    int lo = 0, hi = n - 1;
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (xc >= xs[mid]) lo = mid; else hi = mid; }
-    const S w = (xc - xs[lo]) / (xs[lo + 1] - xs[lo]);
-    return (1.0 - w) * ys[lo] + w * ys[lo + 1];
-}
-template <class S>
-GB_HD inline S redshift_endpoint_g(const GbParams& P, const S x[4], const S v[4], const S& E_obs) {
-    S sth, cth;
-    gd_sincos(x[2], sth, cth);
-    S rho = x[1] * gd_abs(sth);
-    S u0, u1(0.0), u3;
-    const bool kerr = P.metric_kind == GB200_METRIC_KERR;
-    if (!kerr && P.pl_n < 2 && rho < P.r_isco && rho >= P.r_isco * (1.0 - 1e-9)) rho = S(P.r_isco);
-    if (rho < P.r_isco) {
-        if (kerr) { // Cunningham (1975) plunging flow, src/redshift.jl:93-164
-            const double M = P.M, a = P.a, rms = P.r_isco;
-            const S r = rho;
-            const double sM = sqrt(M), srms = sqrt(rms);
-            const double Le = sM * (rms * rms - 2.0 * a * sqrt(M * rms) + a * a) / (rms * srms - 2.0 * M * srms + a * sM);
-            const S Del = r * r - 2.0 * M * r + a * a;
-            const S H = (2.0 * M * r - a * Le) / Del;
-            const double ge = sqrt(1.0 - (2.0 * M) / (3.0 * rms));
-            const S qq = rms / r - 1.0;
-            const S ur = -sqrt((2.0 * M) / (3.0 * rms)) * (qq * gd_sqrt(qq));
-            u3 = ge / (r * r) * (Le + a * H);
-            u0 = ge * (1.0 + 2.0 * M * (1.0 + H) / r);
-            u1 = -ur;
-        } else {
-            if (P.pl_n < 2) return S(nan(""));
-            u0 = table_lerp_g<S>(P.pl_r, P.pl_ut, P.pl_n, rho);
-            u1 = -table_lerp_g<S>(P.pl_r, P.pl_ur, P.pl_n, rho);
-            u3 = table_lerp_g<S>(P.pl_r, P.pl_uphi, P.pl_n, rho);
-        }
-    } else {
-        circular_fourvelocity_g<S>(P, rho, u0, u3);
-    }
-    S g[5], dr[5], dth[5];
-    metric_jacobian_kind<S>(P.metric_kind, P.mp, x[1], sth, cth, g, dr, dth);
-    const S Ed = (g[0] * v[0] + g[4] * v[3]) * u0 + (g[1] * v[1]) * u1 + (g[4] * v[0] + g[3] * v[3]) * u3;
-    return E_obs / Ed;
-}
-
-// constrain_time over S (auto-diff.jl:161-173)
-template <class S>
-GB_HD inline S constrain_vt_g(const S g[5], const S& vr, const S& vth, const S& vph, double mu) {
-    const S disc = -(g[0] * g[1] * vr * vr) - g[0] * g[2] * vth * vth - g[0] * (mu * mu) - (g[0] * g[3] - g[4] * g[4]) * vph * vph;
-    return -(g[4] * vph + gd_sqrt(disc)) / g[0];
-}
-
 // ---------------------------------------------------------------- the integrator
 template <int N>
 struct GenResult {
@@ -312,9 +205,11 @@ struct GenResult {
 };
 
 GB_HD inline void gen_dense_weights(double Th, double b[7], double db[7]) { // b_j(Theta) and d b_j / d Theta of the Tsit5 interpolant
-    const double R2[7] = {GB_R12_V, GB_R22_V, GB_R32_V, GB_R42_V, GB_R52_V, GB_R62_V, GB_R72_V};
-    const double R3[7] = {GB_R13_V, GB_R23_V, GB_R33_V, GB_R43_V, GB_R53_V, GB_R63_V, GB_R73_V};
-    const double R4[7] = {GB_R14_V, GB_R24_V, GB_R34_V, GB_R44_V, GB_R54_V, GB_R64_V, GB_R74_V};
+    // R_jk by name: indexing the list as gb_const(GB_I_R12 + 3 j) inside the loop costs the forward-mode kernels registers
+    // and stack (-Xptxas -v: 2 more registers in gb200_target_kernel<Kerr>, 352 bytes more stack in gb200_dual_kernel<1, Kerr>)
+    const double R2[7] = {gb_const(GB_I_R12), gb_const(GB_I_R22), gb_const(GB_I_R32), gb_const(GB_I_R42), gb_const(GB_I_R52), gb_const(GB_I_R62), gb_const(GB_I_R72)};
+    const double R3[7] = {gb_const(GB_I_R13), gb_const(GB_I_R23), gb_const(GB_I_R33), gb_const(GB_I_R43), gb_const(GB_I_R53), gb_const(GB_I_R63), gb_const(GB_I_R73)};
+    const double R4[7] = {gb_const(GB_I_R14), gb_const(GB_I_R24), gb_const(GB_I_R34), gb_const(GB_I_R44), gb_const(GB_I_R54), gb_const(GB_I_R64), gb_const(GB_I_R74)};
     for (int j = 0; j < 7; ++j) {
         const double lead = (j == 0) ? 1.0 : 0.0;
         b[j] = Th * (lead + Th * (R2[j] + Th * (R3[j] + Th * R4[j])));
@@ -342,23 +237,16 @@ GB_HD inline bool gen_scan_needed(const GbParams& P, double r0, double cprev, do
 // Stage input u + dt sum_l a_{S+1,l+1} k_l with the stage number as a template parameter: the coefficients are immediates
 // and the k rows are read at constant offsets (the run-time loop over l cost a fifth of the forward-mode kernel's
 // instructions in index arithmetic, compares and branches).  Same order of operations as the run-time loop.
-GB_HD constexpr double gen_a(int s, int l) {
-    return s == 1 ? GB_A21_V
-         : s == 2 ? (l == 0 ? GB_A31_V : GB_A32_V)
-         : s == 3 ? (l == 0 ? GB_A41_V : l == 1 ? GB_A42_V : GB_A43_V)
-         : s == 4 ? (l == 0 ? GB_A51_V : l == 1 ? GB_A52_V : l == 2 ? GB_A53_V : GB_A54_V)
-         : s == 5 ? (l == 0 ? GB_A61_V : l == 1 ? GB_A62_V : l == 2 ? GB_A63_V : l == 3 ? GB_A64_V : GB_A65_V)
-                  : (l == 0 ? GB_A71_V : l == 1 ? GB_A72_V : l == 2 ? GB_A73_V : l == 3 ? GB_A74_V : l == 4 ? GB_A75_V : GB_A76_V);
-}
 template <int N, int S>
 GB_HD inline void gen_stage_input(const GD<N> u[8], double dt, const GD<N> k[7][8], GD<N> tmp[8]) {
+    constexpr int a = GB_I_A21 + S * (S - 1) / 2; // a_{S+1,1}: the list holds the a_ij row by row
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-        if (S == 1) tmp[i] = u[i] + (dt * gen_a(1, 0)) * k[0][i];
+        if (S == 1) tmp[i] = u[i] + (dt * gb_const(a)) * k[0][i];
         else {
-            GD<N> acc = gen_a(S, 0) * k[0][i];
+            GD<N> acc = gb_const(a) * k[0][i];
 #pragma unroll
-            for (int l = 1; l < S; ++l) acc = acc + gen_a(S, l) * k[l][i];
+            for (int l = 1; l < S; ++l) acc = acc + gb_const(a + l) * k[l][i];
             tmp[i] = u[i] + dt * acc;
         }
     }
@@ -368,7 +256,6 @@ GB_HD inline void gen_stage_input(const GD<N> u[8], double dt, const GD<N> k[7][
 template <int N, int MK = -1, class REC>
 GB_HD inline void gen_trace_ray(const GbParams& P, const GD<N> u_init[8], double hgt, bool norm_partials, GenResult<N>& res, REC&& rec) {
     typedef GD<N> S;
-    const double BT[7] = {GB_BT1_V, GB_BT2_V, GB_BT3_V, GB_BT4_V, GB_BT5_V, GB_BT6_V, GB_BT7_V};
     const double abstol = P.abstol, reltol = P.reltol, dtmax = P.dtmax, dtmin = 2.220446049250313e-16, tstop = P.lam1;
     const double beta1 = 7.0 / 50.0, beta2 = 2.0 / 25.0, gamma = 9.0 / 10.0, qmin = 1.0 / 5.0, qmax = 10.0, qoldinit = 1e-4;
     const bool fast32 = P.pow_mode == GB200_POW_FAST32;
@@ -381,7 +268,7 @@ GB_HD inline void gen_trace_ray(const GbParams& P, const GD<N> u_init[8], double
     S s_, c_;
     rhs_g<N, MK>(P, u, k[0], s_, c_);
     const bool target = P.geometry_kind == GB200_GEOMETRY_TARGET_POINT;
-    double cprev = has_geom ? disc_condition_g<S>(P, u[1], s_, c_, hgt, u[3].v).v : 1.0;
+    double cprev = has_geom ? disc_condition<-1>(P, u[1], s_, c_, hgt, u[3].v).v : 1.0;
     res.closest = target ? cprev + P.gtol : nan("");
     double dt;
     { // ode_determine_initdt
@@ -428,8 +315,8 @@ GB_HD inline void gen_trace_ray(const GbParams& P, const GD<N> u_init[8], double
         {
             S at[8];
             for (int i = 0; i < 8; ++i) {
-                S e = BT[0] * k[0][i];
-                for (int l = 1; l < 7; ++l) e = e + BT[l] * k[l][i];
+                S e = gb_const(GB_I_BT1) * k[0][i];
+                for (int l = 1; l < 7; ++l) e = e + gb_const(GB_I_BT1 + l) * k[l][i];
                 at[i] = (dt * e) / (abstol + fmax(gd_norm1(u[i], norm_partials), gd_norm1(un[i], norm_partials)) * reltol);
             }
             EEst = gd_norm8(at, norm_partials);
@@ -456,7 +343,7 @@ GB_HD inline void gen_trace_ray(const GbParams& P, const GD<N> u_init[8], double
         bool event = false;
         double cnext = 1.0;
         if (has_geom) {
-            cnext = disc_condition_g<S>(P, un[1], s_, c_, hgt, un[3].v).v;
+            cnext = disc_condition<-1>(P, un[1], s_, c_, hgt, un[3].v).v;
             if (target) res.closest = fmin(res.closest, cnext + P.gtol);
             const double sprev = (cprev > 0.0) ? 1.0 : ((cprev < 0.0) ? -1.0 : 0.0);
             const double snext = (cnext > 0.0) ? 1.0 : ((cnext < 0.0) ? -1.0 : 0.0);
@@ -471,7 +358,7 @@ GB_HD inline void gen_trace_ray(const GbParams& P, const GD<N> u_init[8], double
                 rr = u[1].v + dt * rr; tt = u[2].v + dt * tt; pp = u[3].v + dt * pp;
                 double sv, cv;
                 sincos(tt, &sv, &cv);
-                const double cv_ = disc_condition_g<double>(P, rr, sv, cv, hgt, pp);
+                const double cv_ = disc_condition<-1>(P, rr, sv, cv, hgt, pp);
                 if (target) res.closest = fmin(res.closest, cv_ + P.gtol); // closest_approach[] is updated by every evaluation
                 return cv_;
             };
@@ -542,11 +429,11 @@ GB_HD inline void gen_trace_ray(const GbParams& P, const GD<N> u_init[8], double
                 if (N > 0) { // the event time moves with the parameters: Theta_p = -(dc/dp) / (dc/dTheta)
                     S se, ce;
                     gd_sincos(ue[2], se, ce);
-                    const S cD = disc_condition_g<S>(P, ue[1], se, ce, hgt);
+                    const S cD = disc_condition<-1>(P, ue[1], se, ce, hgt);
                     GD<2> r2(ue[1].v), t2(ue[2].v), s2, c2;
                     r2.d[0] = 1.0; t2.d[1] = 1.0;
                     gd_sincos(t2, s2, c2);
-                    const GD<2> cg = disc_condition_g<GD<2>>(P, r2, s2, c2, hgt);
+                    const GD<2> cg = disc_condition<-1>(P, r2, s2, c2, hgt);
                     const double dcdTh = cg.d[0] * dudTh[1] + cg.d[1] * dudTh[2];
                     if (dcdTh != 0.0 && dcdTh == dcdTh && fabs(dcdTh) < 1e300)
                         for (int kk = 0; kk < N; ++kk) {
@@ -591,6 +478,6 @@ GB_HD inline void gen_initial_state(const GbParams& P, const GD<N>& alpha, const
     u0[7] = P.c_ph0 + P.c_ph1 * pph;
     S go[5];
     for (int k = 0; k < 5; ++k) go[k] = S(P.go[k]);
-    u0[4] = constrain_vt_g<S>(go, u0[5], u0[6], u0[7], P.mu);
+    u0[4] = constrain_vt(go, u0[5], u0[6], u0[7], P.mu);
     E_obs = P.go[0] * u0[4] + P.go[4] * u0[7];
 }

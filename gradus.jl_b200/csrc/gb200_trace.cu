@@ -47,25 +47,25 @@ struct GbK {
 // k0 is the FSAL slope (k1 of the tableau); k[1..5] are k2..k6.
 template <int S>
 GB_D double comb(double u, double dt, double k0, const GbK& k) {
-    if (S == 1) return fma(dt * GB_A21, k0, u);
-    if (S == 2) return fma(dt, fma(GB_A32, k.get(1), GB_A31 * k0), u);
-    if (S == 3) return fma(dt, fma(GB_A43, k.get(2), fma(GB_A42, k.get(1), GB_A41 * k0)), u);
-    if (S == 4) return fma(dt, fma(GB_A54, k.get(3), fma(GB_A53, k.get(2), fma(GB_A52, k.get(1), GB_A51 * k0))), u);
-    if (S == 5) return fma(dt, fma(GB_A65, k.get(4), fma(GB_A64, k.get(3), fma(GB_A63, k.get(2), fma(GB_A62, k.get(1), GB_A61 * k0)))), u);
-    return fma(dt, fma(GB_A76, k.get(5), fma(GB_A75, k.get(4), fma(GB_A74, k.get(3), fma(GB_A73, k.get(2), fma(GB_A72, k.get(1), GB_A71 * k0))))), u);
+    if (S == 1) return fma(dt * GB_C(A21), k0, u);
+    if (S == 2) return fma(dt, fma(GB_C(A32), k.get(1), GB_C(A31) * k0), u);
+    if (S == 3) return fma(dt, fma(GB_C(A43), k.get(2), fma(GB_C(A42), k.get(1), GB_C(A41) * k0)), u);
+    if (S == 4) return fma(dt, fma(GB_C(A54), k.get(3), fma(GB_C(A53), k.get(2), fma(GB_C(A52), k.get(1), GB_C(A51) * k0))), u);
+    if (S == 5) return fma(dt, fma(GB_C(A65), k.get(4), fma(GB_C(A64), k.get(3), fma(GB_C(A63), k.get(2), fma(GB_C(A62), k.get(1), GB_C(A61) * k0)))), u);
+    return fma(dt, fma(GB_C(A76), k.get(5), fma(GB_C(A75), k.get(4), fma(GB_C(A74), k.get(3), fma(GB_C(A73), k.get(2), fma(GB_C(A72), k.get(1), GB_C(A71) * k0))))), u);
 }
 template <int S> GB_D constexpr double a7coef() {
-    return S == 0 ? GB_A71 : S == 1 ? GB_A72 : S == 2 ? GB_A73 : S == 3 ? GB_A74 : S == 4 ? GB_A75 : GB_A76;
+    return S == 0 ? GB_C(A71) : S == 1 ? GB_C(A72) : S == 2 ? GB_C(A73) : S == 3 ? GB_C(A74) : S == 4 ? GB_C(A75) : GB_C(A76);
 }
 template <int S> GB_D constexpr double btcoef() {
-    return S == 0 ? GB_BT1 : S == 1 ? GB_BT2 : S == 2 ? GB_BT3 : S == 3 ? GB_BT4 : S == 4 ? GB_BT5 : S == 5 ? GB_BT6 : GB_BT7;
+    return S == 0 ? GB_C(BT1) : S == 1 ? GB_C(BT2) : S == 2 ? GB_C(BT3) : S == 3 ? GB_C(BT4) : S == 4 ? GB_C(BT5) : S == 5 ? GB_C(BT6) : GB_C(BT7);
 }
 // dense-output polynomial coefficients  u(Th) = u0 + dt*Th*(k0 + Th*(C2 + Th*(C3 + Th*C4)))
 GB_D void dense_coeffs(double k0, const GbK& k, double k6, double& C2, double& C3, double& C4) {
     const double k2 = k.get(1), k3 = k.get(2), k4 = k.get(3), k5 = k.get(4), k6_ = k.get(5);
-    C2 = fma(GB_R72, k6, fma(GB_R62, k6_, fma(GB_R52, k5, fma(GB_R42, k4, fma(GB_R32, k3, fma(GB_R22, k2, GB_R12 * k0))))));
-    C3 = fma(GB_R73, k6, fma(GB_R63, k6_, fma(GB_R53, k5, fma(GB_R43, k4, fma(GB_R33, k3, fma(GB_R23, k2, GB_R13 * k0))))));
-    C4 = fma(GB_R74, k6, fma(GB_R64, k6_, fma(GB_R54, k5, fma(GB_R44, k4, fma(GB_R34, k3, fma(GB_R24, k2, GB_R14 * k0))))));
+    C2 = fma(GB_C(R72), k6, fma(GB_C(R62), k6_, fma(GB_C(R52), k5, fma(GB_C(R42), k4, fma(GB_C(R32), k3, fma(GB_C(R22), k2, GB_C(R12) * k0))))));
+    C3 = fma(GB_C(R73), k6, fma(GB_C(R63), k6_, fma(GB_C(R53), k5, fma(GB_C(R43), k4, fma(GB_C(R33), k3, fma(GB_C(R23), k2, GB_C(R13) * k0))))));
+    C4 = fma(GB_C(R74), k6, fma(GB_C(R64), k6_, fma(GB_C(R54), k5, fma(GB_C(R44), k4, fma(GB_C(R34), k3, fma(GB_C(R24), k2, GB_C(R14) * k0))))));
 }
 GB_D double dense_eval(double u0, double dt, double Th, double C1, double C2, double C3, double C4) {
     return fma(dt * Th, fma(Th, fma(Th, fma(Th, C4, C3), C2), C1), u0);
@@ -268,13 +268,13 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
                     // change_t_via_interpolation!: full state from the Tsit5 interpolant at Theta = lo
                     const double Th = lo, Th2 = Th * Th;
                     double b[7];
-                    b[0] = Th * fma(Th, fma(Th, fma(Th, GB_R14, GB_R13), GB_R12), 1.0);
-                    b[1] = Th2 * fma(Th, fma(Th, GB_R24, GB_R23), GB_R22);
-                    b[2] = Th2 * fma(Th, fma(Th, GB_R34, GB_R33), GB_R32);
-                    b[3] = Th2 * fma(Th, fma(Th, GB_R44, GB_R43), GB_R42);
-                    b[4] = Th2 * fma(Th, fma(Th, GB_R54, GB_R53), GB_R52);
-                    b[5] = Th2 * fma(Th, fma(Th, GB_R64, GB_R63), GB_R62);
-                    b[6] = Th2 * fma(Th, fma(Th, GB_R74, GB_R73), GB_R72);
+                    b[0] = Th * fma(Th, fma(Th, fma(Th, GB_C(R14), GB_C(R13)), GB_C(R12)), 1.0);
+                    b[1] = Th2 * fma(Th, fma(Th, GB_C(R24), GB_C(R23)), GB_C(R22));
+                    b[2] = Th2 * fma(Th, fma(Th, GB_C(R34), GB_C(R33)), GB_C(R32));
+                    b[3] = Th2 * fma(Th, fma(Th, GB_C(R44), GB_C(R43)), GB_C(R42));
+                    b[4] = Th2 * fma(Th, fma(Th, GB_C(R54), GB_C(R53)), GB_C(R52));
+                    b[5] = Th2 * fma(Th, fma(Th, GB_C(R64), GB_C(R63)), GB_C(R62));
+                    b[6] = Th2 * fma(Th, fma(Th, GB_C(R74), GB_C(R73)), GB_C(R72));
                     // stage v^t, v^phi are recomputed from the stored accelerations (bitwise the same values)
                     double W0[7], W3[7], WR[7], WT[7];
                     double st = 0, sr = 0, sth = 0, sph = 0, s0 = 0, s1 = 0, s2 = 0, s3 = 0;
@@ -444,12 +444,12 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
         }
         if (state == LANE_RUN) {
             double acc[4], s_ = 0, c_ = 1;
-            double tsum = GB_A71 * vt, psum = GB_A71 * vph; // sum_j a7j k_j[1], k_j[4]
-            double terr = GB_BT1 * vt, perr = GB_BT1 * vph; // sum_j btilde_j k_j[1], k_j[4]
+            double tsum = GB_C(A71) * vt, psum = GB_C(A71) * vph; // sum_j a7j k_j[1], k_j[4]
+            double terr = GB_C(BT1) * vt, perr = GB_C(BT1) * vph; // sum_j btilde_j k_j[1], k_j[4]
             // the other six error sums are accumulated stage by stage too (btilde_1 .. btilde_7 in order): their FMAs fill
             // the latency gaps of the next stage instead of forming a serial tail after the seventh
-            double rerr = GB_BT1 * vr, therr = GB_BT1 * vth;
-            double a0err = GB_BT1 * kA0.get(0), a1err = GB_BT1 * kA1.get(0), a2err = GB_BT1 * kA2.get(0), a3err = GB_BT1 * kA3.get(0);
+            double rerr = GB_C(BT1) * vr, therr = GB_C(BT1) * vth;
+            double a0err = GB_C(BT1) * kA0.get(0), a1err = GB_C(BT1) * kA1.get(0), a2err = GB_C(BT1) * kA2.get(0), a3err = GB_C(BT1) * kA3.get(0);
             // running maxima of the high words of |k_j[r]|, |k_j[theta]| for the event-scan pre-test (no re-read from shared memory)
             int mxr = __double2hiint(vr) & 0x7fffffff, mxt = __double2hiint(vth) & 0x7fffffff;
 #define GB_STAGE(S)                                                                                                     \
@@ -475,8 +475,8 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
             nvt = comb<6>(vt, dt, kA0.get(0), kA0); nvr = comb<6>(vr, dt, kA1.get(0), kA1);
             nvth = comb<6>(vth, dt, kA2.get(0), kA2); nvph = comb<6>(vph, dt, kA3.get(0), kA3);
             nct = fma(dt, tsum, ct); nph = fma(dt, psum, ph);
-            terr = fma(GB_BT7, nvt, terr); perr = fma(GB_BT7, nvph, perr);
-            rerr = fma(GB_BT7, nvr, rerr); therr = fma(GB_BT7, nvth, therr);
+            terr = fma(GB_C(BT7), nvt, terr); perr = fma(GB_C(BT7), nvph, perr);
+            rerr = fma(GB_C(BT7), nvr, rerr); therr = fma(GB_C(BT7), nvth, therr);
             // the eight error scales only need u_prev and u: they are formed while the seventh RHS is in flight
             const double is0 = gb_inv_scale(ct, nct, reltol, abstol), is1 = gb_inv_scale(r, nr, reltol, abstol);
             const double is2 = gb_inv_scale(th, nth, reltol, abstol), is3 = gb_inv_scale(ph, nph, reltol, abstol);
@@ -495,10 +495,10 @@ __global__ void __launch_bounds__(GB_BLOCK, GB_MIN_BLOCKS) gb200_trace_kernel(co
             // ---- error estimate: rms( dt*sum btilde_j k_j / (abstol + max(|u_prev|,|u|) reltol) )
             {
                 double q_;
-                q_ = fma(GB_BT7, acc[0], a0err) * is4; ee = fma(q_, q_, ee);
-                q_ = fma(GB_BT7, acc[1], a1err) * is5; ee = fma(q_, q_, ee);
-                q_ = fma(GB_BT7, acc[2], a2err) * is6; ee = fma(q_, q_, ee);
-                q_ = fma(GB_BT7, acc[3], a3err) * is7; ee = fma(q_, q_, ee);
+                q_ = fma(GB_C(BT7), acc[0], a0err) * is4; ee = fma(q_, q_, ee);
+                q_ = fma(GB_C(BT7), acc[1], a1err) * is5; ee = fma(q_, q_, ee);
+                q_ = fma(GB_C(BT7), acc[2], a2err) * is6; ee = fma(q_, q_, ee);
+                q_ = fma(GB_C(BT7), acc[3], a3err) * is7; ee = fma(q_, q_, ee);
             }
             // EEst^2 = dt^2 sum_i (.)^2 / 8; the controller only needs log EEst = log(EEst^2) / 2 and the test EEst <= 1, so no
             // square root is taken (the Float32 controller mode takes it where it needs EEst itself).  An exactly zero
